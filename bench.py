@@ -25,6 +25,12 @@ buffers are summed onto rank 0 with an NCCL reduce), so scaling is STRONG: the t
   load_s, cli_s  scene file -> HBM (parse, both BVH builds, upload), and the wall time of run.sh on the scene.
 
 `--impl reference` times the reference arm as its own JSON line.
+
+`--dump-outputs DIR` writes what the last device-resident timed step computed, the float32 radiance sums over its
+samples that render_accumulate leaves in the caller's buffer, as DIR/radiance_sum.npy (H x W x 3).  A frame larger
+than 2,097,152 pixels is stored as a fixed, seeded sample of that many pixels: DIR/radiance_sum.npy (n x 3) and the
+flat pixel indices it came from, DIR/radiance_sum_pixel.npy (float64).  Seeds depend on the step number only, so two
+runs with the same arguments render the same paths and agree up to float summation order.
 """
 import argparse
 import ctypes
@@ -50,6 +56,7 @@ CONFIGS = {
     4: {"scene": "practice5_dragon_100k_glass"},
     5: {"scene": "practice5_dragon_100k_metal", "width": 3840, "height": 2160, "spp": 1024},
 }
+DUMP_PIXELS = 1 << 21   # --dump-outputs: at most 24 MB of sums + 16 MB of pixel indices
 
 
 def scene_file(name):
@@ -146,6 +153,22 @@ class ClockSampler(threading.Thread):
         reasons = sorted(r for r in self.reasons if r not in ("GpuIdle", "None", "ApplicationsClocksSetting"))
         return {"sm_mhz": float(np.median(self.samples)), "sm_max_mhz": self.max_mhz, "reasons": reasons,
                 "samples": len(self.samples)}
+
+
+def dump_outputs(out_dir, accum, width, height):
+    """Writes the float32 accumulation buffer `accum` (a device tensor of H * W * 3 sums) under out_dir, sampled
+    to DUMP_PIXELS seeded pixels when the frame is larger."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    npix = width * height
+    rgb = accum.view(npix, 3)
+    if npix <= DUMP_PIXELS:
+        np.save(os.path.join(out_dir, "radiance_sum.npy"), rgb.view(height, width, 3).cpu().numpy())
+        return
+    pick = np.sort(np.random.default_rng(0).choice(npix, DUMP_PIXELS, replace=False))
+    sample = rgb.index_select(0, torch.from_numpy(pick).to(accum.device))
+    np.save(os.path.join(out_dir, "radiance_sum.npy"), sample.cpu().numpy())
+    np.save(os.path.join(out_dir, "radiance_sum_pixel.npy"), pick.astype(np.float64))
 
 
 def resolve_config(args):
@@ -246,7 +269,11 @@ def main():
     ap.add_argument("--traversal", type=int, default=0)
     ap.add_argument("--frames-in-flight", type=int, default=2, choices=[1, 2],
                     help="device-resident timing: frames queued on alternating streams (every frame still complete in the timed region)")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write the radiance sums of the last device-resident timed step as DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -383,6 +410,9 @@ def main():
     ms_total = timed(args.steps, 100, pipelined)
     clocks = sampler.result()
     cnt = scene.counters()
+    if args.dump_outputs and rank == 0:   # rank 0 holds the reduced sums; the passes below reuse the buffers
+        last = 100 + args.steps - 1
+        dump_outputs(args.dump_outputs, accums[last % nflight if pipelined else 0], W, H)
     # ---- the same steps again with CUDA events around every kernel (roofline durations)
     scene.set_profiling(kernel_events=True, count_visits=False)
     render_step(0, False)   # the single-stream pass may need larger wavefront buffers: allocate them untimed
