@@ -135,6 +135,22 @@ int rtc_render_u8(rtc_scene* s, uint32_t seed, uint8_t* rgb_host);
 int rtc_render_sum(rtc_scene* s, uint32_t seed, uint32_t sample_begin, uint32_t sample_count, float* sum_host);
 /* run.sh <scene> <out.ppm> in one call: "P6\nW H\n255\n" + bytes (src/scene.cpp:206-208,243-251) */
 int rtc_render_ppm(rtc_scene* s, uint32_t seed, const char* out_path);
+/* ---- adaptive sampling: Scene::Render with a noise threshold instead of a fixed sample count per pixel (single
+ *      device).  The frame is cut into RTC_ADAPTIVE_TILE x RTC_ADAPTIVE_TILE tiles (partial at the right and bottom
+ *      edges).  Every tile starts with samples [0, n0), n0 = min(min_samples, max); a pass renders [n, target) for each
+ *      still-active tile, the even samples into one half sum A and the odd ones into another, B.  A tile then stops when
+ *      its error E < tolerance, else it goes on to target = min(2 target, max).  E = the mean over the tile's pixels of
+ *      (|D(a_r) - D(b_r)| + |D(a_g) - D(b_g)| + |D(a_b) - D(b_b)|) / 3 with a = A / ceil(n/2), b = B / floor(n/2) and
+ *      D = the display value before 8-bit rounding (ACES, gamma 1/2.2); a NaN error keeps the tile.  tolerance = 0
+ *      renders max samples everywhere.  Samples use the streams of rtc_render_accumulate: a pixel that took n samples
+ *      holds the sums of its samples [0, n).  max_samples = 0: the scene's SAMPLES.  tolerance must be finite and >= 0,
+ *      min_samples >= 2 (else RTC_ERR_ARG).  hw1 / hw2 render their one frame: spp = 1, A = the frame, B = 0.
+ * stats: passes, paths rendered, tiles, tiles stopped below max_samples.  Every output may be NULL.
+ * rgb_host: 3 bytes per pixel, to_u8(aces(1/spp * (A + B))).
+ * halves_host: 6 floats per pixel (even-sample sum rgb, odd-sample sum rgb); spp_host: 1 per pixel. */
+#define RTC_ADAPTIVE_TILE 8
+int rtc_render_adaptive(rtc_scene* s, uint32_t seed, float tolerance, uint32_t min_samples, uint32_t max_samples,
+                        uint8_t* rgb_host, float* halves_host, uint32_t* spp_host, uint64_t stats[4]);
 /* ---- Scene::Render on several devices of this process (src/scene.cpp:205-252 uses every hardware thread of the
  *      machine, :212): the samples are split over devices[0..ndev) (a device may be listed more than once), each
  *      renders its range into its own buffer, and devices[0] sums them where they lie -- peer access over NVLink --

@@ -72,6 +72,7 @@ _SIGNATURES = {
     "rtc_render_u8": (C.c_int, [C.c_void_p, C.c_uint32, _u8]),
     "rtc_render_sum": (C.c_int, [C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, _f32]),
     "rtc_render_ppm": (C.c_int, [C.c_void_p, C.c_uint32, C.c_char_p]),
+    "rtc_render_adaptive": (C.c_int, [C.c_void_p, C.c_uint32, C.c_float, C.c_uint32, C.c_uint32, _u8, _f32, _u32, _u64]),
     "rtc_set_batch_paths": (C.c_int, [C.c_void_p, C.c_uint64]),
     "rtc_set_profiling": (C.c_int, [C.c_void_p, C.c_int, C.c_int]),
     "rtc_render_profile": (C.c_int, [C.c_void_p, C.c_void_p, np.ctypeslib.ndpointer(dtype=np.float64, flags="C_CONTIGUOUS"), _u64, C.c_int]),
@@ -294,6 +295,20 @@ class Scene:
         out = np.zeros((self.height, self.width, 3), np.uint8)
         _check(self.lib, self.lib.rtc_render_u8(self.h, seed, out))
         return out
+
+    def RenderAdaptive(self, tolerance, min_samples=16, max_samples=0, seed=0):
+        """Scene::Render with a noise threshold (rtc_render_adaptive): each 8x8 tile takes samples until the difference
+        between the means of its even and its odd samples, in display units, is below `tolerance`, at most
+        `max_samples` (0 = the scene's SAMPLES).  Returns the 8-bit image (H, W, 3), the even / odd sample sums
+        (H, W, 2, 3 float32), the samples per pixel (H, W uint32) and the stats dict (passes, paths, tiles,
+        tiles_stopped)."""
+        img = np.zeros((self.height, self.width, 3), np.uint8)
+        halves = np.zeros((self.height, self.width, 2, 3), np.float32)
+        spp = np.zeros((self.height, self.width), np.uint32)
+        st = np.zeros(4, np.uint64)
+        _check(self.lib, self.lib.rtc_render_adaptive(self.h, seed, float(tolerance), min_samples, max_samples,
+                                                      img, halves, spp, st))
+        return img, halves, spp, dict(zip(["passes", "paths", "tiles", "tiles_stopped"], [int(v) for v in st]))
 
     def RenderMulti(self, devices, seed=0, want_sum=False):
         """Scene::Render on several CUDA devices of this process: samples split over `devices`, summed over peer

@@ -154,6 +154,22 @@ struct rtc_scene {
     DevBuf<unsigned long long> stats;    // 16 words: rtc_render_counters (8) + rtc_traverse_lanes (8)
     DevBuf<float> accum;                 // internal accumulation buffer for the convenience calls
     DevBuf<uint8_t> rgb;
+    // rtc_render_adaptive: the even- and odd-sample sums per pixel, the active tile and pixel lists of the current and the
+    // next pass, the samples every tile took, the list lengths (tiles, pixels) of both passes and their pinned host copy
+    struct Adaptive {
+        DevBuf<float4> half[2];
+        DevBuf<uint32_t> tiles[2], pixels[2], tile_n, counts, spp;
+        DevBuf<float> halves;
+        uint32_t* counts_host = nullptr;   // cudaMallocHost
+        void release() {
+            for (auto& b : half) b.release();
+            for (auto& b : tiles) b.release();
+            for (auto& b : pixels) b.release();
+            tile_n.release(); counts.release(); spp.release(); halves.release();
+            if (counts_host) cudaFreeHost(counts_host);
+            counts_host = nullptr;
+        }
+    } adaptive;
     uint64_t launches = 0;
     // optional per-kernel timing (CUDA events on the launching stream)
     bool profiling = false;
@@ -233,7 +249,7 @@ struct rtc_scene {
         multi_done = nullptr;
         if (fork) cudaEventDestroy(fork);
         fork = nullptr;
-        stats.release(); accum.release(); rgb.release();
+        stats.release(); accum.release(); rgb.release(); adaptive.release();
         for (auto& b : accum4) b.release();
         for (auto& b : probe.fin) b.release();
         for (auto& b : probe.fout) b.release();
@@ -569,6 +585,91 @@ int ensure_wavefront(rtc_scene* s, uint64_t cap, int nlanes) {
     return RTC_OK;
 }
 
+// Which (pixel, sample) path p of a render is: pixel p % npix of the frame and sample sample_first + p / npix when
+// plist is null (rtc_render_accumulate), else pixel plist[p % npix] and sample sample_first + 2 (p / npix) (an adaptive
+// pass renders the even or the odd samples of its pixel list)
+struct PathMap {
+    const uint32_t* plist;
+    uint32_t npix;
+    uint32_t sample_first;
+};
+// fork: the lane streams of the next render_paths calls start after everything already queued on the caller's stream
+int fork_lanes(rtc_scene* s, cudaStream_t user) {
+    if (!s->fork) CU(cudaEventCreateWithFlags(&s->fork, cudaEventDisableTiming));
+    CU(cudaEventRecord(s->fork, user));
+    return RTC_OK;
+}
+// join: the caller's stream continues when the lanes in `used` (bit i = lane i) are done
+int join_lanes(rtc_scene* s, unsigned used, cudaStream_t user) {
+    for (int i = 0; i < rtc_scene::kMaxLanes; ++i) {
+        if (!(used >> i & 1u)) continue;
+        CU(cudaEventRecord(s->lanes[i].done, s->lanes[i].stream));
+        CU(cudaStreamWaitEvent(user, s->lanes[i].done, 0));
+    }
+    return RTC_OK;
+}
+// The wavefront batches of `total` paths laid out by `map`: every hit deposits into `target` (float4 per pixel of the
+// frame).  The lanes wait for the last fork_lanes; the lanes that carry work are added to *used.
+int render_paths(rtc_scene* s, const DevScene& S, uint32_t seed, const PathMap& map, uint64_t total, float4* target, unsigned* used) {
+    int rc;
+    const uint32_t depth = s->host.ray_depth;
+    // batch size: the configured one, but small enough that every lane gets a batch (overlap matters
+    // more than batch size: profiles/r01_experiments.md), rounded up to whole warps
+    uint64_t cap = total < s->batch_paths ? total : s->batch_paths;
+    // A small render (the share of one GPU of eight: 4 Mi paths) is ONE batch on the next lane in turn instead of one
+    // batch per lane: its launches are twice as large (a persistent k_traverse launch ends with its longest ray, ~30 us
+    // whatever its size), and the overlap comes from the caller's next render, which takes the other lane.
+    const bool whole = !s->profiling && s->nlanes > 1 && total <= s->small_render_paths;
+    if (!s->profiling && s->nlanes > 1 && !whole) {
+        uint64_t per_lane = ((total + s->nlanes - 1) / s->nlanes + 31) & ~(uint64_t)31;
+        if (per_lane < cap) cap = per_lane;
+    }
+    const uint64_t nbatches = (total + cap - 1) / cap;
+    // per-kernel event timing needs the kernels back to back on one stream
+    const int nlanes = s->profiling ? 1 : whole ? s->nlanes : (int)(nbatches < (uint64_t)s->nlanes ? nbatches : (uint64_t)s->nlanes);
+    const int lane_first = whole ? (int)(s->next_lane++ % (unsigned)s->nlanes) : 0;
+    if ((rc = ensure_wavefront(s, cap, nlanes))) return rc;
+    for (int i = 0; i < nlanes; ++i)
+        if (!whole || i == lane_first) {   // the other lanes belong to the caller's other renders
+            CU(cudaStreamWaitEvent(s->lanes[i].stream, s->fork, 0));
+            *used |= 1u << i;
+        }
+    uint64_t batch = 0;
+    for (uint64_t first = 0; first < total; first += cap, ++batch) {
+        rtc_scene::Lane& L = s->lanes[(lane_first + batch) % nlanes];
+        cudaStream_t st = L.stream;
+        LaunchCtx c{st, s->sms};
+        uint32_t* tqc = L.queue.p + 2 * kMaxDepthSlots;    // rays queued for k_traverse, per bounce
+        uint32_t* cursor = L.queue.p + 3 * kMaxDepthSlots; // k_traverse work cursors, per bounce
+        uint32_t count = (uint32_t)((total - first) < cap ? (total - first) : cap);
+        CU(cudaMemsetAsync(L.queue.p, 0, 4 * kMaxDepthSlots * sizeof(uint32_t), st));
+        PathSoA cur{L.path[0][0].p, L.path[0][1].p, L.path[0][2].p};
+        PathSoA nxt{L.path[1][0].p, L.path[1][1].p, L.path[1][2].p};
+        HitSoA hcur{L.hit_id[0].p}, hnxt{L.hit_id[1].p};
+        s->span_begin(0, st);
+        if (map.plist) launch_generate_list(c, S, cur, hcur, L.queue.p, L.trav_queue.p, tqc, first, count, seed, map.plist, map.npix, map.sample_first);
+        else launch_generate(c, S, cur, hcur, L.queue.p, L.trav_queue.p, tqc, first, count, seed, map.sample_first);
+        s->span_end(st);
+        s->launches++;
+        for (uint32_t b = 1; b <= depth; ++b) {
+            s->span_begin(1, st);
+            if (s->traversal == RTC_TRAVERSAL_REFTREE) launch_extend_reftree(c, S, cur, hcur, L.queue.p + 2 * (b - 1), count);
+            else launch_traverse(c, S, cur, hcur, count, L.trav_queue.p, tqc + (b - 1), cursor + (b - 1), s->count_visits, s->stats.p);
+            s->span_end(st);
+            s->span_begin(2, st);
+            launch_shade(c, S, cur, hcur, nxt, hnxt, L.queue.p + 2 * (b - 1), L.queue.p + 2 * b, L.trav_queue.p, tqc + b, count,
+                         target, b, seed);
+            s->span_end(st);
+            s->launches += 2;
+            PathSoA tmp = cur; cur = nxt; nxt = tmp;
+            HitSoA htmp = hcur; hcur = hnxt; hnxt = htmp;
+        }
+        launch_tally(c, L.queue.p, tqc, depth, s->stats.p);
+        s->launches++;
+    }
+    return RTC_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -852,23 +953,6 @@ int rtc_render_accumulate(rtc_scene* s, uint32_t seed, uint32_t sample_begin, ui
         CU(cudaGetLastError());
         return RTC_OK;
     }
-    const uint32_t depth = s->host.ray_depth;
-    // batch size: the configured one, but small enough that every lane gets a batch (overlap matters
-    // more than batch size: profiles/r01_experiments.md), rounded up to whole warps
-    uint64_t cap = total < s->batch_paths ? total : s->batch_paths;
-    // A small render (the share of one GPU of eight: 4 Mi paths) is ONE batch on the next lane in turn instead of one
-    // batch per lane: its launches are twice as large (a persistent k_traverse launch ends with its longest ray, ~30 us
-    // whatever its size), and the overlap comes from the caller's next render, which takes the other lane.
-    const bool whole = !s->profiling && s->nlanes > 1 && total <= s->small_render_paths;
-    if (!s->profiling && s->nlanes > 1 && !whole) {
-        uint64_t per_lane = ((total + s->nlanes - 1) / s->nlanes + 31) & ~(uint64_t)31;
-        if (per_lane < cap) cap = per_lane;
-    }
-    const uint64_t nbatches = (total + cap - 1) / cap;
-    // per-kernel event timing needs the kernels back to back on one stream
-    const int nlanes = s->profiling ? 1 : whole ? s->nlanes : (int)(nbatches < (uint64_t)s->nlanes ? nbatches : (uint64_t)s->nlanes);
-    const int lane_first = whole ? (int)(s->next_lane++ % (unsigned)s->nlanes) : 0;
-    if ((rc = ensure_wavefront(s, cap, nlanes))) return rc;
     cudaStream_t user = (cudaStream_t)stream;
     // the float4 pixel sums of this render: two buffers used alternately, so that two renders may be in flight on
     // two streams; a third waits for the first to have been folded
@@ -882,48 +966,10 @@ int rtc_render_accumulate(rtc_scene* s, uint32_t seed, uint32_t sample_begin, ui
     const int arena = s->arena_cur;
     if (s->arena_pending) CU(cudaStreamWaitEvent(user, s->arena_ready[arena], 0));
     DevScene S = s->dev();
-    // fork: the lane streams start after everything already queued on the caller's stream
-    CU(cudaEventRecord(s->fork, user));
-    for (int i = 0; i < nlanes; ++i)
-        if (!whole || i == lane_first) CU(cudaStreamWaitEvent(s->lanes[i].stream, s->fork, 0));
-    uint64_t batch = 0;
-    for (uint64_t first = 0; first < total; first += cap, ++batch) {
-        rtc_scene::Lane& L = s->lanes[(lane_first + batch) % nlanes];
-        cudaStream_t st = L.stream;
-        LaunchCtx c{st, s->sms};
-        uint32_t* tqc = L.queue.p + 2 * kMaxDepthSlots;    // rays queued for k_traverse, per bounce
-        uint32_t* cursor = L.queue.p + 3 * kMaxDepthSlots; // k_traverse work cursors, per bounce
-        uint32_t count = (uint32_t)((total - first) < cap ? (total - first) : cap);
-        CU(cudaMemsetAsync(L.queue.p, 0, 4 * kMaxDepthSlots * sizeof(uint32_t), st));
-        PathSoA cur{L.path[0][0].p, L.path[0][1].p, L.path[0][2].p};
-        PathSoA nxt{L.path[1][0].p, L.path[1][1].p, L.path[1][2].p};
-        HitSoA hcur{L.hit_id[0].p}, hnxt{L.hit_id[1].p};
-        s->span_begin(0, st);
-        launch_generate(c, S, cur, hcur, L.queue.p, L.trav_queue.p, tqc, first, count, seed, sample_begin);
-        s->span_end(st);
-        s->launches++;
-        for (uint32_t b = 1; b <= depth; ++b) {
-            s->span_begin(1, st);
-            if (s->traversal == RTC_TRAVERSAL_REFTREE) launch_extend_reftree(c, S, cur, hcur, L.queue.p + 2 * (b - 1), count);
-            else launch_traverse(c, S, cur, hcur, count, L.trav_queue.p, tqc + (b - 1), cursor + (b - 1), s->count_visits, s->stats.p);
-            s->span_end(st);
-            s->span_begin(2, st);
-            launch_shade(c, S, cur, hcur, nxt, hnxt, L.queue.p + 2 * (b - 1), L.queue.p + 2 * b, L.trav_queue.p, tqc + b, count,
-                         accum4.p, b, seed);
-            s->span_end(st);
-            s->launches += 2;
-            PathSoA tmp = cur; cur = nxt; nxt = tmp;
-            HitSoA htmp = hcur; hcur = hnxt; hnxt = htmp;
-        }
-        launch_tally(c, L.queue.p, tqc, depth, s->stats.p);
-        s->launches++;
-    }
-    // join: the caller's stream continues when every lane is done
-    for (int i = 0; i < nlanes; ++i) {
-        if (whole && i != lane_first) continue;   // the other lanes belong to the caller's other renders
-        CU(cudaEventRecord(s->lanes[i].done, s->lanes[i].stream));
-        CU(cudaStreamWaitEvent(user, s->lanes[i].done, 0));
-    }
+    if ((rc = fork_lanes(s, user))) return rc;
+    unsigned used = 0;
+    if ((rc = render_paths(s, S, seed, PathMap{nullptr, (uint32_t)npix, sample_begin}, total, accum4.p, &used))) return rc;
+    if ((rc = join_lanes(s, used, user))) return rc;
     launch_fold(LaunchCtx{user, s->sms}, accum4.p, accum_dev, (uint32_t)npix);
     s->launches++;
     CU(cudaEventRecord(s->accum4_idle[a4], user));
@@ -1012,6 +1058,113 @@ int rtc_render_ppm(rtc_scene* s, uint32_t seed, const char* out_path) {
     out << "P6\n" << s->host.cam.width << " " << s->host.cam.height << "\n" << 255 << "\n";  // src/scene.cpp:206-208
     out.write(reinterpret_cast<const char*>(img.data()), (std::streamsize)img.size());
     if (!out) return fail(RTC_ERR_IO, std::string("write failed: ") + out_path);
+    return RTC_OK;
+}
+
+// ------------------------------------------------------------------ adaptive sampling
+// Passes over the still-active 8x8 tiles: every active tile renders samples [n, target) -- the even ones into one
+// half-sum buffer, the odd ones into the other, one render_paths call each, so that small passes run on two lanes at
+// once -- then k_adaptive_tiles measures the tiles' error from the two halves and lists the tiles (and their pixels) that
+// go on to target = min(2 target, max).  The length of the next pixel list is the one read back per pass.
+static_assert(kAdaptiveTile == RTC_ADAPTIVE_TILE, "rt_kernels.h and rtc_b200.h disagree on the tile size");
+int rtc_render_adaptive(rtc_scene* s, uint32_t seed, float tolerance, uint32_t min_samples, uint32_t max_samples,
+                        uint8_t* rgb_host, float* halves_host, uint32_t* spp_host, uint64_t stats[4]) {
+    if (!s) return fail(RTC_ERR_ARG, "null scene");
+    if (!std::isfinite(tolerance) || tolerance < 0.f) return fail(RTC_ERR_ARG, "tolerance must be finite and >= 0");
+    if (min_samples < 2) return fail(RTC_ERR_ARG, "min_samples must be at least 2");
+    int rc = need_device(s);
+    if (rc) return rc;
+    const uint32_t width = s->host.cam.width, height = s->host.cam.height;
+    const uint32_t npix = width * height;
+    const uint32_t ntiles = ((width + kAdaptiveTile - 1) / kAdaptiveTile) * ((height + kAdaptiveTile - 1) / kAdaptiveTile);
+    uint64_t st[4] = {0, 0, 0, 0};   // passes, paths, tiles, tiles stopped below the maximum
+    if (stats) std::memcpy(stats, st, sizeof st);
+    if (npix == 0) return RTC_OK;
+    const size_t nvalues = 3 * (size_t)npix;
+    CU(s->rgb.ensure(nvalues));
+    if (s->host.dialect <= DIALECT_HW2) {
+        // hw1 / hw2: the one deterministic frame, resolved as rtc_render_u8 does; it is the "even" half, spp = 1
+        CU(s->accum.ensure(nvalues));
+        CU(cudaMemsetAsync(s->accum.p, 0, nvalues * sizeof(float), nullptr));
+        if ((rc = rtc_render_accumulate(s, seed, 0, 1, s->accum.p, nullptr))) return rc;
+        if ((rc = rtc_render_resolve(s, s->accum.p, 1, s->rgb.p, nullptr))) return rc;
+        if (rgb_host) CU(cudaMemcpy(rgb_host, s->rgb.p, nvalues, cudaMemcpyDeviceToHost));
+        if (halves_host) {
+            std::vector<float> frame(nvalues);
+            CU(cudaMemcpy(frame.data(), s->accum.p, nvalues * sizeof(float), cudaMemcpyDeviceToHost));
+            for (size_t i = 0; i < npix; ++i)
+                for (int c = 0; c < 3; ++c) { halves_host[6 * i + c] = frame[3 * i + c]; halves_host[6 * i + 3 + c] = 0.f; }
+        }
+        if (spp_host) for (size_t i = 0; i < npix; ++i) spp_host[i] = 1;
+        const uint64_t one[4] = {1, npix, ntiles, 0};
+        if (stats) std::memcpy(stats, one, sizeof one);
+        return RTC_OK;
+    }
+    const uint32_t smax = max_samples ? max_samples : s->host.samples;
+    if (smax == 0) return fail(RTC_ERR_ARG, "scene has SAMPLES 0");
+    rtc_scene::Adaptive& ad = s->adaptive;
+    for (auto& b : ad.half) CU(b.ensure(npix));
+    for (auto& b : ad.tiles) CU(b.ensure(ntiles));
+    for (auto& b : ad.pixels) CU(b.ensure(npix));
+    CU(ad.tile_n.ensure(ntiles));
+    CU(ad.counts.ensure(4));
+    if (!ad.counts_host) CU(cudaMallocHost(&ad.counts_host, 2 * sizeof(uint32_t)));
+    cudaStream_t user = nullptr;
+    LaunchCtx c{user, s->sms};
+    for (auto& b : ad.half) CU(cudaMemsetAsync(b.p, 0, npix * sizeof(float4), user));
+    CU(cudaMemsetAsync(ad.counts.p, 0, 4 * sizeof(uint32_t), user));
+    const int arena = s->arena_cur;
+    if (s->arena_pending) CU(cudaStreamWaitEvent(user, s->arena_ready[arena], 0));
+    DevScene S = s->dev();
+    // every tile is active with n = 0; lists of pass 0 in set 0
+    launch_adaptive_tiles(c, nullptr, nullptr, width, height, nullptr, ntiles, 0, 0.f, 0.f, tolerance, ADAPTIVE_FIRST, ad.tile_n.p,
+                          ad.tiles[0].p, ad.pixels[0].p, ad.counts.p);
+    s->launches++;
+    uint32_t active_tiles = ntiles, active_pix = npix, n = 0, target = min_samples < smax ? min_samples : smax;
+    int cur = 0;
+    st[2] = ntiles;
+    for (;;) {
+        ++st[0];
+        if ((rc = fork_lanes(s, user))) return rc;
+        unsigned used = 0;
+        for (uint32_t h = 0; h < 2; ++h) {   // h = 0: the even samples of [n, target) into half 0, h = 1: the odd ones
+            const uint32_t first = n + ((n ^ h) & 1u);
+            if (first >= target) continue;
+            const uint64_t total = (uint64_t)((target - first + 1) / 2) * active_pix;
+            if ((rc = render_paths(s, S, seed, PathMap{ad.pixels[cur].p, active_pix, first}, total, ad.half[h].p, &used))) return rc;
+            st[1] += total;
+        }
+        if ((rc = join_lanes(s, used, user))) return rc;
+        n = target;
+        const bool last = n == smax;
+        const int nxt = cur ^ 1;
+        if (!last) CU(cudaMemsetAsync(ad.counts.p + 2 * nxt, 0, 2 * sizeof(uint32_t), user));
+        launch_adaptive_tiles(c, ad.half[0].p, ad.half[1].p, width, height, ad.tiles[cur].p, active_tiles, n, 1.f / (float)((n + 1) / 2),
+                              1.f / (float)(n / 2), tolerance, last ? ADAPTIVE_LAST : ADAPTIVE_DECIDE, ad.tile_n.p, ad.tiles[nxt].p,
+                              ad.pixels[nxt].p, ad.counts.p + 2 * nxt);
+        s->launches++;
+        if (last) break;
+        CU(cudaMemcpyAsync(ad.counts_host, ad.counts.p + 2 * nxt, 2 * sizeof(uint32_t), cudaMemcpyDeviceToHost, user));
+        CU(cudaStreamSynchronize(user));
+        st[3] += active_tiles - ad.counts_host[0];
+        active_tiles = ad.counts_host[0];
+        active_pix = ad.counts_host[1];
+        if (active_tiles == 0) break;
+        cur = nxt;
+        target = (uint64_t)2 * target < smax ? 2 * target : smax;
+    }
+    CU(ad.halves.ensure(halves_host ? 6 * (size_t)npix : 0));
+    CU(ad.spp.ensure(spp_host ? npix : 0));
+    launch_resolve_adaptive(c, ad.half[0].p, ad.half[1].p, ad.tile_n.p, width, npix, s->rgb.p, halves_host ? ad.halves.p : nullptr,
+                            spp_host ? ad.spp.p : nullptr);
+    s->launches++;
+    CU(cudaEventRecord(s->arena_idle[arena], user));
+    CU(cudaGetLastError());
+    if (rgb_host) CU(cudaMemcpy(rgb_host, s->rgb.p, nvalues, cudaMemcpyDeviceToHost));
+    if (halves_host) CU(cudaMemcpy(halves_host, ad.halves.p, 6 * (size_t)npix * sizeof(float), cudaMemcpyDeviceToHost));
+    if (spp_host) CU(cudaMemcpy(spp_host, ad.spp.p, (size_t)npix * sizeof(uint32_t), cudaMemcpyDeviceToHost));
+    CU(cudaStreamSynchronize(user));
+    if (stats) std::memcpy(stats, st, sizeof st);
     return RTC_OK;
 }
 

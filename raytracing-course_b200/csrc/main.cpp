@@ -4,10 +4,16 @@
 //   RTC_SAMPLES / RTC_WIDTH / RTC_HEIGHT / RTC_RAY_DEPTH   override the scene file
 //   RTC_DEVICES=<list>   render on several devices of the machine, e.g. "0,1,2,3" or "0-7" (samples split over them,
 //                        summed over NVLink peer access on the first): Scene::Render uses the whole machine too
+//   RTC_ADAPTIVE=<tau>   adaptive sampling (rtc_render_adaptive, one device): every 8x8 tile takes samples until its
+//                        noise is below tau display units (1/255 = one 8-bit level), at most the scene's SAMPLES (after
+//                        RTC_SAMPLES); 0 renders every pixel at SAMPLES.  A value that is not a finite number >= 0 or a
+//                        list of several RTC_DEVICES is an error.
+//   RTC_TIMING=1     phase times on stderr (with RTC_ADAPTIVE also the passes and paths rendered)
 // The same program serves the four earlier homework snapshots (hwN/run.sh -> build/raytracing_hwN): the dialect
 // is the digit in the name it is called by (raytracing_hw1 .. raytracing_hw4 are links to this binary), or
 // RTC_DIALECT=<1..5>.
 #include <chrono>
+#include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -39,6 +45,15 @@ static std::vector<int> parse_devices(const char* text) {
     return out;
 }
 
+// "P6\nW H\n255\n" + bytes (src/scene.cpp:206-208, 243-251), as rtc_render_ppm writes it
+static bool write_ppm(const char* path, uint32_t w, uint32_t h, const std::vector<uint8_t>& img) {
+    FILE* f = std::fopen(path, "wb");
+    if (!f) return false;
+    std::fprintf(f, "P6\n%u %u\n255\n", w, h);
+    const bool ok = std::fwrite(img.data(), 1, img.size(), f) == img.size();
+    return std::fclose(f) == 0 && ok;
+}
+
 static int env_int(const char* name, int dflt) {
     const char* v = std::getenv(name);
     return v && *v ? std::atoi(v) : dflt;
@@ -62,6 +77,21 @@ int main(int argc, const char* argv[]) {
     const auto t_start = now();
     const std::vector<int> devices = parse_devices(std::getenv("RTC_DEVICES"));
     const int device0 = devices.empty() ? env_int("RTC_DEVICE", 0) : devices[0];
+    const char* adaptive = std::getenv("RTC_ADAPTIVE");
+    if (adaptive && !*adaptive) adaptive = nullptr;
+    float tau = 0.f;
+    if (adaptive) {
+        char* end = nullptr;
+        tau = std::strtof(adaptive, &end);
+        if (end == adaptive || *end || !std::isfinite(tau) || tau < 0.f) {
+            std::fprintf(stderr, "raytracing_hw5: RTC_ADAPTIVE=%s is not a finite number >= 0\n", adaptive);
+            return 1;
+        }
+        if (devices.size() > 1) {
+            std::fprintf(stderr, "raytracing_hw5: RTC_ADAPTIVE renders on one device; RTC_DEVICES lists %zu\n", devices.size());
+            return 1;
+        }
+    }
     rtc_scene* scene = rtc_scene_load_dialect(argv[1], device0, dialect);
     if (!scene) {
         std::fprintf(stderr, "raytracing_hw5: %s\n", rtc_last_error());
@@ -75,13 +105,29 @@ int main(int argc, const char* argv[]) {
         rtc_scene_free(scene);
         return 1;
     }
-    if (devices.size() > 1) rc = rtc_render_ppm_multi(scene, devices.data(), (int)devices.size(), (uint32_t)env_int("RTC_SEED", 0), argv[2]);
+    uint32_t info[8];
+    rtc_scene_info(scene, info);
+    uint64_t astats[4] = {0, 0, 0, 0};
+    bool written_error = false;
+    if (adaptive) {
+        std::vector<uint8_t> img(3 * (size_t)info[0] * info[1]);
+        rc = rtc_render_adaptive(scene, (uint32_t)env_int("RTC_SEED", 0), tau, 16, 0, img.data(), nullptr, nullptr, astats);
+        if (rc == RTC_OK && !write_ppm(argv[2], info[0], info[1], img)) {
+            std::fprintf(stderr, "raytracing_hw5: cannot write %s\n", argv[2]);
+            rc = RTC_ERR_IO;
+            written_error = true;
+        }
+    } else if (devices.size() > 1) rc = rtc_render_ppm_multi(scene, devices.data(), (int)devices.size(), (uint32_t)env_int("RTC_SEED", 0), argv[2]);
     else rc = rtc_render_ppm(scene, (uint32_t)env_int("RTC_SEED", 0), argv[2]);
-    if (rc != RTC_OK) std::fprintf(stderr, "raytracing_hw5: %s\n", rtc_last_error());
+    if (rc != RTC_OK && !written_error) std::fprintf(stderr, "raytracing_hw5: %s\n", rtc_last_error());
     const auto t_rendered = now();
     if (timing)
         std::fprintf(stderr, "[rtc timing] %-28s %8.1f ms\n[rtc timing] %-28s %8.1f ms\n",
                      "load (file -> HBM, CUDA init)", ms(t_start, t_loaded), "render + PPM", ms(t_loaded, t_rendered));
+    if (timing && adaptive)
+        std::fprintf(stderr, "[rtc timing] adaptive: %llu passes, %llu paths, %llu of %llu tiles stopped below SAMPLES\n",
+                     (unsigned long long)astats[0], (unsigned long long)astats[1], (unsigned long long)astats[3],
+                     (unsigned long long)astats[2]);
     // The image is on disk: leave without unmapping 2 GB of device memory buffer by buffer (0.15 - 1.1 s measured on the
     // B200 box); the driver reclaims everything when the process ends, as it does for the reference's own heap.
     std::fflush(nullptr);

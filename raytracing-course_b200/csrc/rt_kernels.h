@@ -21,6 +21,20 @@ struct LaunchCtx {
 // camera rays of one wavefront batch + their pre_step (planes, index root, traverse queue)
 void launch_generate(const LaunchCtx& c, const DevScene& S, PathSoA P, HitSoA H, uint32_t* q, uint32_t* tq, uint32_t* tq_count,
                      uint64_t first_path, uint32_t count, uint32_t seed, uint32_t sample_begin);
+// the same over a pixel list: path p = pixel plist[p % npix], sample sample_first + 2 (p / npix)
+void launch_generate_list(const LaunchCtx& c, const DevScene& S, PathSoA P, HitSoA H, uint32_t* q, uint32_t* tq, uint32_t* tq_count,
+                          uint64_t first_path, uint32_t count, uint32_t seed, const uint32_t* plist, uint32_t npix, uint32_t sample_first);
+// adaptive sampling (rtc_render_adaptive): square tiles of kAdaptiveTile pixels a side (= RTC_ADAPTIVE_TILE), one warp each
+constexpr uint32_t kAdaptiveTile = 8;
+static_assert(kAdaptiveTile * kAdaptiveTile == 64, "k_adaptive_tiles: one warp per tile, two pixels per lane");
+enum { ADAPTIVE_FIRST = 0, ADAPTIVE_DECIDE = 1, ADAPTIVE_LAST = 2 };
+// per active tile: record n, decide (mode), append the kept tiles and their pixels to the next lists
+void launch_adaptive_tiles(const LaunchCtx& c, const float4* A, const float4* B, uint32_t width, uint32_t height,
+                           const uint32_t* tiles_in, uint32_t ntiles, uint32_t n, float inv_a, float inv_b, float tau, int mode,
+                           uint32_t* tile_n, uint32_t* tiles_out, uint32_t* pixels_out, uint32_t* counts_out);
+// u8 image (and optionally the half sums, 6 floats per pixel, and the samples per pixel) from the even / odd sums
+void launch_resolve_adaptive(const LaunchCtx& c, const float4* A, const float4* B, const uint32_t* tile_n, uint32_t width, uint32_t npix,
+                             uint8_t* out, float* halves, uint32_t* spp);
 // Scene::RayIntersection for the rays of queue P (fills H): launch_pre then launch_traverse
 // (index BVH), or launch_extend_reftree alone (the reference-tree twin).
 void launch_pre(const LaunchCtx& c, const DevScene& S, PathSoA P, HitSoA H, const uint32_t* qcount, uint32_t max_count,
