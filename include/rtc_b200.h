@@ -158,6 +158,18 @@ int rtc_render_adaptive(rtc_scene* s, uint32_t seed, float tolerance, uint32_t m
  *      run.sh takes the list from RTC_DEVICES ("0,1,2,3" or "0-7"). */
 int rtc_render_u8_multi(rtc_scene* s, const int* devices, int ndev, uint32_t seed, uint8_t* rgb_host, float* sum_host);
 int rtc_render_ppm_multi(rtc_scene* s, const int* devices, int ndev, uint32_t seed, const char* out_path);
+/* ---- rtc_render_adaptive on several devices of this process.  Tile t (row-major over the frame, the tiles of
+ *      rtc_render_adaptive) belongs to devices[t % ndev]; each device runs the passes of rtc_render_adaptive on its own
+ *      tiles, and devices[0] resolves every pixel from its owner's half sums over peer access.  A tile's decisions read
+ *      only its own half sums and the samples are those of rtc_render_accumulate, so the result is rtc_render_adaptive's
+ *      up to float summation order.  A device may be listed more than once; one listed beyond the tile count renders
+ *      nothing.  hw1 / hw2 render their one frame on devices[0], as rtc_render_adaptive does.  Arguments and outputs are
+ *      those of rtc_render_adaptive; devices must list 1 to 16 indices in 0..63 (else RTC_ERR_ARG, checked before any
+ *      device is touched).
+ * stats: passes (the most of any device), paths (summed over the devices), tiles (of the frame), tiles stopped below
+ *      max_samples (summed over the devices). */
+int rtc_render_adaptive_multi(rtc_scene* s, const int* devices, int ndev, uint32_t seed, float tolerance, uint32_t min_samples,
+                              uint32_t max_samples, uint8_t* rgb_host, float* halves_host, uint32_t* spp_host, uint64_t stats[4]);
 /* ---- frames in flight: what run.sh does with a parsed scene (flattened scene host -> HBM, render, resolve, 8-bit
  *      image HBM -> host), queued without host synchronisation.  rtc_frame_begin uploads into the arena that is not
  *      being read (rtc_scene_upload_async: on a copy stream, under the kernels of the frame before), renders with the

@@ -73,6 +73,8 @@ _SIGNATURES = {
     "rtc_render_sum": (C.c_int, [C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, _f32]),
     "rtc_render_ppm": (C.c_int, [C.c_void_p, C.c_uint32, C.c_char_p]),
     "rtc_render_adaptive": (C.c_int, [C.c_void_p, C.c_uint32, C.c_float, C.c_uint32, C.c_uint32, _u8, _f32, _u32, _u64]),
+    "rtc_render_adaptive_multi": (C.c_int, [C.c_void_p, _i32, C.c_int, C.c_uint32, C.c_float, C.c_uint32, C.c_uint32, _u8, _f32,
+                                            _u32, _u64]),
     "rtc_set_batch_paths": (C.c_int, [C.c_void_p, C.c_uint64]),
     "rtc_set_profiling": (C.c_int, [C.c_void_p, C.c_int, C.c_int]),
     "rtc_render_profile": (C.c_int, [C.c_void_p, C.c_void_p, np.ctypeslib.ndpointer(dtype=np.float64, flags="C_CONTIGUOUS"), _u64, C.c_int]),
@@ -308,6 +310,19 @@ class Scene:
         st = np.zeros(4, np.uint64)
         _check(self.lib, self.lib.rtc_render_adaptive(self.h, seed, float(tolerance), min_samples, max_samples,
                                                       img, halves, spp, st))
+        return img, halves, spp, dict(zip(["passes", "paths", "tiles", "tiles_stopped"], [int(v) for v in st]))
+
+    def RenderAdaptiveMulti(self, devices, tolerance, min_samples=16, max_samples=0, seed=0):
+        """RenderAdaptive on several CUDA devices of this process (rtc_render_adaptive_multi): tile t is rendered by
+        devices[t % len(devices)], and devices[0] gathers the image over peer access.  Returns what RenderAdaptive
+        returns; stats["passes"] is the most passes of any device."""
+        dv = np.asarray(devices, np.int32)
+        img = np.zeros((self.height, self.width, 3), np.uint8)
+        halves = np.zeros((self.height, self.width, 2, 3), np.float32)
+        spp = np.zeros((self.height, self.width), np.uint32)
+        st = np.zeros(4, np.uint64)
+        _check(self.lib, self.lib.rtc_render_adaptive_multi(self.h, dv, len(dv), seed, float(tolerance), min_samples,
+                                                            max_samples, img, halves, spp, st))
         return img, halves, spp, dict(zip(["passes", "paths", "tiles", "tiles_stopped"], [int(v) for v in st]))
 
     def RenderMulti(self, devices, seed=0, want_sum=False):

@@ -3,12 +3,15 @@
 // on a scene without a device fails with RTC_ERR_NO_DEVICE.
 #include <cuda_runtime.h>
 
+#include <algorithm>
+#include <array>
 #include <cmath>
 #include <chrono>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
 #include <fstream>
+#include <functional>
 #include <map>
 #include <memory>
 #include <sstream>
@@ -1059,6 +1062,84 @@ int rtc_render_ppm(rtc_scene* s, uint32_t seed, const char* out_path) {
 // once -- then k_adaptive_tiles measures the tiles' error from the two halves and lists the tiles (and their pixels) that
 // go on to target = min(2 target, max).  The length of the next pixel list is the one read back per pass.
 static_assert(kAdaptiveTile == RTC_ADAPTIVE_TILE, "rt_kernels.h and rtc_b200.h disagree on the tile size");
+namespace {
+uint32_t adaptive_tiles(uint32_t width, uint32_t height) {
+    return ((width + kAdaptiveTile - 1) / kAdaptiveTile) * ((height + kAdaptiveTile - 1) / kAdaptiveTile);
+}
+// The pass loop of an adaptive render of the tiles shard, shard + nshards, ... of the frame on context `c` (its device
+// current), on stream `user`: it leaves the half sums of those tiles' pixels in c->adaptive.half and their sample counts
+// in c->adaptive.tile_n, and adds its passes, paths and tiles stopped to st[0], st[1] and st[3].  A shard without a tile
+// does nothing.
+int adaptive_passes(rtc_scene* c, cudaStream_t user, uint32_t shard, uint32_t nshards, uint32_t seed, float tolerance,
+                    uint32_t min_samples, uint32_t smax, uint64_t st[4]) {
+    const uint32_t width = c->host.cam.width, height = c->host.cam.height;
+    const uint32_t npix = width * height, ntiles = adaptive_tiles(width, height);
+    if (shard >= ntiles) return RTC_OK;
+    const uint32_t shard_tiles = (ntiles - shard + nshards - 1) / nshards;
+    // the pixels of the shard's tiles: whole tiles, less what the partial tiles of the last column and row lack (a loop
+    // over the edge tiles, not over all of them: this runs on the host before every render)
+    constexpr uint32_t T = kAdaptiveTile;
+    const uint32_t tiles_x = (width + T - 1) / T, tiles_y = ntiles / tiles_x;
+    const uint32_t wl = width - (tiles_x - 1) * T, hl = height - (tiles_y - 1) * T;   // size of the last column / row
+    uint32_t shard_pix = T * T * shard_tiles;
+    if (wl < T)
+        for (uint32_t ty = 0; ty < tiles_y; ++ty)
+            if ((ty * tiles_x + tiles_x - 1) % nshards == shard) shard_pix -= (T - wl) * T;
+    if (hl < T)
+        for (uint32_t tx = 0; tx < tiles_x; ++tx)
+            if (((tiles_y - 1) * tiles_x + tx) % nshards == shard) shard_pix -= (T - hl) * (tx + 1 < tiles_x ? T : wl);
+    int rc;
+    rtc_scene::Adaptive& ad = c->adaptive;
+    for (auto& b : ad.half) CU(b.ensure(npix));
+    for (auto& b : ad.tiles) CU(b.ensure(ntiles));
+    for (auto& b : ad.pixels) CU(b.ensure(npix));
+    CU(ad.tile_n.ensure(ntiles));
+    CU(ad.counts.ensure(4));
+    CU(ad.counts_host.ensure(2));
+    LaunchCtx lc{user, c->sms};
+    for (auto& b : ad.half) CU(cudaMemsetAsync(b.p, 0, npix * sizeof(float4), user));
+    CU(cudaMemsetAsync(ad.counts.p, 0, 4 * sizeof(uint32_t), user));
+    DevScene S;
+    if ((rc = arena_begin(c, user, &S))) return rc;
+    // every tile of the shard is active with n = 0; lists of pass 0 in set 0
+    launch_adaptive_tiles(lc, nullptr, nullptr, width, height, nullptr, shard_tiles, 0, 0.f, 0.f, tolerance, ADAPTIVE_FIRST, ad.tile_n.p,
+                          ad.tiles[0].p, ad.pixels[0].p, ad.counts.p, shard, nshards);
+    c->launches++;
+    uint32_t active_tiles = shard_tiles, active_pix = shard_pix, n = 0, target = min_samples < smax ? min_samples : smax;
+    int cur = 0;
+    for (;;) {
+        ++st[0];
+        if ((rc = fork_lanes(c, user))) return rc;
+        unsigned used = 0;
+        for (uint32_t h = 0; h < 2; ++h) {   // h = 0: the even samples of [n, target) into half 0, h = 1: the odd ones
+            const uint32_t first = n + ((n ^ h) & 1u);
+            if (first >= target) continue;
+            const uint64_t total = (uint64_t)((target - first + 1) / 2) * active_pix;
+            if ((rc = render_paths(c, S, seed, PathMap{ad.pixels[cur].p, active_pix, first}, total, ad.half[h].p, &used))) return rc;
+            st[1] += total;
+        }
+        if ((rc = join_lanes(c, used, user))) return rc;
+        n = target;
+        const bool last = n == smax;
+        const int nxt = cur ^ 1;
+        if (!last) CU(cudaMemsetAsync(ad.counts.p + 2 * nxt, 0, 2 * sizeof(uint32_t), user));
+        launch_adaptive_tiles(lc, ad.half[0].p, ad.half[1].p, width, height, ad.tiles[cur].p, active_tiles, n, 1.f / (float)((n + 1) / 2),
+                              1.f / (float)(n / 2), tolerance, last ? ADAPTIVE_LAST : ADAPTIVE_DECIDE, ad.tile_n.p, ad.tiles[nxt].p,
+                              ad.pixels[nxt].p, ad.counts.p + 2 * nxt, 0, 1);
+        c->launches++;
+        if (last) break;
+        CU(cudaMemcpyAsync(ad.counts_host.p, ad.counts.p + 2 * nxt, 2 * sizeof(uint32_t), cudaMemcpyDeviceToHost, user));
+        CU(cudaStreamSynchronize(user));
+        st[3] += active_tiles - ad.counts_host.p[0];
+        active_tiles = ad.counts_host.p[0];
+        active_pix = ad.counts_host.p[1];
+        if (active_tiles == 0) break;
+        cur = nxt;
+        target = (uint64_t)2 * target < smax ? 2 * target : smax;
+    }
+    return arena_end(c, user);
+}
+}  // namespace
 int rtc_render_adaptive(rtc_scene* s, uint32_t seed, float tolerance, uint32_t min_samples, uint32_t max_samples,
                         uint8_t* rgb_host, float* halves_host, uint32_t* spp_host, uint64_t stats[4]) {
     if (!s) return fail(RTC_ERR_ARG, "null scene");
@@ -1068,7 +1149,7 @@ int rtc_render_adaptive(rtc_scene* s, uint32_t seed, float tolerance, uint32_t m
     if (rc) return rc;
     const uint32_t width = s->host.cam.width, height = s->host.cam.height;
     const uint32_t npix = width * height;
-    const uint32_t ntiles = ((width + kAdaptiveTile - 1) / kAdaptiveTile) * ((height + kAdaptiveTile - 1) / kAdaptiveTile);
+    const uint32_t ntiles = adaptive_tiles(width, height);
     uint64_t st[4] = {0, 0, 0, 0};   // passes, paths, tiles, tiles stopped below the maximum
     if (stats) std::memcpy(stats, st, sizeof st);
     if (npix == 0) return RTC_OK;
@@ -1092,62 +1173,15 @@ int rtc_render_adaptive(rtc_scene* s, uint32_t seed, float tolerance, uint32_t m
     }
     const uint32_t smax = max_samples ? max_samples : s->host.samples;
     if (smax == 0) return fail(RTC_ERR_ARG, "scene has SAMPLES 0");
-    rtc_scene::Adaptive& ad = s->adaptive;
-    for (auto& b : ad.half) CU(b.ensure(npix));
-    for (auto& b : ad.tiles) CU(b.ensure(ntiles));
-    for (auto& b : ad.pixels) CU(b.ensure(npix));
-    CU(ad.tile_n.ensure(ntiles));
-    CU(ad.counts.ensure(4));
-    CU(ad.counts_host.ensure(2));
     cudaStream_t user = nullptr;
-    LaunchCtx c{user, s->sms};
-    for (auto& b : ad.half) CU(cudaMemsetAsync(b.p, 0, npix * sizeof(float4), user));
-    CU(cudaMemsetAsync(ad.counts.p, 0, 4 * sizeof(uint32_t), user));
-    DevScene S;
-    if ((rc = arena_begin(s, user, &S))) return rc;
-    // every tile is active with n = 0; lists of pass 0 in set 0
-    launch_adaptive_tiles(c, nullptr, nullptr, width, height, nullptr, ntiles, 0, 0.f, 0.f, tolerance, ADAPTIVE_FIRST, ad.tile_n.p,
-                          ad.tiles[0].p, ad.pixels[0].p, ad.counts.p);
-    s->launches++;
-    uint32_t active_tiles = ntiles, active_pix = npix, n = 0, target = min_samples < smax ? min_samples : smax;
-    int cur = 0;
     st[2] = ntiles;
-    for (;;) {
-        ++st[0];
-        if ((rc = fork_lanes(s, user))) return rc;
-        unsigned used = 0;
-        for (uint32_t h = 0; h < 2; ++h) {   // h = 0: the even samples of [n, target) into half 0, h = 1: the odd ones
-            const uint32_t first = n + ((n ^ h) & 1u);
-            if (first >= target) continue;
-            const uint64_t total = (uint64_t)((target - first + 1) / 2) * active_pix;
-            if ((rc = render_paths(s, S, seed, PathMap{ad.pixels[cur].p, active_pix, first}, total, ad.half[h].p, &used))) return rc;
-            st[1] += total;
-        }
-        if ((rc = join_lanes(s, used, user))) return rc;
-        n = target;
-        const bool last = n == smax;
-        const int nxt = cur ^ 1;
-        if (!last) CU(cudaMemsetAsync(ad.counts.p + 2 * nxt, 0, 2 * sizeof(uint32_t), user));
-        launch_adaptive_tiles(c, ad.half[0].p, ad.half[1].p, width, height, ad.tiles[cur].p, active_tiles, n, 1.f / (float)((n + 1) / 2),
-                              1.f / (float)(n / 2), tolerance, last ? ADAPTIVE_LAST : ADAPTIVE_DECIDE, ad.tile_n.p, ad.tiles[nxt].p,
-                              ad.pixels[nxt].p, ad.counts.p + 2 * nxt);
-        s->launches++;
-        if (last) break;
-        CU(cudaMemcpyAsync(ad.counts_host.p, ad.counts.p + 2 * nxt, 2 * sizeof(uint32_t), cudaMemcpyDeviceToHost, user));
-        CU(cudaStreamSynchronize(user));
-        st[3] += active_tiles - ad.counts_host.p[0];
-        active_tiles = ad.counts_host.p[0];
-        active_pix = ad.counts_host.p[1];
-        if (active_tiles == 0) break;
-        cur = nxt;
-        target = (uint64_t)2 * target < smax ? 2 * target : smax;
-    }
+    if ((rc = adaptive_passes(s, user, 0, 1, seed, tolerance, min_samples, smax, st))) return rc;
+    rtc_scene::Adaptive& ad = s->adaptive;
     CU(ad.halves.ensure(halves_host ? 6 * (size_t)npix : 0));
     CU(ad.spp.ensure(spp_host ? npix : 0));
-    launch_resolve_adaptive(c, ad.half[0].p, ad.half[1].p, ad.tile_n.p, width, npix, s->rgb.p, halves_host ? ad.halves.p : nullptr,
-                            spp_host ? ad.spp.p : nullptr);
+    launch_resolve_adaptive(LaunchCtx{user, s->sms}, ad.half[0].p, ad.half[1].p, ad.tile_n.p, width, npix, s->rgb.p,
+                            halves_host ? ad.halves.p : nullptr, spp_host ? ad.spp.p : nullptr);
     s->launches++;
-    if ((rc = arena_end(s, user))) return rc;
     CU(cudaGetLastError());
     if (rgb_host) CU(cudaMemcpy(rgb_host, s->rgb.p, nvalues, cudaMemcpyDeviceToHost));
     if (halves_host) CU(cudaMemcpy(halves_host, ad.halves.p, 6 * (size_t)npix * sizeof(float), cudaMemcpyDeviceToHost));
@@ -1256,6 +1290,54 @@ rtc_scene* replica_on(rtc_scene* s, int device, int ordinal) {
     s->replicas.push_back(std::move(r));
     return s->replicas.back().get();
 }
+// issue(i) for i in [0, n): i >= 1 on host threads of their own, i = 0 on the caller's; the first failure in list order
+// is returned, with its message
+int fan_out(int n, const std::function<int(int)>& issue) {
+    std::vector<int> rcs((size_t)n, RTC_OK);
+    std::vector<std::string> errs((size_t)n);
+    std::vector<std::thread> workers;
+    for (int i = 1; i < n; ++i)
+        workers.emplace_back([&, i] { rcs[i] = issue(i); if (rcs[i]) errs[i] = g_error; });   // g_error is per thread
+    rcs[0] = issue(0);
+    for (std::thread& w : workers) w.join();
+    for (int i = 0; i < n; ++i)
+        if (rcs[i]) return i == 0 ? rcs[0] : fail(rcs[i], errs[i]);
+    return RTC_OK;
+}
+// Whether device `head` (current) reads the memory of device `dev` in place: the same device, or peer access, which
+// this enables.  When it cannot, the caller copies what it needs over with stage_peer.
+int peer_mapped(int head, int dev, bool* mapped) {
+    *mapped = head == dev;
+    if (*mapped) return RTC_OK;
+    int can = 0;
+    CU(cudaDeviceCanAccessPeer(&can, head, dev));
+    if (can) {
+        cudaError_t e = cudaDeviceEnablePeerAccess(dev, 0);
+        if (e == cudaSuccess || e == cudaErrorPeerAccessAlreadyEnabled) { cudaGetLastError(); *mapped = true; }
+        else cudaGetLastError();
+    }
+    return RTC_OK;
+}
+// a copy on device `head` (current) of `bytes` at `src` on device `dev`, queued on `st` and held by `staged`; null when
+// it cannot be made (the message in rtc_last_error)
+void* stage_peer(int head, int dev, const void* src, size_t bytes, cudaStream_t st, std::vector<DevBuf<unsigned char>>& staged) {
+    staged.emplace_back();
+    cudaError_t e = staged.back().ensure(bytes);
+    if (e == cudaSuccess) e = cudaMemcpyPeerAsync(staged.back().p, head, src, dev, bytes, st);
+    if (e != cudaSuccess) { fail(RTC_ERR_CUDA, std::string("staging a peer copy: ") + cudaGetErrorString(e)); return nullptr; }
+    return staged.back().p;
+}
+// the context of every entry of `devices`: this scene for the first use of its own device, replicas for the others
+int device_contexts(rtc_scene* s, const int* devices, int ndev, std::vector<rtc_scene*>& ctx) {
+    ctx.assign((size_t)ndev, nullptr);
+    std::vector<int> uses(64, 0);
+    for (int i = 0; i < ndev; ++i) {
+        if (devices[i] < 0 || devices[i] >= 64) return fail(RTC_ERR_ARG, "bad device index");
+        ctx[i] = replica_on(s, devices[i], uses[devices[i]]++);
+        if (!ctx[i]) return RTC_ERR_CUDA;
+    }
+    return RTC_OK;
+}
 }  // namespace
 int rtc_render_u8_multi(rtc_scene* s, const int* devices, int ndev, uint32_t seed, uint8_t* rgb_host, float* sum_host) {
     int rc = need_device(s);
@@ -1266,13 +1348,8 @@ int rtc_render_u8_multi(rtc_scene* s, const int* devices, int ndev, uint32_t see
     const size_t nvalues = 3 * (size_t)s->host.cam.width * s->host.cam.height;
     if (nvalues == 0) return RTC_OK;
     // the first listed device reduces: make it this scene's device or a replica there
-    std::vector<rtc_scene*> ctx((size_t)ndev, nullptr);
-    std::vector<int> uses(64, 0);
-    for (int i = 0; i < ndev; ++i) {
-        if (devices[i] < 0 || devices[i] >= 64) return fail(RTC_ERR_ARG, "bad device index");
-        ctx[i] = replica_on(s, devices[i], uses[devices[i]]++);
-        if (!ctx[i]) return RTC_ERR_CUDA;
-    }
+    std::vector<rtc_scene*> ctx;
+    if ((rc = device_contexts(s, devices, ndev, ctx))) return rc;
     PeerAccums A;
     std::memset(&A, 0, sizeof A);
     A.n = ndev;
@@ -1292,40 +1369,20 @@ int rtc_render_u8_multi(rtc_scene* s, const int* devices, int ndev, uint32_t see
         CU(cudaEventRecord(c->multi_done, c->multi_stream));
         return RTC_OK;
     };
-    {
-        std::vector<int> rcs((size_t)ndev, RTC_OK);
-        std::vector<std::string> errs((size_t)ndev);
-        std::vector<std::thread> workers;
-        for (int i = 1; i < ndev; ++i)
-            workers.emplace_back([&, i] { rcs[i] = issue(i); if (rcs[i]) errs[i] = g_error; });   // g_error is per thread
-        rcs[0] = issue(0);
-        for (std::thread& w : workers) w.join();
-        for (int i = 0; i < ndev; ++i) {
-            if (rcs[i]) return i == 0 ? rcs[0] : fail(rcs[i], errs[i]);
-            A.p[i] = ctx[i]->accum.p;
-        }
-    }
+    if ((rc = fan_out(ndev, issue))) return rc;
+    for (int i = 0; i < ndev; ++i) A.p[i] = ctx[i]->accum.p;
     // the head device reads the others' buffers in place (peer access), or copies them over when it cannot
     CU(cudaSetDevice(head->device));
-    std::vector<DevBuf<float>> staged;
+    std::vector<DevBuf<unsigned char>> staged;
     for (int i = 1; i < ndev; ++i) {
         rtc_scene* c = ctx[i];
         CU(cudaStreamWaitEvent(head->multi_stream, c->multi_done, 0));
-        if (c->device == head->device) continue;
-        int can = 0;
-        CU(cudaDeviceCanAccessPeer(&can, head->device, c->device));
-        bool mapped = false;
-        if (can) {
-            cudaError_t e = cudaDeviceEnablePeerAccess(c->device, 0);
-            if (e == cudaSuccess || e == cudaErrorPeerAccessAlreadyEnabled) { cudaGetLastError(); mapped = true; }
-            else cudaGetLastError();
-        }
-        if (!mapped) {
-            staged.emplace_back();
-            CU(staged.back().ensure(nvalues));
-            CU(cudaMemcpyPeerAsync(staged.back().p, head->device, c->accum.p, c->device, nvalues * sizeof(float), head->multi_stream));
-            A.p[i] = staged.back().p;
-        }
+        bool mapped;
+        if ((rc = peer_mapped(head->device, c->device, &mapped))) return rc;
+        if (mapped) continue;
+        void* p = stage_peer(head->device, c->device, A.p[i], nvalues * sizeof(float), head->multi_stream, staged);
+        if (!p) return RTC_ERR_CUDA;
+        A.p[i] = (const float*)p;
     }
     CU(head->rgb.ensure(nvalues));
     float* sum_dev = nullptr;
@@ -1350,6 +1407,102 @@ int rtc_render_ppm_multi(rtc_scene* s, const int* devices, int ndev, uint32_t se
     std::vector<uint8_t> img(3 * (size_t)s->host.cam.width * s->host.cam.height);
     int rc = rtc_render_u8_multi(s, devices, ndev, seed, img.data(), nullptr);
     return rc ? rc : write_ppm(out_path, s->host.cam.width, s->host.cam.height, img);
+}
+
+// Adaptive sampling on several devices: tile t of the frame belongs to devices[t % ndev], and every device runs the
+// pass loop of rtc_render_adaptive on its own tiles, on its own stream and host thread.  A tile's decisions read only its
+// own half sums, so the devices do not talk to each other until devices[0] resolves every pixel from its owner's
+// half sums and tile counts (k_resolve_adaptive_peers).
+int rtc_render_adaptive_multi(rtc_scene* s, const int* devices, int ndev, uint32_t seed, float tolerance, uint32_t min_samples,
+                              uint32_t max_samples, uint8_t* rgb_host, float* halves_host, uint32_t* spp_host, uint64_t stats[4]) {
+    if (!s) return fail(RTC_ERR_ARG, "null scene");
+    if (!std::isfinite(tolerance) || tolerance < 0.f) return fail(RTC_ERR_ARG, "tolerance must be finite and >= 0");
+    if (min_samples < 2) return fail(RTC_ERR_ARG, "min_samples must be at least 2");
+    if (!devices || ndev < 1 || ndev > kMaxPeers) return fail(RTC_ERR_ARG, "devices must list 1 to 16 entries");
+    for (int i = 0; i < ndev; ++i)
+        if (devices[i] < 0 || devices[i] >= 64) return fail(RTC_ERR_ARG, "bad device index");
+    int rc = need_device(s);
+    if (rc) return rc;
+    const uint32_t width = s->host.cam.width, height = s->host.cam.height;
+    const uint32_t npix = width * height, ntiles = adaptive_tiles(width, height);
+    uint64_t st[4] = {0, 0, 0, 0};   // passes (the most of any device), paths, tiles, tiles stopped below the maximum
+    if (stats) std::memcpy(stats, st, sizeof st);
+    if (npix == 0) return RTC_OK;
+    const size_t nvalues = 3 * (size_t)npix;
+    if (s->host.dialect <= DIALECT_HW2) {
+        // one deterministic frame, not split: rtc_render_adaptive on the first listed device
+        rtc_scene* head = replica_on(s, devices[0], 0);
+        if (!head) return RTC_ERR_CUDA;
+        if ((rc = rtc_render_adaptive(head, seed, tolerance, min_samples, max_samples, rgb_host, halves_host, spp_host, stats)))
+            return rc;
+        CU(cudaSetDevice(s->device));
+        return RTC_OK;
+    }
+    const uint32_t smax = max_samples ? max_samples : s->host.samples;
+    if (smax == 0) return fail(RTC_ERR_ARG, "scene has SAMPLES 0");
+    std::vector<rtc_scene*> ctx;
+    if ((rc = device_contexts(s, devices, ndev, ctx))) return rc;
+    rtc_scene* head = ctx[0];
+    std::vector<std::array<uint64_t, 4>> dev_st((size_t)ndev, std::array<uint64_t, 4>{0, 0, 0, 0});
+    auto issue = [&](int i) -> int {
+        rtc_scene* c = ctx[i];
+        CU(cudaSetDevice(c->device));
+        CU(c->multi_stream.ensure());
+        CU(c->multi_done.ensure());
+        int r = adaptive_passes(c, c->multi_stream, (uint32_t)i, (uint32_t)ndev, seed, tolerance, min_samples, smax, dev_st[i].data());
+        if (r) return r;
+        CU(cudaEventRecord(c->multi_done, c->multi_stream));
+        return RTC_OK;
+    };
+    if ((rc = fan_out(ndev, issue))) return rc;
+    // the head device reads the owners' half sums and tile counts in place (peer access), or copies them over
+    CU(cudaSetDevice(head->device));
+    PeerHalves P;
+    std::memset(&P, 0, sizeof P);
+    P.n = ndev;
+    const int owners = (uint32_t)ndev < ntiles ? ndev : (int)ntiles;   // the others have no tile
+    std::vector<DevBuf<unsigned char>> staged;
+    for (int i = 0; i < owners; ++i) {
+        rtc_scene* c = ctx[i];
+        P.a[i] = c->adaptive.half[0].p;
+        P.b[i] = c->adaptive.half[1].p;
+        P.tile_n[i] = c->adaptive.tile_n.p;
+        if (i == 0) continue;
+        CU(cudaStreamWaitEvent(head->multi_stream, c->multi_done, 0));
+        bool mapped;
+        if ((rc = peer_mapped(head->device, c->device, &mapped))) return rc;
+        if (mapped) continue;
+        void* a = stage_peer(head->device, c->device, P.a[i], npix * sizeof(float4), head->multi_stream, staged);
+        void* b = a ? stage_peer(head->device, c->device, P.b[i], npix * sizeof(float4), head->multi_stream, staged) : nullptr;
+        void* n = b ? stage_peer(head->device, c->device, P.tile_n[i], ntiles * sizeof(uint32_t), head->multi_stream, staged) : nullptr;
+        if (!n) return RTC_ERR_CUDA;
+        P.a[i] = (const float4*)a;
+        P.b[i] = (const float4*)b;
+        P.tile_n[i] = (const uint32_t*)n;
+    }
+    rtc_scene::Adaptive& ad = head->adaptive;
+    CU(head->rgb.ensure(nvalues));
+    CU(ad.halves.ensure(halves_host ? 6 * (size_t)npix : 0));
+    CU(ad.spp.ensure(spp_host ? npix : 0));
+    launch_resolve_adaptive_peers(LaunchCtx{head->multi_stream, head->sms}, P, width, npix, head->rgb.p,
+                                  halves_host ? ad.halves.p : nullptr, spp_host ? ad.spp.p : nullptr);
+    head->launches++;
+    CU(cudaGetLastError());
+    if (rgb_host) CU(cudaMemcpyAsync(rgb_host, head->rgb.p, nvalues, cudaMemcpyDeviceToHost, head->multi_stream));
+    if (halves_host)
+        CU(cudaMemcpyAsync(halves_host, ad.halves.p, 6 * (size_t)npix * sizeof(float), cudaMemcpyDeviceToHost, head->multi_stream));
+    if (spp_host) CU(cudaMemcpyAsync(spp_host, ad.spp.p, (size_t)npix * sizeof(uint32_t), cudaMemcpyDeviceToHost, head->multi_stream));
+    CU(cudaStreamSynchronize(head->multi_stream));
+    staged.clear();   // while the head device is current
+    CU(cudaSetDevice(s->device));
+    st[2] = ntiles;
+    for (const auto& d : dev_st) {
+        st[0] = std::max(st[0], d[0]);
+        st[1] += d[1];
+        st[3] += d[3];
+    }
+    if (stats) std::memcpy(stats, st, sizeof st);
+    return RTC_OK;
 }
 
 int rtc_set_profiling(rtc_scene* s, int kernel_events, int count_visits) {

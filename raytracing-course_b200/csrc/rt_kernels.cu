@@ -648,19 +648,22 @@ RT_D float half_error(float4 A, float4 B, float inv_a, float inv_b) {
     return __fdiv_rn(__fadd_rn(__fadd_rn(er, eg), eb), 3.f);
 }
 // One warp per active tile; pixel k of the tile (row-major within the tile) is on lane k % 32, so a lane holds
-// pixels (x, y) and (x, y + 4).  ADAPTIVE_FIRST lists every tile of the frame (tiles_in unused), ADAPTIVE_DECIDE computes
+// pixels (x, y) and (x, y + 4).  ADAPTIVE_FIRST lists every tile of a shard (tiles_in unused), ADAPTIVE_DECIDE computes
 // the tile error E from the half sums (n samples: inv_a = 1 / ceil(n/2), inv_b = 1 / floor(n/2)) and keeps the tile
 // while !(E < tau), ADAPTIVE_LAST keeps none.  Every visited tile records n; a kept tile is appended to tiles_out and
 // its in-image pixels, row by row, to pixels_out (counts_out[0] tiles, counts_out[1] pixels; one atomic per warp).
+// ADAPTIVE_FIRST lists the ntiles tiles of one shard of the frame: the w-th is tile shard + w nshards (the whole frame
+// is shard 0 of 1; a multi-device render gives device d of D the shard (d, D)).
 __global__ void __launch_bounds__(128) k_adaptive_tiles(const float4* A, const float4* B, uint32_t width, uint32_t height,
                                                          const uint32_t* tiles_in, uint32_t ntiles, uint32_t n, float inv_a,
                                                          float inv_b, float tau, int mode, uint32_t* tile_n, uint32_t* tiles_out,
-                                                         uint32_t* pixels_out, uint32_t* counts_out) {
+                                                         uint32_t* pixels_out, uint32_t* counts_out, uint32_t shard,
+                                                         uint32_t nshards) {
     const uint32_t lane = threadIdx.x & 31;
     const uint32_t tiles_x = (width + kAdaptiveTile - 1) / kAdaptiveTile;
     const uint32_t warps = (gridDim.x * blockDim.x) >> 5;
     for (uint32_t w = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; w < ntiles; w += warps) {   // warp-uniform
-        const uint32_t tile = mode == ADAPTIVE_FIRST ? w : tiles_in[w];
+        const uint32_t tile = mode == ADAPTIVE_FIRST ? shard + w * nshards : tiles_in[w];
         const uint32_t x = (tile % tiles_x) * kAdaptiveTile + (lane & 7u), y0 = (tile / tiles_x) * kAdaptiveTile + (lane >> 3);
         const bool v0 = x < width && y0 < height, v1 = x < width && y0 + 4u < height;
         const uint32_t p0 = y0 * width + x, p1 = p0 + 4u * width;
@@ -690,24 +693,38 @@ __global__ void __launch_bounds__(128) k_adaptive_tiles(const float4* A, const f
         }
     }
 }
-// The image of an adaptive render: pixel i took n = tile_n[its tile] samples, A / B hold its even / odd sums;
-// out = to_u8(aces(1/n * (A + B))) (k_resolve's expression); optionally halves (A.rgb, B.rgb per pixel) and spp (n).
+// The tile (row-major over the frame) of pixel i
+RT_D uint32_t tile_of(uint32_t i, uint32_t width, uint32_t tiles_x) {
+    return (i / width / kAdaptiveTile) * tiles_x + (i % width) / kAdaptiveTile;
+}
+// Pixel i of an adaptive image: it took n samples, a / b are its even / odd sums; out = to_u8(aces(1/n * (a + b)))
+// (k_resolve's expression); optionally halves (a.rgb, b.rgb per pixel) and spp (n).
+RT_D void resolve_adaptive_pixel(uint32_t i, float4 a, float4 b, uint32_t n, uint8_t* out, float* halves, uint32_t* spp) {
+    const float inv = __fdiv_rn(1.f, (float)n);
+    out[3 * (size_t)i + 0] = to_u8(aces(__fmul_rn(inv, __fadd_rn(a.x, b.x))));
+    out[3 * (size_t)i + 1] = to_u8(aces(__fmul_rn(inv, __fadd_rn(a.y, b.y))));
+    out[3 * (size_t)i + 2] = to_u8(aces(__fmul_rn(inv, __fadd_rn(a.z, b.z))));
+    if (halves) {
+        float* h = halves + 6 * (size_t)i;
+        h[0] = a.x; h[1] = a.y; h[2] = a.z; h[3] = b.x; h[4] = b.y; h[5] = b.z;
+    }
+    if (spp) spp[i] = n;
+}
+// The image of an adaptive render: pixel i took tile_n[its tile] samples, A / B hold its even / odd sums
 __global__ void __launch_bounds__(256) k_resolve_adaptive(const float4* A, const float4* B, const uint32_t* tile_n, uint32_t width,
                                                            uint32_t npix, uint8_t* out, float* halves, uint32_t* spp) {
     const uint32_t tiles_x = (width + kAdaptiveTile - 1) / kAdaptiveTile;
+    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < npix; i += gridDim.x * blockDim.x)
+        resolve_adaptive_pixel(i, A[i], B[i], tile_n[tile_of(i, width, tiles_x)], out, halves, spp);
+}
+// The same for a multi-device adaptive render, on the first device: tile t was rendered by device t % P.n, whose
+// half sums and tile counts are read where they lie (peer pointers over NVLink, or copies on this device)
+__global__ void __launch_bounds__(256) k_resolve_adaptive_peers(PeerHalves P, uint32_t width, uint32_t npix, uint8_t* out,
+                                                                 float* halves, uint32_t* spp) {
+    const uint32_t tiles_x = (width + kAdaptiveTile - 1) / kAdaptiveTile;
     for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < npix; i += gridDim.x * blockDim.x) {
-        const uint32_t x = i % width, y = i / width;
-        const uint32_t n = tile_n[(y / kAdaptiveTile) * tiles_x + x / kAdaptiveTile];
-        const float4 a = A[i], b = B[i];
-        const float inv = __fdiv_rn(1.f, (float)n);
-        out[3 * (size_t)i + 0] = to_u8(aces(__fmul_rn(inv, __fadd_rn(a.x, b.x))));
-        out[3 * (size_t)i + 1] = to_u8(aces(__fmul_rn(inv, __fadd_rn(a.y, b.y))));
-        out[3 * (size_t)i + 2] = to_u8(aces(__fmul_rn(inv, __fadd_rn(a.z, b.z))));
-        if (halves) {
-            float* h = halves + 6 * (size_t)i;
-            h[0] = a.x; h[1] = a.y; h[2] = a.z; h[3] = b.x; h[4] = b.y; h[5] = b.z;
-        }
-        if (spp) spp[i] = n;
+        const uint32_t t = tile_of(i, width, tiles_x), d = t % (uint32_t)P.n;
+        resolve_adaptive_pixel(i, P.a[d][i], P.b[d][i], P.tile_n[d][t], out, halves, spp);
     }
 }
 
@@ -816,15 +833,20 @@ void launch_generate_list(const LaunchCtx& c, const DevScene& S, PathSoA P, HitS
 }
 void launch_adaptive_tiles(const LaunchCtx& c, const float4* A, const float4* B, uint32_t width, uint32_t height,
                            const uint32_t* tiles_in, uint32_t ntiles, uint32_t n, float inv_a, float inv_b, float tau, int mode,
-                           uint32_t* tile_n, uint32_t* tiles_out, uint32_t* pixels_out, uint32_t* counts_out) {
+                           uint32_t* tile_n, uint32_t* tiles_out, uint32_t* pixels_out, uint32_t* counts_out, uint32_t shard,
+                           uint32_t nshards) {
     if (ntiles == 0) return;
     k_adaptive_tiles<<<grid_for((uint64_t)ntiles * 32, 128, c.sms, 16), 128, 0, c.stream>>>(A, B, width, height, tiles_in, ntiles, n, inv_a,
                                                                                           inv_b, tau, mode, tile_n, tiles_out,
-                                                                                          pixels_out, counts_out);
+                                                                                          pixels_out, counts_out, shard, nshards);
 }
 void launch_resolve_adaptive(const LaunchCtx& c, const float4* A, const float4* B, const uint32_t* tile_n, uint32_t width, uint32_t npix,
                              uint8_t* out, float* halves, uint32_t* spp) {
     k_resolve_adaptive<<<grid_for(npix, 256, c.sms, 8), 256, 0, c.stream>>>(A, B, tile_n, width, npix, out, halves, spp);
+}
+void launch_resolve_adaptive_peers(const LaunchCtx& c, const PeerHalves& P, uint32_t width, uint32_t npix, uint8_t* out, float* halves,
+                                   uint32_t* spp) {
+    k_resolve_adaptive_peers<<<grid_for(npix, 256, c.sms, 8), 256, 0, c.stream>>>(P, width, npix, out, halves, spp);
 }
 void launch_pre(const LaunchCtx& c, const DevScene& S, PathSoA P, HitSoA H, const uint32_t* qcount, uint32_t max_count,
                 uint32_t* tq, uint32_t* tq_count) {

@@ -28,10 +28,12 @@ void launch_generate_list(const LaunchCtx& c, const DevScene& S, PathSoA P, HitS
 constexpr uint32_t kAdaptiveTile = 8;
 static_assert(kAdaptiveTile * kAdaptiveTile == 64, "k_adaptive_tiles: one warp per tile, two pixels per lane");
 enum { ADAPTIVE_FIRST = 0, ADAPTIVE_DECIDE = 1, ADAPTIVE_LAST = 2 };
-// per active tile: record n, decide (mode), append the kept tiles and their pixels to the next lists
+// per active tile: record n, decide (mode), append the kept tiles and their pixels to the next lists; ADAPTIVE_FIRST
+// visits the ntiles tiles shard, shard + nshards, shard + 2 nshards, ... of the frame
 void launch_adaptive_tiles(const LaunchCtx& c, const float4* A, const float4* B, uint32_t width, uint32_t height,
                            const uint32_t* tiles_in, uint32_t ntiles, uint32_t n, float inv_a, float inv_b, float tau, int mode,
-                           uint32_t* tile_n, uint32_t* tiles_out, uint32_t* pixels_out, uint32_t* counts_out);
+                           uint32_t* tile_n, uint32_t* tiles_out, uint32_t* pixels_out, uint32_t* counts_out, uint32_t shard,
+                           uint32_t nshards);
 // u8 image (and optionally the half sums, 6 floats per pixel, and the samples per pixel) from the even / odd sums
 void launch_resolve_adaptive(const LaunchCtx& c, const float4* A, const float4* B, const uint32_t* tile_n, uint32_t width, uint32_t npix,
                              uint8_t* out, float* halves, uint32_t* spp);
@@ -64,6 +66,16 @@ struct PeerAccums {
     int n;
 };
 void launch_resolve_peers(const LaunchCtx& c, const PeerAccums& A, float inv_samples, uint32_t nvalues, uint8_t* out, float* sum);
+// per-device half sums and tile counts of one multi-device adaptive render (tile t belongs to device t % n; pointers
+// valid on the device that launches), resolved as launch_resolve_adaptive does
+struct PeerHalves {
+    const float4* a[kMaxPeers];
+    const float4* b[kMaxPeers];
+    const uint32_t* tile_n[kMaxPeers];
+    int n;
+};
+void launch_resolve_adaptive_peers(const LaunchCtx& c, const PeerHalves& P, uint32_t width, uint32_t npix, uint8_t* out, float* halves,
+                                   uint32_t* spp);
 void launch_pack_rays(const LaunchCtx& c, long n, const float* o, const float* d, PathSoA P, uint32_t* q);
 void launch_unpack_hits(const LaunchCtx& c, const DevScene& S, long n, PathSoA P, HitSoA H, int32_t* id, float* t, float* nrm,
                         int32_t* interior);
