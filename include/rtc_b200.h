@@ -170,6 +170,25 @@ int rtc_render_ppm_multi(rtc_scene* s, const int* devices, int ndev, uint32_t se
  *      max_samples (summed over the devices). */
 int rtc_render_adaptive_multi(rtc_scene* s, const int* devices, int ndev, uint32_t seed, float tolerance, uint32_t min_samples,
                               uint32_t max_samples, uint8_t* rgb_host, float* halves_host, uint32_t* spp_host, uint64_t stats[4]);
+/* ---- denoising: non-local means on the even / odd half sums of a render (Rousselle, Knaus and Zwicker, "Adaptive
+ *      Rendering with Non-Local Means Filtering", 2012; DESIGN.md "Denoising").  Per pixel with n >= 2 samples: the mean
+ *      u = 1/n (A + B), D = display(u) (ACES, gamma 1/2.2, before 8-bit rounding) and, per channel, the variance estimate
+ *      V = ((D(A / ceil(n/2)) - D(B / floor(n/2))) / 2)^2.  The filtered mean of p is the weighted mean of u_q over the
+ *      15x15 window around p (q in the image, u_q finite), with w(p,q) = exp(-max(0, d2)), d2 = the mean over a 7x7 patch
+ *      (coordinates clamped to the image) and the channels of ((D_p - D_q)^2 - (V_p + min(V_p, V_q))) /
+ *      (1e-8 + strength^2 (V_p + V_q)).  A pixel whose mean is not finite keeps it.  strength must be finite and >= 0 (else
+ *      RTC_ERR_ARG); 0 is the identity, and the filter does not run.  rgb_host: 3 bytes per pixel, to_u8(aces(filtered
+ *      mean)); mean_host (may be NULL): the filtered mean, 3 floats per pixel.
+ * rtc_denoise filters halves the caller has, in the layout rtc_render_adaptive and rtc_render_adaptive_multi return
+ *      (6 floats and 1 spp per pixel of the scene's frame).  RTC_ERR_ARG, checked before any device call: a null halves or
+ *      spp pointer, a bad strength, any spp < 2, a hw1 / hw2 scene (no noise to estimate). */
+int rtc_denoise(rtc_scene* s, const float* halves_host, const uint32_t* spp_host, float strength, uint8_t* rgb_host, float* mean_host);
+/* rtc_render_denoised runs rtc_render_adaptive's passes and filters the half sums where they lie.  Arguments and stats are
+ *      rtc_render_adaptive's; min_samples >= the maximum (max_samples, or SAMPLES when it is 0) renders every pixel at
+ *      the maximum in one pass.  A maximum below 2 is RTC_ERR_ARG.  hw1 / hw2 return their one frame unfiltered, and the
+ *      frame as the mean. */
+int rtc_render_denoised(rtc_scene* s, uint32_t seed, float tolerance, uint32_t min_samples, uint32_t max_samples, float strength,
+                        uint8_t* rgb_host, float* mean_host, uint64_t stats[4]);
 /* ---- frames in flight: what run.sh does with a parsed scene (flattened scene host -> HBM, render, resolve, 8-bit
  *      image HBM -> host), queued without host synchronisation.  rtc_frame_begin uploads into the arena that is not
  *      being read (rtc_scene_upload_async: on a copy stream, under the kernels of the frame before), renders with the

@@ -22,6 +22,8 @@ HEADER_PATH = os.path.join(os.path.dirname(HERE), "include", "rtc_b200.h")
 
 TRAVERSAL_INDEX = 0
 TRAVERSAL_REFTREE = 1
+# recommended strength of the denoiser (Scene.Denoise, Scene.RenderDenoised; DESIGN.md "Denoising")
+DENOISE_STRENGTH = 0.45
 
 _f32 = np.ctypeslib.ndpointer(dtype=np.float32, flags="C_CONTIGUOUS")
 _i32 = np.ctypeslib.ndpointer(dtype=np.int32, flags="C_CONTIGUOUS")
@@ -75,6 +77,8 @@ _SIGNATURES = {
     "rtc_render_adaptive": (C.c_int, [C.c_void_p, C.c_uint32, C.c_float, C.c_uint32, C.c_uint32, _u8, _f32, _u32, _u64]),
     "rtc_render_adaptive_multi": (C.c_int, [C.c_void_p, _i32, C.c_int, C.c_uint32, C.c_float, C.c_uint32, C.c_uint32, _u8, _f32,
                                             _u32, _u64]),
+    "rtc_denoise": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_float, _u8, C.c_void_p]),
+    "rtc_render_denoised": (C.c_int, [C.c_void_p, C.c_uint32, C.c_float, C.c_uint32, C.c_uint32, C.c_float, _u8, C.c_void_p, _u64]),
     "rtc_set_batch_paths": (C.c_int, [C.c_void_p, C.c_uint64]),
     "rtc_set_profiling": (C.c_int, [C.c_void_p, C.c_int, C.c_int]),
     "rtc_render_profile": (C.c_int, [C.c_void_p, C.c_void_p, np.ctypeslib.ndpointer(dtype=np.float64, flags="C_CONTIGUOUS"), _u64, C.c_int]),
@@ -324,6 +328,34 @@ class Scene:
         _check(self.lib, self.lib.rtc_render_adaptive_multi(self.h, dv, len(dv), seed, float(tolerance), min_samples,
                                                             max_samples, img, halves, spp, st))
         return img, halves, spp, dict(zip(["passes", "paths", "tiles", "tiles_stopped"], [int(v) for v in st]))
+
+    def Denoise(self, halves, spp, strength=DENOISE_STRENGTH):
+        """Non-local-means filter (rtc_denoise) on the (H, W, 2, 3) half sums and (H, W) samples per pixel that
+        RenderAdaptive / RenderAdaptiveMulti return; every pixel needs at least 2 samples.  Returns the 8-bit image
+        (H, W, 3) and the filtered linear mean (H, W, 3 float32); strength 0 returns the unfiltered image."""
+        halves = np.ascontiguousarray(halves, np.float32)
+        spp = np.ascontiguousarray(spp, np.uint32)
+        if halves.shape != (self.height, self.width, 2, 3) or spp.shape != (self.height, self.width):
+            raise ValueError("expected halves (%d, %d, 2, 3) and spp (%d, %d), got %s and %s"
+                             % (self.height, self.width, self.height, self.width, halves.shape, spp.shape))
+        img = np.zeros((self.height, self.width, 3), np.uint8)
+        mean = np.zeros((self.height, self.width, 3), np.float32)
+        _check(self.lib, self.lib.rtc_denoise(self.h, halves.ctypes.data_as(C.c_void_p), spp.ctypes.data_as(C.c_void_p),
+                                              float(strength), img, mean.ctypes.data_as(C.c_void_p)))
+        return img, mean
+
+    def RenderDenoised(self, strength=DENOISE_STRENGTH, tolerance=0.0, min_samples=None, max_samples=0, seed=0):
+        """RenderAdaptive's passes, then the filter of Denoise on the half sums where they lie (rtc_render_denoised).
+        min_samples=None renders every pixel at the maximum (max_samples, or the scene's SAMPLES when it is 0).  Returns
+        the 8-bit image (H, W, 3), the filtered mean (H, W, 3 float32) and RenderAdaptive's stats dict."""
+        if min_samples is None:
+            min_samples = max(2, max_samples or self.samples)
+        img = np.zeros((self.height, self.width, 3), np.uint8)
+        mean = np.zeros((self.height, self.width, 3), np.float32)
+        st = np.zeros(4, np.uint64)
+        _check(self.lib, self.lib.rtc_render_denoised(self.h, seed, float(tolerance), min_samples, max_samples, float(strength),
+                                                      img, mean.ctypes.data_as(C.c_void_p), st))
+        return img, mean, dict(zip(["passes", "paths", "tiles", "tiles_stopped"], [int(v) for v in st]))
 
     def RenderMulti(self, devices, seed=0, want_sum=False):
         """Scene::Render on several CUDA devices of this process: samples split over `devices`, summed over peer

@@ -5,6 +5,7 @@
 
 #include <algorithm>
 #include <array>
+#include <cfloat>
 #include <cmath>
 #include <chrono>
 #include <cstdio>
@@ -182,6 +183,12 @@ struct rtc_scene {
         DevBuf<float> halves;
         PinnedBuf<uint32_t> counts_host;
     } adaptive;
+    // rtc_denoise / rtc_render_denoised: the linear mean u (3 floats per pixel), D and V (k_denoise_prep) and the filtered
+    // mean (k_denoise_nlm)
+    struct Denoise {
+        DevBuf<float> u, mean;
+        DevBuf<float4> d, v;
+    } denoise;
     uint64_t launches = 0;
     // optional per-kernel timing (CUDA events on the launching stream)
     bool profiling = false;
@@ -1187,6 +1194,92 @@ int rtc_render_adaptive(rtc_scene* s, uint32_t seed, float tolerance, uint32_t m
     if (halves_host) CU(cudaMemcpy(halves_host, ad.halves.p, 6 * (size_t)npix * sizeof(float), cudaMemcpyDeviceToHost));
     if (spp_host) CU(cudaMemcpy(spp_host, ad.spp.p, (size_t)npix * sizeof(uint32_t), cudaMemcpyDeviceToHost));
     CU(cudaStreamSynchronize(user));
+    if (stats) std::memcpy(stats, st, sizeof st);
+    return RTC_OK;
+}
+
+// ------------------------------------------------------------------ denoising
+namespace {
+int check_strength(float strength) {
+    if (!std::isfinite(strength) || strength < 0.f) return fail(RTC_ERR_ARG, "strength must be finite and >= 0");
+    return RTC_OK;
+}
+// The filter on the half sums and sample counts in halves_dev / spp_dev (the layout of k_resolve_adaptive's optional
+// outputs, every spp >= 2), on the default stream: k_denoise_prep, then k_denoise_nlm unless strength is 0 (then the
+// image is that of the mean u, as rtc_render_adaptive resolves it).  Copies the image and the mean to the host.
+int denoise(rtc_scene* s, const float* halves_dev, const uint32_t* spp_dev, float strength, uint8_t* rgb_host, float* mean_host) {
+    const uint32_t width = s->host.cam.width, height = s->host.cam.height, npix = width * height;
+    rtc_scene::Denoise& dn = s->denoise;
+    CU(dn.u.ensure(3 * (size_t)npix));
+    CU(dn.d.ensure(npix));
+    CU(dn.v.ensure(npix));
+    CU(s->rgb.ensure(3 * (size_t)npix));
+    const LaunchCtx lc{nullptr, s->sms};
+    const bool filter = strength > 0.f;
+    launch_denoise_prep(lc, halves_dev, spp_dev, npix, dn.u.p, dn.d.p, dn.v.p, filter ? nullptr : s->rgb.p);
+    s->launches++;
+    CU(cudaGetLastError());
+    if (filter) {
+        CU(dn.mean.ensure(3 * (size_t)npix));
+        // k^2 saturates instead of overflowing: the weights are then all 1 where the patches' variance is non-zero
+        CU(launch_denoise_nlm(lc, dn.u.p, dn.d.p, dn.v.p, width, height, std::fmin(strength * strength, FLT_MAX), dn.mean.p, s->rgb.p));
+        s->launches++;
+    }
+    if (rgb_host) CU(cudaMemcpy(rgb_host, s->rgb.p, 3 * (size_t)npix, cudaMemcpyDeviceToHost));
+    if (mean_host) CU(cudaMemcpy(mean_host, filter ? dn.mean.p : dn.u.p, 3 * (size_t)npix * sizeof(float), cudaMemcpyDeviceToHost));
+    CU(cudaStreamSynchronize(nullptr));
+    return RTC_OK;
+}
+}  // namespace
+int rtc_denoise(rtc_scene* s, const float* halves_host, const uint32_t* spp_host, float strength, uint8_t* rgb_host, float* mean_host) {
+    if (!s) return fail(RTC_ERR_ARG, "null scene");
+    if (!halves_host || !spp_host) return fail(RTC_ERR_ARG, "null halves or spp");
+    int rc = check_strength(strength);
+    if (rc) return rc;
+    if (s->host.dialect <= DIALECT_HW2) return fail(RTC_ERR_ARG, "hw1 / hw2 scenes have no noise to filter");
+    const size_t npix = (size_t)s->host.cam.width * s->host.cam.height;
+    for (size_t i = 0; i < npix; ++i)
+        if (spp_host[i] < 2) return fail(RTC_ERR_ARG, "every pixel needs at least 2 samples (pixel " + std::to_string(i) + ")");
+    if ((rc = need_device(s))) return rc;
+    if (npix == 0) return RTC_OK;
+    rtc_scene::Adaptive& ad = s->adaptive;
+    CU(ad.halves.ensure(6 * npix));
+    CU(ad.spp.ensure(npix));
+    CU(cudaMemcpy(ad.halves.p, halves_host, 6 * npix * sizeof(float), cudaMemcpyHostToDevice));
+    CU(cudaMemcpy(ad.spp.p, spp_host, npix * sizeof(uint32_t), cudaMemcpyHostToDevice));
+    return denoise(s, ad.halves.p, ad.spp.p, strength, rgb_host, mean_host);
+}
+int rtc_render_denoised(rtc_scene* s, uint32_t seed, float tolerance, uint32_t min_samples, uint32_t max_samples, float strength,
+                        uint8_t* rgb_host, float* mean_host, uint64_t stats[4]) {
+    if (!s) return fail(RTC_ERR_ARG, "null scene");
+    int rc = check_strength(strength);
+    if (rc) return rc;
+    const uint32_t width = s->host.cam.width, height = s->host.cam.height, npix = width * height;
+    if (s->host.dialect <= DIALECT_HW2) {
+        // the one deterministic frame, unfiltered: rtc_render_adaptive's, whose mean is the frame it leaves in s->accum
+        if ((rc = rtc_render_adaptive(s, seed, tolerance, min_samples, max_samples, rgb_host, nullptr, nullptr, stats))) return rc;
+        if (mean_host && npix) CU(cudaMemcpy(mean_host, s->accum.p, 3 * (size_t)npix * sizeof(float), cudaMemcpyDeviceToHost));
+        return RTC_OK;
+    }
+    if (!std::isfinite(tolerance) || tolerance < 0.f) return fail(RTC_ERR_ARG, "tolerance must be finite and >= 0");
+    if (min_samples < 2) return fail(RTC_ERR_ARG, "min_samples must be at least 2");
+    const uint32_t smax = max_samples ? max_samples : s->host.samples;
+    if (smax < 2) return fail(RTC_ERR_ARG, "the maximum sample count must be at least 2");
+    if ((rc = need_device(s))) return rc;
+    uint64_t st[4] = {0, 0, 0, 0};   // passes, paths, tiles, tiles stopped below the maximum
+    if (stats) std::memcpy(stats, st, sizeof st);
+    if (npix == 0) return RTC_OK;
+    st[2] = adaptive_tiles(width, height);
+    if ((rc = adaptive_passes(s, nullptr, 0, 1, seed, tolerance, min_samples, smax, st))) return rc;
+    rtc_scene::Adaptive& ad = s->adaptive;
+    CU(s->rgb.ensure(3 * (size_t)npix));
+    CU(ad.halves.ensure(6 * (size_t)npix));
+    CU(ad.spp.ensure(npix));
+    launch_resolve_adaptive(LaunchCtx{nullptr, s->sms}, ad.half[0].p, ad.half[1].p, ad.tile_n.p, width, npix, s->rgb.p, ad.halves.p,
+                            ad.spp.p);
+    s->launches++;
+    CU(cudaGetLastError());
+    if ((rc = denoise(s, ad.halves.p, ad.spp.p, strength, rgb_host, mean_host))) return rc;
     if (stats) std::memcpy(stats, st, sizeof st);
     return RTC_OK;
 }

@@ -8,7 +8,11 @@
 //                        noise is below tau display units (1/255 = one 8-bit level), at most the scene's SAMPLES (after
 //                        RTC_SAMPLES); 0 renders every pixel at SAMPLES.  A value that is not a finite number >= 0 or a
 //                        list of several RTC_DEVICES is an error.
-//   RTC_TIMING=1     phase times on stderr (with RTC_ADAPTIVE also the passes and paths rendered)
+//   RTC_DENOISE=<k>      filter the render with non-local means of strength k (rtc_render_denoised, one device; 0.45 is
+//                        the recommended strength, 0 leaves the image as rendered): every pixel at SAMPLES, or with
+//                        RTC_ADAPTIVE=<tau> adaptive sampling as above.  A value that is not a finite number >= 0 or a list
+//                        of several RTC_DEVICES is an error.
+//   RTC_TIMING=1     phase times on stderr (with RTC_ADAPTIVE or RTC_DENOISE also the passes and paths rendered)
 // The same program serves the four earlier homework snapshots (hwN/run.sh -> build/raytracing_hwN): the dialect
 // is the digit in the name it is called by (raytracing_hw1 .. raytracing_hw4 are links to this binary), or
 // RTC_DIALECT=<1..5>.
@@ -92,6 +96,21 @@ int main(int argc, const char* argv[]) {
             return 1;
         }
     }
+    const char* denoise = std::getenv("RTC_DENOISE");
+    if (denoise && !*denoise) denoise = nullptr;
+    float strength = 0.f;
+    if (denoise) {
+        char* end = nullptr;
+        strength = std::strtof(denoise, &end);
+        if (end == denoise || *end || !std::isfinite(strength) || strength < 0.f) {
+            std::fprintf(stderr, "raytracing_hw5: RTC_DENOISE=%s is not a finite number >= 0\n", denoise);
+            return 1;
+        }
+        if (devices.size() > 1) {
+            std::fprintf(stderr, "raytracing_hw5: RTC_DENOISE renders on one device; RTC_DEVICES lists %zu\n", devices.size());
+            return 1;
+        }
+    }
     rtc_scene* scene = rtc_scene_load_dialect(argv[1], device0, dialect);
     if (!scene) {
         std::fprintf(stderr, "raytracing_hw5: %s\n", rtc_last_error());
@@ -109,9 +128,13 @@ int main(int argc, const char* argv[]) {
     rtc_scene_info(scene, info);
     uint64_t astats[4] = {0, 0, 0, 0};
     bool written_error = false;
-    if (adaptive) {
+    if (adaptive || denoise) {
         std::vector<uint8_t> img(3 * (size_t)info[0] * info[1]);
-        rc = rtc_render_adaptive(scene, (uint32_t)env_int("RTC_SEED", 0), tau, 16, 0, img.data(), nullptr, nullptr, astats);
+        const uint32_t seed = (uint32_t)env_int("RTC_SEED", 0);
+        // without RTC_ADAPTIVE: min_samples = SAMPLES (at least 2) renders every pixel at SAMPLES
+        const uint32_t min_samples = adaptive ? 16u : (info[3] > 2 ? info[3] : 2u);
+        if (denoise) rc = rtc_render_denoised(scene, seed, tau, min_samples, 0, strength, img.data(), nullptr, astats);
+        else rc = rtc_render_adaptive(scene, seed, tau, min_samples, 0, img.data(), nullptr, nullptr, astats);
         if (rc == RTC_OK && !write_ppm(argv[2], info[0], info[1], img)) {
             std::fprintf(stderr, "raytracing_hw5: cannot write %s\n", argv[2]);
             rc = RTC_ERR_IO;
@@ -124,7 +147,7 @@ int main(int argc, const char* argv[]) {
     if (timing)
         std::fprintf(stderr, "[rtc timing] %-28s %8.1f ms\n[rtc timing] %-28s %8.1f ms\n",
                      "load (file -> HBM, CUDA init)", ms(t_start, t_loaded), "render + PPM", ms(t_loaded, t_rendered));
-    if (timing && adaptive)
+    if (timing && (adaptive || denoise))
         std::fprintf(stderr, "[rtc timing] adaptive: %llu passes, %llu paths, %llu of %llu tiles stopped below SAMPLES\n",
                      (unsigned long long)astats[0], (unsigned long long)astats[1], (unsigned long long)astats[3],
                      (unsigned long long)astats[2]);

@@ -728,6 +728,137 @@ __global__ void __launch_bounds__(256) k_resolve_adaptive_peers(PeerHalves P, ui
     }
 }
 
+// ------------------------------------------------------------------------------- denoising (rtc_denoise, rtc_render_denoised)
+// Non-local means on the even / odd half sums (Rousselle, Knaus and Zwicker 2012; DESIGN.md "Denoising").  Per pixel
+// with n >= 2 samples: u = 1/n (A + B) (resolve_adaptive_pixel's floats), D = display(u) and, per channel, the variance
+// estimate V = ((display(A / ceil(n/2)) - display(B / floor(n/2))) / 2)^2 (k_adaptive_tiles' half means).  rgb, when
+// given (the filter is not run), gets resolve_adaptive_pixel's image of u.
+__global__ void __launch_bounds__(256) k_denoise_prep(const float* halves, const uint32_t* spp, uint32_t npix, float* u, float4* D,
+                                                       float4* V, uint8_t* rgb) {
+    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < npix; i += gridDim.x * blockDim.x) {
+        const uint32_t n = spp[i];
+        const float inv = __fdiv_rn(1.f, (float)n), inv_a = __fdiv_rn(1.f, (float)((n + 1) / 2)), inv_b = __fdiv_rn(1.f, (float)(n / 2));
+        const float* h = halves + 6 * (size_t)i;
+        float uc[3], dc[3], vc[3];
+#pragma unroll
+        for (int c = 0; c < 3; ++c) {
+            uc[c] = __fmul_rn(inv, __fadd_rn(h[c], h[3 + c]));
+            dc[c] = display(uc[c]);
+            const float e = __fmul_rn(__fsub_rn(display(__fmul_rn(h[c], inv_a)), display(__fmul_rn(h[3 + c], inv_b))), 0.5f);
+            vc[c] = __fmul_rn(e, e);
+            u[3 * (size_t)i + c] = uc[c];
+            if (rgb) rgb[3 * (size_t)i + c] = to_u8(aces(uc[c]));
+        }
+        D[i] = make_float4(dc[0], dc[1], dc[2], 0.f);
+        V[i] = make_float4(vc[0], vc[1], vc[2], 0.f);
+    }
+}
+// One block filters a kDenoiseTileW x kDenoiseTileH tile of pixels.  It stages D and the smoothed V (the mean of V over
+// the (2S+1)^2 box around the pixel) of the tile and its apron of R + F (coordinates clamped to the image: patches repeat
+// the edge pixels) and u of the tile and its apron of R (NaN
+// outside the image, so that such neighbours fail the finiteness test), then walks the (2R+1)^2 offsets: per offset
+// the distance term of every pixel of the tile plus F, a row box sum of width 2F+1, and per pixel the column box sum,
+// the weight and the weighted sums in registers.  Two barriers per offset; each thread owns two pixels of a column.
+constexpr int kDnR = kDenoiseRadius, kDnF = kDenoisePatch, kDnS = kDenoiseVarRadius, kDnA = kDnR + kDnF;
+constexpr int kDnTW = kDenoiseTileW, kDnTH = kDenoiseTileH, kDnThreads = 256, kDnRows = kDnThreads / kDnTW;
+constexpr int kDnSW = kDnTW + 2 * kDnA, kDnSH = kDnTH + 2 * kDnA;   // D, V staging
+constexpr int kDnUW = kDnTW + 2 * kDnR, kDnUH = kDnTH + 2 * kDnR;   // u staging
+constexpr int kDnEW = kDnTW + 2 * kDnF, kDnEH = kDnTH + 2 * kDnF;   // distance terms of one offset
+constexpr int kDnPix = kDnTH / kDnRows;                              // pixels per thread
+static_assert(kDnTW == 32 && kDnTH % kDnRows == 0, "k_denoise_nlm: a warp per tile row");
+constexpr size_t kDenoiseSmemFloats = 6 * (size_t)kDnSW * kDnSH + 3 * (size_t)kDnUW * kDnUH + kDnEW * kDnEH + kDnTW * kDnEH;
+__global__ void __launch_bounds__(kDnThreads) k_denoise_nlm(const float* u, const float4* D, const float4* V, uint32_t width,
+                                                             uint32_t height, float k2, float* mean, uint8_t* rgb) {
+    extern __shared__ float smem[];
+    float* sD = smem;                              // [3][kDnSH][kDnSW]
+    float* sV = sD + 3 * kDnSW * kDnSH;            // [3][kDnSH][kDnSW]
+    float* sU = sV + 3 * kDnSW * kDnSH;            // [3][kDnUH][kDnUW]
+    float* sT = sU + 3 * kDnUW * kDnUH;            // [kDnEH][kDnEW]
+    float* sH = sT + kDnEW * kDnEH;                // [kDnEH][kDnTW]
+    const int x0 = blockIdx.x * kDnTW, y0 = blockIdx.y * kDnTH, W = (int)width, H = (int)height;
+    for (int i = threadIdx.x; i < kDnSW * kDnSH; i += kDnThreads) {
+        const int gx = min(max(x0 - kDnA + i % kDnSW, 0), W - 1), gy = min(max(y0 - kDnA + i / kDnSW, 0), H - 1);
+        const float4 d = D[(size_t)gy * W + gx];
+        float4 v = make_float4(0.f, 0.f, 0.f, 0.f);   // V smoothed over the (2S+1)^2 box around (gx, gy), clamped
+        for (int oy = -kDnS; oy <= kDnS; ++oy)
+            for (int ox = -kDnS; ox <= kDnS; ++ox) {
+                const float4 t = V[(size_t)min(max(gy + oy, 0), H - 1) * W + min(max(gx + ox, 0), W - 1)];
+                v.x += t.x; v.y += t.y; v.z += t.z;
+            }
+        constexpr float inv_box = 1.f / ((2 * kDnS + 1) * (2 * kDnS + 1));
+        v.x *= inv_box; v.y *= inv_box; v.z *= inv_box;
+        sD[i] = d.x; sD[i + kDnSW * kDnSH] = d.y; sD[i + 2 * kDnSW * kDnSH] = d.z;
+        sV[i] = v.x; sV[i + kDnSW * kDnSH] = v.y; sV[i + 2 * kDnSW * kDnSH] = v.z;
+    }
+    for (int i = threadIdx.x; i < kDnUW * kDnUH; i += kDnThreads) {
+        const int gx = x0 - kDnR + i % kDnUW, gy = y0 - kDnR + i / kDnUW;
+        const bool in = gx >= 0 && gx < W && gy >= 0 && gy < H;
+#pragma unroll
+        for (int c = 0; c < 3; ++c) sU[i + c * kDnUW * kDnUH] = in ? u[3 * ((size_t)gy * W + gx) + c] : __int_as_float(0x7fc00000);
+    }
+    __syncthreads();
+    const int tx = threadIdx.x % kDnTW, ty = threadIdx.x / kDnTW;
+    float sw[kDnPix], su[kDnPix][3];
+#pragma unroll
+    for (int j = 0; j < kDnPix; ++j) sw[j] = su[j][0] = su[j][1] = su[j][2] = 0.f;
+    const float inv_patch = 1.f / (3.f * (2 * kDnF + 1) * (2 * kDnF + 1));
+    for (int dy = -kDnR; dy <= kDnR; ++dy) {
+        for (int dx = -kDnR; dx <= kDnR; ++dx) {
+            // distance term of extended pixel e (the tile plus F): p + o at staging (ey + R, ex + R), q + o shifted by (dy, dx)
+            for (int e = threadIdx.x; e < kDnEW * kDnEH; e += kDnThreads) {
+                const int ip = (e / kDnEW + kDnR) * kDnSW + e % kDnEW + kDnR, iq = ip + dy * kDnSW + dx;
+                float t = 0.f;
+#pragma unroll
+                for (int c = 0; c < 3; ++c) {
+                    const float dp = sD[ip + c * kDnSW * kDnSH], dq = sD[iq + c * kDnSW * kDnSH];
+                    const float vp = sV[ip + c * kDnSW * kDnSH], vq = sV[iq + c * kDnSW * kDnSH];
+                    const float num = (dp - dq) * (dp - dq) - kDenoiseAlpha * (vp + fminf(vp, vq));
+                    t += __fdividef(num, kDenoiseEps + k2 * (vp + vq));
+                }
+                sT[e] = t;
+            }
+            __syncthreads();
+            for (int e = threadIdx.x; e < kDnTW * kDnEH; e += kDnThreads) {
+                const float* row = sT + (e / kDnTW) * kDnEW + e % kDnTW;
+                float s = 0.f;
+#pragma unroll
+                for (int o = 0; o <= 2 * kDnF; ++o) s += row[o];
+                sH[e] = s;
+            }
+            __syncthreads();
+#pragma unroll
+            for (int j = 0; j < kDnPix; ++j) {
+                const int ly = ty + j * kDnRows;
+                float s = 0.f;
+#pragma unroll
+                for (int o = 0; o <= 2 * kDnF; ++o) s += sH[(ly + o) * kDnTW + tx];
+                const int iq = (ly + kDnR + dy) * kDnUW + tx + kDnR + dx;
+                const float qr = sU[iq], qg = sU[iq + kDnUW * kDnUH], qb = sU[iq + 2 * kDnUW * kDnUH];
+                if (isfinite(qr) && isfinite(qg) && isfinite(qb)) {
+                    const float w = __expf(-fmaxf(0.f, s * inv_patch));
+                    sw[j] += w;
+                    su[j][0] += w * qr; su[j][1] += w * qg; su[j][2] += w * qb;
+                }
+            }
+        }
+    }
+#pragma unroll
+    for (int j = 0; j < kDnPix; ++j) {
+        const int x = x0 + tx, y = y0 + ty + j * kDnRows;
+        if (x >= W || y >= H) continue;
+        const int ip = (ty + j * kDnRows + kDnR) * kDnUW + tx + kDnR;
+        float up[3] = {sU[ip], sU[ip + kDnUW * kDnUH], sU[ip + 2 * kDnUW * kDnUH]};
+        const bool finite = isfinite(up[0]) && isfinite(up[1]) && isfinite(up[2]);   // else it passes through
+        const size_t i = (size_t)y * W + x;
+#pragma unroll
+        for (int c = 0; c < 3; ++c) {
+            const float v = finite ? __fdiv_rn(su[j][c], sw[j]) : up[c];
+            mean[3 * i + c] = v;
+            rgb[3 * i + c] = to_u8(aces(v));
+        }
+    }
+}
+
 // ------------------------------------------------------------------------------- scene arena, device-built tail
 // Levels >= 1 of the LCA range-minimum table (bvh_build.cpp: lca[l][c] = the shallower of lca[l-1][c] and
 // lca[l-1][c + 2^(l-1)]) from level 0, which is uploaded; one launch per level.
@@ -847,6 +978,19 @@ void launch_resolve_adaptive(const LaunchCtx& c, const float4* A, const float4* 
 void launch_resolve_adaptive_peers(const LaunchCtx& c, const PeerHalves& P, uint32_t width, uint32_t npix, uint8_t* out, float* halves,
                                    uint32_t* spp) {
     k_resolve_adaptive_peers<<<grid_for(npix, 256, c.sms, 8), 256, 0, c.stream>>>(P, width, npix, out, halves, spp);
+}
+void launch_denoise_prep(const LaunchCtx& c, const float* halves, const uint32_t* spp, uint32_t npix, float* u, float4* D, float4* V,
+                         uint8_t* rgb) {
+    k_denoise_prep<<<grid_for(npix, 256, c.sms, 8), 256, 0, c.stream>>>(halves, spp, npix, u, D, V, rgb);
+}
+cudaError_t launch_denoise_nlm(const LaunchCtx& c, const float* u, const float4* D, const float4* V, uint32_t width, uint32_t height,
+                               float k2, float* mean, uint8_t* rgb) {
+    const size_t bytes = kDenoiseSmemFloats * sizeof(float);
+    cudaError_t e = cudaFuncSetAttribute(k_denoise_nlm, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+    if (e != cudaSuccess) return e;
+    const dim3 grid((width + kDnTW - 1) / kDnTW, (height + kDnTH - 1) / kDnTH);
+    k_denoise_nlm<<<grid, kDnThreads, bytes, c.stream>>>(u, D, V, width, height, k2, mean, rgb);
+    return cudaGetLastError();
 }
 void launch_pre(const LaunchCtx& c, const DevScene& S, PathSoA P, HitSoA H, const uint32_t* qcount, uint32_t max_count,
                 uint32_t* tq, uint32_t* tq_count) {

@@ -37,6 +37,19 @@ void launch_adaptive_tiles(const LaunchCtx& c, const float4* A, const float4* B,
 // u8 image (and optionally the half sums, 6 floats per pixel, and the samples per pixel) from the even / odd sums
 void launch_resolve_adaptive(const LaunchCtx& c, const float4* A, const float4* B, const uint32_t* tile_n, uint32_t width, uint32_t npix,
                              uint8_t* out, float* halves, uint32_t* spp);
+// denoising (rtc_denoise, rtc_render_denoised; DESIGN.md "Denoising"): the fixed constants of the non-local-means rule
+// -- search window (2R+1)^2, patch (2F+1)^2, box (2S+1)^2 that smooths the variance estimate, variance cancellation
+// alpha, epsilon -- and the output tile of one block
+constexpr int kDenoiseRadius = 7, kDenoisePatch = 3, kDenoiseVarRadius = 1;
+constexpr float kDenoiseAlpha = 1.f, kDenoiseEps = 1e-8f;
+constexpr int kDenoiseTileW = 32, kDenoiseTileH = 16;
+// per pixel from the half sums (6 floats) and spp (>= 2): the linear mean u (3 floats), D = display(u) and the variance
+// estimate V (float4, w unused); rgb (optional) = the 8-bit image of u
+void launch_denoise_prep(const LaunchCtx& c, const float* halves, const uint32_t* spp, uint32_t npix, float* u, float4* D, float4* V,
+                         uint8_t* rgb);
+// the filter with k2 = strength^2: mean (3 floats per pixel) and its 8-bit image
+cudaError_t launch_denoise_nlm(const LaunchCtx& c, const float* u, const float4* D, const float4* V, uint32_t width, uint32_t height,
+                               float k2, float* mean, uint8_t* rgb);
 // Scene::RayIntersection for the rays of queue P (fills H): launch_pre then launch_traverse
 // (index BVH), or launch_extend_reftree alone (the reference-tree twin).
 void launch_pre(const LaunchCtx& c, const DevScene& S, PathSoA P, HitSoA H, const uint32_t* qcount, uint32_t max_count,
