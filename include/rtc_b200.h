@@ -189,6 +189,18 @@ int rtc_denoise(rtc_scene* s, const float* halves_host, const uint32_t* spp_host
  *      frame as the mean. */
 int rtc_render_denoised(rtc_scene* s, uint32_t seed, float tolerance, uint32_t min_samples, uint32_t max_samples, float strength,
                         uint8_t* rgb_host, float* mean_host, uint64_t stats[4]);
+/* rtc_render_denoised on several devices of this process: the passes of rtc_render_adaptive_multi (tile t belongs to
+ *      devices[t % ndev]), then the filter split into bands of rows.  With T = ceil(H / 16) tile rows of the filter,
+ *      entry i filters the rows [16 floor(i T / ndev), min(H, 16 floor((i + 1) T / ndev))) -- none when ndev > T -- on
+ *      its own device, reading those rows and 11 more on either side from the tiles' owners over peer access (or copies
+ *      of those rows when a pair cannot map each other), and writes its rows of rgb_host and mean_host.  The result is
+ *      rtc_denoise's on the same half sums, bit for bit.  halves_host / spp_host (optional, rtc_render_adaptive_multi's
+ *      layout) are gathered on devices[0]; they are the half sums the filter read.  Arguments, errors and stats are the
+ *      union of rtc_render_denoised's and rtc_render_adaptive_multi's, every check before any device call.  hw1 / hw2
+ *      return rtc_render_denoised's unfiltered frame, rendered on devices[0]. */
+int rtc_render_denoised_multi(rtc_scene* s, const int* devices, int ndev, uint32_t seed, float tolerance, uint32_t min_samples,
+                              uint32_t max_samples, float strength, uint8_t* rgb_host, float* mean_host, float* halves_host,
+                              uint32_t* spp_host, uint64_t stats[4]);
 /* ---- frames in flight: what run.sh does with a parsed scene (flattened scene host -> HBM, render, resolve, 8-bit
  *      image HBM -> host), queued without host synchronisation.  rtc_frame_begin uploads into the arena that is not
  *      being read (rtc_scene_upload_async: on a copy stream, under the kernels of the frame before), renders with the

@@ -79,6 +79,8 @@ _SIGNATURES = {
                                             _u32, _u64]),
     "rtc_denoise": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_float, _u8, C.c_void_p]),
     "rtc_render_denoised": (C.c_int, [C.c_void_p, C.c_uint32, C.c_float, C.c_uint32, C.c_uint32, C.c_float, _u8, C.c_void_p, _u64]),
+    "rtc_render_denoised_multi": (C.c_int, [C.c_void_p, _i32, C.c_int, C.c_uint32, C.c_float, C.c_uint32, C.c_uint32, C.c_float, _u8,
+                                            C.c_void_p, C.c_void_p, C.c_void_p, _u64]),
     "rtc_set_batch_paths": (C.c_int, [C.c_void_p, C.c_uint64]),
     "rtc_set_profiling": (C.c_int, [C.c_void_p, C.c_int, C.c_int]),
     "rtc_render_profile": (C.c_int, [C.c_void_p, C.c_void_p, np.ctypeslib.ndpointer(dtype=np.float64, flags="C_CONTIGUOUS"), _u64, C.c_int]),
@@ -356,6 +358,24 @@ class Scene:
         _check(self.lib, self.lib.rtc_render_denoised(self.h, seed, float(tolerance), min_samples, max_samples, float(strength),
                                                       img, mean.ctypes.data_as(C.c_void_p), st))
         return img, mean, dict(zip(["passes", "paths", "tiles", "tiles_stopped"], [int(v) for v in st]))
+
+    def RenderDenoisedMulti(self, devices, strength=DENOISE_STRENGTH, tolerance=0.0, min_samples=None, max_samples=0, seed=0):
+        """RenderDenoised on several CUDA devices of this process (rtc_render_denoised_multi): RenderAdaptiveMulti's
+        passes, then every entry filters a band of rows where the half sums lie.  min_samples=None means what it means
+        for RenderDenoised.  Returns the 8-bit image (H, W, 3), the filtered mean (H, W, 3 float32), the half sums
+        (H, W, 2, 3 float32) and samples per pixel (H, W uint32) the filter read, and RenderAdaptiveMulti's stats dict."""
+        if min_samples is None:
+            min_samples = max(2, max_samples or self.samples)
+        dv = np.asarray(devices, np.int32)
+        img = np.zeros((self.height, self.width, 3), np.uint8)
+        mean = np.zeros((self.height, self.width, 3), np.float32)
+        halves = np.zeros((self.height, self.width, 2, 3), np.float32)
+        spp = np.zeros((self.height, self.width), np.uint32)
+        st = np.zeros(4, np.uint64)
+        _check(self.lib, self.lib.rtc_render_denoised_multi(self.h, dv, len(dv), seed, float(tolerance), min_samples, max_samples,
+                                                            float(strength), img, mean.ctypes.data_as(C.c_void_p),
+                                                            halves.ctypes.data_as(C.c_void_p), spp.ctypes.data_as(C.c_void_p), st))
+        return img, mean, halves, spp, dict(zip(["passes", "paths", "tiles", "tiles_stopped"], [int(v) for v in st]))
 
     def RenderMulti(self, devices, seed=0, want_sum=False):
         """Scene::Render on several CUDA devices of this process: samples split over `devices`, summed over peer

@@ -1222,7 +1222,8 @@ int denoise(rtc_scene* s, const float* halves_dev, const uint32_t* spp_dev, floa
     if (filter) {
         CU(dn.mean.ensure(3 * (size_t)npix));
         // k^2 saturates instead of overflowing: the weights are then all 1 where the patches' variance is non-zero
-        CU(launch_denoise_nlm(lc, dn.u.p, dn.d.p, dn.v.p, width, height, std::fmin(strength * strength, FLT_MAX), dn.mean.p, s->rgb.p));
+        CU(launch_denoise_nlm(lc, dn.u.p, dn.d.p, dn.v.p, width, height, 0, (height + kDenoiseTileH - 1) / kDenoiseTileH, 0,
+                              std::fmin(strength * strength, FLT_MAX), dn.mean.p, s->rgb.p));
         s->launches++;
     }
     if (rgb_host) CU(cudaMemcpy(rgb_host, s->rgb.p, 3 * (size_t)npix, cudaMemcpyDeviceToHost));
@@ -1506,15 +1507,78 @@ int rtc_render_ppm_multi(rtc_scene* s, const int* devices, int ndev, uint32_t se
 // pass loop of rtc_render_adaptive on its own tiles, on its own stream and host thread.  A tile's decisions read only its
 // own half sums, so the devices do not talk to each other until devices[0] resolves every pixel from its owner's
 // half sums and tile counts (k_resolve_adaptive_peers).
-int rtc_render_adaptive_multi(rtc_scene* s, const int* devices, int ndev, uint32_t seed, float tolerance, uint32_t min_samples,
-                              uint32_t max_samples, uint8_t* rgb_host, float* halves_host, uint32_t* spp_host, uint64_t stats[4]) {
-    if (!s) return fail(RTC_ERR_ARG, "null scene");
+namespace {
+int check_adaptive_multi_args(float tolerance, uint32_t min_samples, const int* devices, int ndev) {
     if (!std::isfinite(tolerance) || tolerance < 0.f) return fail(RTC_ERR_ARG, "tolerance must be finite and >= 0");
     if (min_samples < 2) return fail(RTC_ERR_ARG, "min_samples must be at least 2");
     if (!devices || ndev < 1 || ndev > kMaxPeers) return fail(RTC_ERR_ARG, "devices must list 1 to 16 entries");
     for (int i = 0; i < ndev; ++i)
         if (devices[i] < 0 || devices[i] >= 64) return fail(RTC_ERR_ARG, "bad device index");
-    int rc = need_device(s);
+    return RTC_OK;
+}
+// The passes of every entry of `ctx`: entry i runs adaptive_passes on the tiles i, i + n, ... on its multi_stream and a
+// host thread of its own, and records its multi_done.  st: passes (the most of any entry), paths, tiles, tiles stopped.
+int adaptive_passes_multi(const std::vector<rtc_scene*>& ctx, uint32_t seed, float tolerance, uint32_t min_samples, uint32_t smax,
+                          uint32_t ntiles, uint64_t st[4]) {
+    const int ndev = (int)ctx.size();
+    std::vector<std::array<uint64_t, 4>> dev_st((size_t)ndev, std::array<uint64_t, 4>{0, 0, 0, 0});
+    auto issue = [&](int i) -> int {
+        rtc_scene* c = ctx[i];
+        CU(cudaSetDevice(c->device));
+        CU(c->multi_stream.ensure());
+        CU(c->multi_done.ensure());
+        int r = adaptive_passes(c, c->multi_stream, (uint32_t)i, (uint32_t)ndev, seed, tolerance, min_samples, smax, dev_st[i].data());
+        if (r) return r;
+        CU(cudaEventRecord(c->multi_done, c->multi_stream));
+        return RTC_OK;
+    };
+    int rc = fan_out(ndev, issue);
+    if (rc) return rc;
+    st[2] = ntiles;
+    for (const auto& d : dev_st) {
+        st[0] = std::max(st[0], d[0]);
+        st[1] += d[1];
+        st[3] += d[3];
+    }
+    return RTC_OK;
+}
+// The owners' half sums of the image rows [row0, row0 + nrows) and their whole tile counts, for entry `c` (its device
+// current) after adaptive_passes_multi: c's multi_stream waits for every other owner, and reads its buffers in place
+// (peer access) or copies those rows over (held by `staged`).
+int owner_halves(rtc_scene* c, const std::vector<rtc_scene*>& ctx, uint32_t width, uint32_t row0, uint32_t nrows, uint32_t ntiles,
+                 std::vector<DevBuf<unsigned char>>& staged, PeerHalves* P) {
+    std::memset(P, 0, sizeof *P);
+    P->n = (int)ctx.size();
+    const int owners = ctx.size() < ntiles ? (int)ctx.size() : (int)ntiles;   // the others have no tile
+    const size_t first = (size_t)row0 * width, npix = (size_t)nrows * width;
+    for (int i = 0; i < owners; ++i) {
+        rtc_scene* o = ctx[i];
+        P->a[i] = o->adaptive.half[0].p + first;
+        P->b[i] = o->adaptive.half[1].p + first;
+        P->tile_n[i] = o->adaptive.tile_n.p;
+        if (o == c) continue;
+        CU(cudaStreamWaitEvent(c->multi_stream, o->multi_done, 0));
+        bool mapped;
+        int rc = peer_mapped(c->device, o->device, &mapped);
+        if (rc) return rc;
+        if (mapped) continue;
+        void* a = stage_peer(c->device, o->device, P->a[i], npix * sizeof(float4), c->multi_stream, staged);
+        void* b = a ? stage_peer(c->device, o->device, P->b[i], npix * sizeof(float4), c->multi_stream, staged) : nullptr;
+        void* n = b ? stage_peer(c->device, o->device, P->tile_n[i], ntiles * sizeof(uint32_t), c->multi_stream, staged) : nullptr;
+        if (!n) return RTC_ERR_CUDA;
+        P->a[i] = (const float4*)a;
+        P->b[i] = (const float4*)b;
+        P->tile_n[i] = (const uint32_t*)n;
+    }
+    return RTC_OK;
+}
+}  // namespace
+int rtc_render_adaptive_multi(rtc_scene* s, const int* devices, int ndev, uint32_t seed, float tolerance, uint32_t min_samples,
+                              uint32_t max_samples, uint8_t* rgb_host, float* halves_host, uint32_t* spp_host, uint64_t stats[4]) {
+    if (!s) return fail(RTC_ERR_ARG, "null scene");
+    int rc = check_adaptive_multi_args(tolerance, min_samples, devices, ndev);
+    if (rc) return rc;
+    rc = need_device(s);
     if (rc) return rc;
     const uint32_t width = s->host.cam.width, height = s->host.cam.height;
     const uint32_t npix = width * height, ntiles = adaptive_tiles(width, height);
@@ -1536,43 +1600,12 @@ int rtc_render_adaptive_multi(rtc_scene* s, const int* devices, int ndev, uint32
     std::vector<rtc_scene*> ctx;
     if ((rc = device_contexts(s, devices, ndev, ctx))) return rc;
     rtc_scene* head = ctx[0];
-    std::vector<std::array<uint64_t, 4>> dev_st((size_t)ndev, std::array<uint64_t, 4>{0, 0, 0, 0});
-    auto issue = [&](int i) -> int {
-        rtc_scene* c = ctx[i];
-        CU(cudaSetDevice(c->device));
-        CU(c->multi_stream.ensure());
-        CU(c->multi_done.ensure());
-        int r = adaptive_passes(c, c->multi_stream, (uint32_t)i, (uint32_t)ndev, seed, tolerance, min_samples, smax, dev_st[i].data());
-        if (r) return r;
-        CU(cudaEventRecord(c->multi_done, c->multi_stream));
-        return RTC_OK;
-    };
-    if ((rc = fan_out(ndev, issue))) return rc;
+    if ((rc = adaptive_passes_multi(ctx, seed, tolerance, min_samples, smax, ntiles, st))) return rc;
     // the head device reads the owners' half sums and tile counts in place (peer access), or copies them over
     CU(cudaSetDevice(head->device));
     PeerHalves P;
-    std::memset(&P, 0, sizeof P);
-    P.n = ndev;
-    const int owners = (uint32_t)ndev < ntiles ? ndev : (int)ntiles;   // the others have no tile
     std::vector<DevBuf<unsigned char>> staged;
-    for (int i = 0; i < owners; ++i) {
-        rtc_scene* c = ctx[i];
-        P.a[i] = c->adaptive.half[0].p;
-        P.b[i] = c->adaptive.half[1].p;
-        P.tile_n[i] = c->adaptive.tile_n.p;
-        if (i == 0) continue;
-        CU(cudaStreamWaitEvent(head->multi_stream, c->multi_done, 0));
-        bool mapped;
-        if ((rc = peer_mapped(head->device, c->device, &mapped))) return rc;
-        if (mapped) continue;
-        void* a = stage_peer(head->device, c->device, P.a[i], npix * sizeof(float4), head->multi_stream, staged);
-        void* b = a ? stage_peer(head->device, c->device, P.b[i], npix * sizeof(float4), head->multi_stream, staged) : nullptr;
-        void* n = b ? stage_peer(head->device, c->device, P.tile_n[i], ntiles * sizeof(uint32_t), head->multi_stream, staged) : nullptr;
-        if (!n) return RTC_ERR_CUDA;
-        P.a[i] = (const float4*)a;
-        P.b[i] = (const float4*)b;
-        P.tile_n[i] = (const uint32_t*)n;
-    }
+    if ((rc = owner_halves(head, ctx, width, 0, height, ntiles, staged, &P))) return rc;
     rtc_scene::Adaptive& ad = head->adaptive;
     CU(head->rgb.ensure(nvalues));
     CU(ad.halves.ensure(halves_host ? 6 * (size_t)npix : 0));
@@ -1588,12 +1621,97 @@ int rtc_render_adaptive_multi(rtc_scene* s, const int* devices, int ndev, uint32
     CU(cudaStreamSynchronize(head->multi_stream));
     staged.clear();   // while the head device is current
     CU(cudaSetDevice(s->device));
-    st[2] = ntiles;
-    for (const auto& d : dev_st) {
-        st[0] = std::max(st[0], d[0]);
-        st[1] += d[1];
-        st[3] += d[3];
+    if (stats) std::memcpy(stats, st, sizeof st);
+    return RTC_OK;
+}
+
+// Denoising on several devices: rtc_render_adaptive_multi's passes, then entry i filters the image rows of the tile rows
+// [i T / n, (i + 1) T / n) of k_denoise_nlm's grid (T = ceil(H / kDenoiseTileH)), so that the bands together are the
+// one-device grid block for block.  It reads the rows it filters and kDenoiseApron more on either side from the tiles'
+// owners where they lie, on its own stream and host thread, and copies its rows of the image and the mean to the host.
+int rtc_render_denoised_multi(rtc_scene* s, const int* devices, int ndev, uint32_t seed, float tolerance, uint32_t min_samples,
+                              uint32_t max_samples, float strength, uint8_t* rgb_host, float* mean_host, float* halves_host,
+                              uint32_t* spp_host, uint64_t stats[4]) {
+    if (!s) return fail(RTC_ERR_ARG, "null scene");
+    int rc = check_strength(strength);
+    if (rc) return rc;
+    if ((rc = check_adaptive_multi_args(tolerance, min_samples, devices, ndev))) return rc;
+    const bool deterministic = s->host.dialect <= DIALECT_HW2;
+    const uint32_t smax = max_samples ? max_samples : s->host.samples;
+    if (!deterministic && smax < 2) return fail(RTC_ERR_ARG, "the maximum sample count must be at least 2");
+    if ((rc = need_device(s))) return rc;
+    const uint32_t width = s->host.cam.width, height = s->host.cam.height;
+    const uint32_t npix = width * height, ntiles = adaptive_tiles(width, height);
+    uint64_t st[4] = {0, 0, 0, 0};
+    if (stats) std::memcpy(stats, st, sizeof st);
+    if (npix == 0) return RTC_OK;
+    if (deterministic) {
+        // rtc_render_denoised's unfiltered frame on the first listed device, with rtc_render_adaptive's halves and spp
+        rtc_scene* head = replica_on(s, devices[0], 0);
+        if (!head) return RTC_ERR_CUDA;
+        if ((rc = rtc_render_adaptive(head, seed, tolerance, min_samples, max_samples, rgb_host, halves_host, spp_host, stats))) return rc;
+        if (mean_host) CU(cudaMemcpy(mean_host, head->accum.p, 3 * (size_t)npix * sizeof(float), cudaMemcpyDeviceToHost));
+        CU(cudaSetDevice(s->device));
+        return RTC_OK;
     }
+    std::vector<rtc_scene*> ctx;
+    if ((rc = device_contexts(s, devices, ndev, ctx))) return rc;
+    if ((rc = adaptive_passes_multi(ctx, seed, tolerance, min_samples, smax, ntiles, st))) return rc;
+    const bool filter = strength > 0.f;
+    const float k2 = std::fmin(strength * strength, FLT_MAX);   // as in denoise()
+    const uint32_t tile_rows = (height + kDenoiseTileH - 1) / kDenoiseTileH;
+    auto band = [&](int i) -> int {
+        rtc_scene* c = ctx[i];
+        CU(cudaSetDevice(c->device));
+        const cudaStream_t st_i = c->multi_stream;
+        const LaunchCtx lc{st_i, c->sms};
+        std::vector<DevBuf<unsigned char>> staged;   // freed on return, with c's device current
+        PeerHalves P;
+        int r;
+        if (i == 0 && (halves_host || spp_host)) {
+            // the whole half sums and spp, as rtc_render_adaptive_multi gathers them
+            rtc_scene::Adaptive& ad = c->adaptive;
+            CU(c->rgb.ensure(3 * (size_t)npix));
+            CU(ad.halves.ensure(halves_host ? 6 * (size_t)npix : 0));
+            CU(ad.spp.ensure(spp_host ? npix : 0));
+            if ((r = owner_halves(c, ctx, width, 0, height, ntiles, staged, &P))) return r;
+            launch_resolve_adaptive_peers(lc, P, width, npix, c->rgb.p, halves_host ? ad.halves.p : nullptr, spp_host ? ad.spp.p : nullptr);
+            c->launches++;
+            CU(cudaGetLastError());
+            if (halves_host) CU(cudaMemcpyAsync(halves_host, ad.halves.p, 6 * (size_t)npix * sizeof(float), cudaMemcpyDeviceToHost, st_i));
+            if (spp_host) CU(cudaMemcpyAsync(spp_host, ad.spp.p, (size_t)npix * sizeof(uint32_t), cudaMemcpyDeviceToHost, st_i));
+        }
+        const uint32_t t0 = (uint32_t)((uint64_t)i * tile_rows / ndev), t1 = (uint32_t)((uint64_t)(i + 1) * tile_rows / ndev);
+        if (t0 < t1) {
+            const uint32_t y0 = t0 * kDenoiseTileH, y1 = std::min(height, t1 * kDenoiseTileH);
+            const uint32_t apron = kDenoiseApron;
+            const uint32_t r0 = y0 > apron ? y0 - apron : 0, r1 = std::min(height, y1 + apron);
+            const size_t prep_pix = (size_t)(r1 - r0) * width, out_pix = (size_t)(y1 - y0) * width, out_first = (size_t)(y0 - r0) * width;
+            rtc_scene::Denoise& dn = c->denoise;
+            CU(dn.u.ensure(3 * prep_pix));
+            CU(dn.d.ensure(prep_pix));
+            CU(dn.v.ensure(prep_pix));
+            CU(dn.mean.ensure(3 * out_pix));
+            CU(c->rgb.ensure(3 * out_pix));
+            if ((r = owner_halves(c, ctx, width, r0, r1 - r0, ntiles, staged, &P))) return r;
+            launch_denoise_prep_peers(lc, P, width, r0, r1 - r0, dn.u.p, dn.d.p, dn.v.p, filter ? nullptr : c->rgb.p, (uint32_t)out_first,
+                                      (uint32_t)out_pix);
+            c->launches++;
+            CU(cudaGetLastError());
+            if (filter) {
+                CU(launch_denoise_nlm(lc, dn.u.p, dn.d.p, dn.v.p, width, height, t0, t1 - t0, r0, k2, dn.mean.p, c->rgb.p));
+                c->launches++;
+            }
+            if (rgb_host) CU(cudaMemcpyAsync(rgb_host + 3 * (size_t)y0 * width, c->rgb.p, 3 * out_pix, cudaMemcpyDeviceToHost, st_i));
+            if (mean_host)
+                CU(cudaMemcpyAsync(mean_host + 3 * (size_t)y0 * width, filter ? dn.mean.p : dn.u.p + 3 * out_first,
+                                   3 * out_pix * sizeof(float), cudaMemcpyDeviceToHost, st_i));
+        }
+        CU(cudaStreamSynchronize(st_i));
+        return RTC_OK;
+    };
+    if ((rc = fan_out(ndev, band))) return rc;
+    CU(cudaSetDevice(s->device));
     if (stats) std::memcpy(stats, st, sizeof st);
     return RTC_OK;
 }

@@ -9,6 +9,8 @@
 //               done: all reference leaves a ray touches, then the replay of the reference recursion;
 //   k_shade     recomputes the hit of the winning primitive (normal, interior), applies the material, writes
 //               surviving paths compacted into the next queue.
+#include <cassert>
+
 #include "rt_device.cuh"
 #include "rt_kernels.h"
 
@@ -732,25 +734,44 @@ __global__ void __launch_bounds__(256) k_resolve_adaptive_peers(PeerHalves P, ui
 // Non-local means on the even / odd half sums (Rousselle, Knaus and Zwicker 2012; DESIGN.md "Denoising").  Per pixel
 // with n >= 2 samples: u = 1/n (A + B) (resolve_adaptive_pixel's floats), D = display(u) and, per channel, the variance
 // estimate V = ((display(A / ceil(n/2)) - display(B / floor(n/2))) / 2)^2 (k_adaptive_tiles' half means).  rgb, when
-// given (the filter is not run), gets resolve_adaptive_pixel's image of u.
+// given (the filter is not run), gets resolve_adaptive_pixel's image of u.  One pixel: a / b its even / odd sums, the
+// outputs point at its own u (3 floats), D, V and rgb (3 bytes, or null).
+RT_D void denoise_prep_pixel(const float a[3], const float b[3], uint32_t n, float* u, float4* D, float4* V, uint8_t* rgb) {
+    const float inv = __fdiv_rn(1.f, (float)n), inv_a = __fdiv_rn(1.f, (float)((n + 1) / 2)), inv_b = __fdiv_rn(1.f, (float)(n / 2));
+    float uc[3], dc[3], vc[3];
+#pragma unroll
+    for (int c = 0; c < 3; ++c) {
+        uc[c] = __fmul_rn(inv, __fadd_rn(a[c], b[c]));
+        dc[c] = display(uc[c]);
+        const float e = __fmul_rn(__fsub_rn(display(__fmul_rn(a[c], inv_a)), display(__fmul_rn(b[c], inv_b))), 0.5f);
+        vc[c] = __fmul_rn(e, e);
+        u[c] = uc[c];
+        if (rgb) rgb[c] = to_u8(aces(uc[c]));
+    }
+    *D = make_float4(dc[0], dc[1], dc[2], 0.f);
+    *V = make_float4(vc[0], vc[1], vc[2], 0.f);
+}
 __global__ void __launch_bounds__(256) k_denoise_prep(const float* halves, const uint32_t* spp, uint32_t npix, float* u, float4* D,
                                                        float4* V, uint8_t* rgb) {
     for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < npix; i += gridDim.x * blockDim.x) {
-        const uint32_t n = spp[i];
-        const float inv = __fdiv_rn(1.f, (float)n), inv_a = __fdiv_rn(1.f, (float)((n + 1) / 2)), inv_b = __fdiv_rn(1.f, (float)(n / 2));
         const float* h = halves + 6 * (size_t)i;
-        float uc[3], dc[3], vc[3];
-#pragma unroll
-        for (int c = 0; c < 3; ++c) {
-            uc[c] = __fmul_rn(inv, __fadd_rn(h[c], h[3 + c]));
-            dc[c] = display(uc[c]);
-            const float e = __fmul_rn(__fsub_rn(display(__fmul_rn(h[c], inv_a)), display(__fmul_rn(h[3 + c], inv_b))), 0.5f);
-            vc[c] = __fmul_rn(e, e);
-            u[3 * (size_t)i + c] = uc[c];
-            if (rgb) rgb[3 * (size_t)i + c] = to_u8(aces(uc[c]));
-        }
-        D[i] = make_float4(dc[0], dc[1], dc[2], 0.f);
-        V[i] = make_float4(vc[0], vc[1], vc[2], 0.f);
+        const float a[3] = {h[0], h[1], h[2]}, b[3] = {h[3], h[4], h[5]};
+        denoise_prep_pixel(a, b, spp[i], u + 3 * (size_t)i, D + i, V + i, rgb ? rgb + 3 * (size_t)i : nullptr);
+    }
+}
+// The same for the rows [row0, row0 + npix / width) of a multi-device adaptive render, straight from the owners' half sums
+// (k_resolve_adaptive_peers' ownership: tile t is device t % P.n's).  P.a / P.b point at those rows' first pixel, P.tile_n
+// at whole tile-count arrays; u, D and V are band-local.  rgb, when given, gets the image of the pixels
+// [rgb_first, rgb_first + rgb_count) of the band.
+__global__ void __launch_bounds__(256) k_denoise_prep_peers(PeerHalves P, uint32_t width, uint32_t row0, uint32_t npix, float* u,
+                                                             float4* D, float4* V, uint8_t* rgb, uint32_t rgb_first, uint32_t rgb_count) {
+    const uint32_t tiles_x = (width + kAdaptiveTile - 1) / kAdaptiveTile;
+    for (uint32_t j = blockIdx.x * blockDim.x + threadIdx.x; j < npix; j += gridDim.x * blockDim.x) {
+        const uint32_t t = tile_of(row0 * width + j, width, tiles_x), d = t % (uint32_t)P.n;
+        const float4 fa = P.a[d][j], fb = P.b[d][j];
+        const float a[3] = {fa.x, fa.y, fa.z}, b[3] = {fb.x, fb.y, fb.z};
+        const bool out = rgb && j - rgb_first < rgb_count;
+        denoise_prep_pixel(a, b, P.tile_n[d][t], u + 3 * (size_t)j, D + j, V + j, out ? rgb + 3 * (size_t)(j - rgb_first) : nullptr);
     }
 }
 // One block filters a kDenoiseTileW x kDenoiseTileH tile of pixels.  It stages D and the smoothed V (the mean of V over
@@ -759,7 +780,10 @@ __global__ void __launch_bounds__(256) k_denoise_prep(const float* halves, const
 // outside the image, so that such neighbours fail the finiteness test), then walks the (2R+1)^2 offsets: per offset
 // the distance term of every pixel of the tile plus F, a row box sum of width 2F+1, and per pixel the column box sum,
 // the weight and the weighted sums in registers.  Two barriers per offset; each thread owns two pixels of a column.
+// The grid covers the tile rows [tile_row0, tile_row0 + gridDim.y) (a band of a multi-device filter; the whole frame is
+// (0, 0)); u, D and V hold the image rows [buf_row0, min(H, band end + kDenoiseApron)), mean and rgb the band's rows.
 constexpr int kDnR = kDenoiseRadius, kDnF = kDenoisePatch, kDnS = kDenoiseVarRadius, kDnA = kDnR + kDnF;
+static_assert(kDenoiseApron == kDnA + kDnS, "k_denoise_nlm: the rows a block reads beyond its tile");
 constexpr int kDnTW = kDenoiseTileW, kDnTH = kDenoiseTileH, kDnThreads = 256, kDnRows = kDnThreads / kDnTW;
 constexpr int kDnSW = kDnTW + 2 * kDnA, kDnSH = kDnTH + 2 * kDnA;   // D, V staging
 constexpr int kDnUW = kDnTW + 2 * kDnR, kDnUH = kDnTH + 2 * kDnR;   // u staging
@@ -768,21 +792,26 @@ constexpr int kDnPix = kDnTH / kDnRows;                              // pixels p
 static_assert(kDnTW == 32 && kDnTH % kDnRows == 0, "k_denoise_nlm: a warp per tile row");
 constexpr size_t kDenoiseSmemFloats = 6 * (size_t)kDnSW * kDnSH + 3 * (size_t)kDnUW * kDnUH + kDnEW * kDnEH + kDnTW * kDnEH;
 __global__ void __launch_bounds__(kDnThreads) k_denoise_nlm(const float* u, const float4* D, const float4* V, uint32_t width,
-                                                             uint32_t height, float k2, float* mean, uint8_t* rgb) {
+                                                             uint32_t height, uint32_t tile_row0, uint32_t buf_row0, float k2,
+                                                             float* mean, uint8_t* rgb) {
     extern __shared__ float smem[];
     float* sD = smem;                              // [3][kDnSH][kDnSW]
     float* sV = sD + 3 * kDnSW * kDnSH;            // [3][kDnSH][kDnSW]
     float* sU = sV + 3 * kDnSW * kDnSH;            // [3][kDnUH][kDnUW]
     float* sT = sU + 3 * kDnUW * kDnUH;            // [kDnEH][kDnEW]
     float* sH = sT + kDnEW * kDnEH;                // [kDnEH][kDnTW]
-    const int x0 = blockIdx.x * kDnTW, y0 = blockIdx.y * kDnTH, W = (int)width, H = (int)height;
+    const int x0 = blockIdx.x * kDnTW, y0 = (tile_row0 + blockIdx.y) * kDnTH, W = (int)width, H = (int)height;
+    const int band0 = tile_row0 * kDnTH, r0 = (int)buf_row0;
+    // the rows read below: D and the centres of V's boxes within A of the tile, V's boxes S further, u within R
+    assert(max(y0 - kDnA - kDnS, 0) >= r0 &&
+           min(y0 + kDnTH + kDnA + kDnS, H) <= min(min((int)(tile_row0 + gridDim.y) * kDnTH, H) + kDenoiseApron, H));
     for (int i = threadIdx.x; i < kDnSW * kDnSH; i += kDnThreads) {
         const int gx = min(max(x0 - kDnA + i % kDnSW, 0), W - 1), gy = min(max(y0 - kDnA + i / kDnSW, 0), H - 1);
-        const float4 d = D[(size_t)gy * W + gx];
+        const float4 d = D[(size_t)(gy - r0) * W + gx];
         float4 v = make_float4(0.f, 0.f, 0.f, 0.f);   // V smoothed over the (2S+1)^2 box around (gx, gy), clamped
         for (int oy = -kDnS; oy <= kDnS; ++oy)
             for (int ox = -kDnS; ox <= kDnS; ++ox) {
-                const float4 t = V[(size_t)min(max(gy + oy, 0), H - 1) * W + min(max(gx + ox, 0), W - 1)];
+                const float4 t = V[(size_t)(min(max(gy + oy, 0), H - 1) - r0) * W + min(max(gx + ox, 0), W - 1)];
                 v.x += t.x; v.y += t.y; v.z += t.z;
             }
         constexpr float inv_box = 1.f / ((2 * kDnS + 1) * (2 * kDnS + 1));
@@ -794,7 +823,7 @@ __global__ void __launch_bounds__(kDnThreads) k_denoise_nlm(const float* u, cons
         const int gx = x0 - kDnR + i % kDnUW, gy = y0 - kDnR + i / kDnUW;
         const bool in = gx >= 0 && gx < W && gy >= 0 && gy < H;
 #pragma unroll
-        for (int c = 0; c < 3; ++c) sU[i + c * kDnUW * kDnUH] = in ? u[3 * ((size_t)gy * W + gx) + c] : __int_as_float(0x7fc00000);
+        for (int c = 0; c < 3; ++c) sU[i + c * kDnUW * kDnUH] = in ? u[3 * ((size_t)(gy - r0) * W + gx) + c] : __int_as_float(0x7fc00000);
     }
     __syncthreads();
     const int tx = threadIdx.x % kDnTW, ty = threadIdx.x / kDnTW;
@@ -849,7 +878,7 @@ __global__ void __launch_bounds__(kDnThreads) k_denoise_nlm(const float* u, cons
         const int ip = (ty + j * kDnRows + kDnR) * kDnUW + tx + kDnR;
         float up[3] = {sU[ip], sU[ip + kDnUW * kDnUH], sU[ip + 2 * kDnUW * kDnUH]};
         const bool finite = isfinite(up[0]) && isfinite(up[1]) && isfinite(up[2]);   // else it passes through
-        const size_t i = (size_t)y * W + x;
+        const size_t i = (size_t)(y - band0) * W + x;
 #pragma unroll
         for (int c = 0; c < 3; ++c) {
             const float v = finite ? __fdiv_rn(su[j][c], sw[j]) : up[c];
@@ -983,13 +1012,18 @@ void launch_denoise_prep(const LaunchCtx& c, const float* halves, const uint32_t
                          uint8_t* rgb) {
     k_denoise_prep<<<grid_for(npix, 256, c.sms, 8), 256, 0, c.stream>>>(halves, spp, npix, u, D, V, rgb);
 }
+void launch_denoise_prep_peers(const LaunchCtx& c, const PeerHalves& P, uint32_t width, uint32_t row0, uint32_t nrows, float* u,
+                               float4* D, float4* V, uint8_t* rgb, uint32_t rgb_first, uint32_t rgb_count) {
+    const uint32_t npix = width * nrows;
+    k_denoise_prep_peers<<<grid_for(npix, 256, c.sms, 8), 256, 0, c.stream>>>(P, width, row0, npix, u, D, V, rgb, rgb_first, rgb_count);
+}
 cudaError_t launch_denoise_nlm(const LaunchCtx& c, const float* u, const float4* D, const float4* V, uint32_t width, uint32_t height,
-                               float k2, float* mean, uint8_t* rgb) {
+                               uint32_t tile_row0, uint32_t tile_rows, uint32_t buf_row0, float k2, float* mean, uint8_t* rgb) {
     const size_t bytes = kDenoiseSmemFloats * sizeof(float);
     cudaError_t e = cudaFuncSetAttribute(k_denoise_nlm, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
     if (e != cudaSuccess) return e;
-    const dim3 grid((width + kDnTW - 1) / kDnTW, (height + kDnTH - 1) / kDnTH);
-    k_denoise_nlm<<<grid, kDnThreads, bytes, c.stream>>>(u, D, V, width, height, k2, mean, rgb);
+    const dim3 grid((width + kDnTW - 1) / kDnTW, tile_rows);
+    k_denoise_nlm<<<grid, kDnThreads, bytes, c.stream>>>(u, D, V, width, height, tile_row0, buf_row0, k2, mean, rgb);
     return cudaGetLastError();
 }
 void launch_pre(const LaunchCtx& c, const DevScene& S, PathSoA P, HitSoA H, const uint32_t* qcount, uint32_t max_count,

@@ -43,13 +43,17 @@ void launch_resolve_adaptive(const LaunchCtx& c, const float4* A, const float4* 
 constexpr int kDenoiseRadius = 7, kDenoisePatch = 3, kDenoiseVarRadius = 1;
 constexpr float kDenoiseAlpha = 1.f, kDenoiseEps = 1e-8f;
 constexpr int kDenoiseTileW = 32, kDenoiseTileH = 16;
+// the rows of u, D and V beyond its tile that a filter block reads: the window and the patch, then the box around V
+constexpr int kDenoiseApron = kDenoiseRadius + kDenoisePatch + kDenoiseVarRadius;
 // per pixel from the half sums (6 floats) and spp (>= 2): the linear mean u (3 floats), D = display(u) and the variance
 // estimate V (float4, w unused); rgb (optional) = the 8-bit image of u
 void launch_denoise_prep(const LaunchCtx& c, const float* halves, const uint32_t* spp, uint32_t npix, float* u, float4* D, float4* V,
                          uint8_t* rgb);
-// the filter with k2 = strength^2: mean (3 floats per pixel) and its 8-bit image
+// the filter with k2 = strength^2 on the tile rows [tile_row0, tile_row0 + tile_rows) of kDenoiseTileH pixels: mean (3
+// floats per pixel) and its 8-bit image, from the first row of the band on; u, D and V hold the image rows [buf_row0,
+// min(height, band end + kDenoiseApron)).  The whole frame: (0, ceil(height / kDenoiseTileH), 0).
 cudaError_t launch_denoise_nlm(const LaunchCtx& c, const float* u, const float4* D, const float4* V, uint32_t width, uint32_t height,
-                               float k2, float* mean, uint8_t* rgb);
+                               uint32_t tile_row0, uint32_t tile_rows, uint32_t buf_row0, float k2, float* mean, uint8_t* rgb);
 // Scene::RayIntersection for the rays of queue P (fills H): launch_pre then launch_traverse
 // (index BVH), or launch_extend_reftree alone (the reference-tree twin).
 void launch_pre(const LaunchCtx& c, const DevScene& S, PathSoA P, HitSoA H, const uint32_t* qcount, uint32_t max_count,
@@ -89,6 +93,11 @@ struct PeerHalves {
 };
 void launch_resolve_adaptive_peers(const LaunchCtx& c, const PeerHalves& P, uint32_t width, uint32_t npix, uint8_t* out, float* halves,
                                    uint32_t* spp);
+// launch_denoise_prep for the image rows [row0, row0 + nrows) of such a render (P.a / P.b point at row row0, P.tile_n at
+// the whole tile counts); u, D and V are band-local, rgb (optional) gets the pixels [rgb_first, rgb_first + rgb_count)
+// of the band
+void launch_denoise_prep_peers(const LaunchCtx& c, const PeerHalves& P, uint32_t width, uint32_t row0, uint32_t nrows, float* u,
+                               float4* D, float4* V, uint8_t* rgb, uint32_t rgb_first, uint32_t rgb_count);
 void launch_pack_rays(const LaunchCtx& c, long n, const float* o, const float* d, PathSoA P, uint32_t* q);
 void launch_unpack_hits(const LaunchCtx& c, const DevScene& S, long n, PathSoA P, HitSoA H, int32_t* id, float* t, float* nrm,
                         int32_t* interior);
