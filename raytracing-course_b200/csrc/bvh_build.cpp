@@ -131,6 +131,9 @@ struct RefBuilder {
                 break;
             }
         }
+        // No cut costs less than kInf, but the leaf costs more (or is NaN): boxes whose surface areas reach 1e18.  The
+        // reference then builds an empty child and recurses on the same range until its stack overflows.
+        if (cut == 0) throw std::runtime_error("the SAH finds no cut below 1e18 for a BVH node that is too costly as a leaf (primitive boxes too large)");
         if (par > 0 && last - first >= 4096) {
             std::vector<RefNode> lhs, rhs;
             auto other = std::async(std::launch::async, [&] { build(lhs, first, cut, par - 1); });

@@ -13,6 +13,7 @@ import pytest
 
 import orclib
 from conftest import golden, scene_path
+from test_limits import CLOSED_ROOM, fence, triangle_stack
 
 pytestmark = pytest.mark.gpu
 
@@ -319,7 +320,16 @@ EDGE_SCENES = {
                       "NEW_PRIMITIVE\nBOX 3 2 0.1\nPOSITION 0 1 -2\nROTATION 0 0.0871557 0 0.9961947\nMETALLIC\nCOLOR 0.9 0.9 0.9\n\n"
                       "NEW_PRIMITIVE\nELLIPSOID 0.3 0.2 0.3\nPOSITION 2 3 1\nROTATION 0.2 0.1 0 0.9746794\nEMISSION 8 7 6\n\n"
                       "NEW_PRIMITIVE\nPLANE 0 1 0\nCOLOR 0.6 0.6 0.6\n",
+    # rays along the axis record 25 leaves with a hit, one more than the index traversal keeps: they walk the reference
+    # tree instead (test_limits.py checks that they do)
+    "fence_25": fence(25),
+    "triangle_stack_25": triangle_stack(25),
+    # RAY_DEPTH 62: nearly every path takes all 62 bounces
+    "closed_room_depth_62": CLOSED_ROOM,
 }
+# paths whose length or direction turns on rounding: Fresnel coin flips and total internal reflection in the chain;
+# 62 bounces, some off a curved mirror, in the room
+CHAOTIC_EDGE_SCENES = ("specular_chain", "closed_room_depth_62")
 
 
 @pytest.mark.parametrize("name", sorted(EDGE_SCENES))
@@ -348,7 +358,7 @@ def test_edge_scenes_vs_oracle(rtc, oracle_lib, name):
     assert c["paths"] == paths
     # deep specular chains amplify rounding differences (total-internal-reflection thresholds, Fresnel
     # coin flips): path lengths then differ on a fraction of a percent of the paths
-    chaotic = name == "specular_chain"
+    chaotic = name in CHAOTIC_EDGE_SCENES
     assert abs(c["rays"] - rays) <= (1e-2 if chaotic else 2e-3) * rays + 2
     ok = np.isfinite(ref).all(1) & np.isfinite(got).all(1)
     rel = np.abs(got - ref).max(1) / (np.abs(ref).max(1) + 1e-3)
