@@ -73,6 +73,15 @@ int rtc_scene_arena_check(rtc_scene* s, uint64_t* mismatching_bytes);
 int rtc_scene_stats(const rtc_scene* s, uint64_t out[8]);
 /* DIMENSIONS / SAMPLES / RAY_DEPTH overrides (value < 0 keeps the file's) */
 int rtc_scene_override(rtc_scene* s, int width, int height, int samples, int ray_depth);
+/* ---- camera override: every later call of the scene (renders, adaptive, denoised, multi-device, rtc_camera_rays,
+ *      rtc_frame_begin) uses the camera set here instead of the file's.  width and height stay (rtc_scene_override).
+ *      Works on host-only scenes too.  RTC_ERR_ARG, before any change: a null pointer, a value that is not finite, or
+ *      fov_x outside (0, pi).  A camera whose |position|inf exceeds the extent the index BVH was built for rebuilds the
+ *      index BVH for it and uploads the scene again (DESIGN.md "Camera views"). */
+/* camera: position3 right3 up3 forward3 fov_x (radians, as CAMERA_FOV_X) */
+#define RTC_CAMERA_FLOATS 13
+int rtc_scene_camera(const rtc_scene* s, float out[13]);
+int rtc_scene_set_camera(rtc_scene* s, const float cam[13]);
 /* final primitive order after std::partition + the BVH sorts (scene.cpp:17, bvh.cpp:129,168):
  * original file index of every slot; and the per-primitive record type,material + 26 floats
  * (col3 emission3 pos3 rot4(xyzw) ior d0(3) d1(3) d2(3) pad3) */
@@ -135,6 +144,17 @@ int rtc_render_u8(rtc_scene* s, uint32_t seed, uint8_t* rgb_host);
 int rtc_render_sum(rtc_scene* s, uint32_t seed, uint32_t sample_begin, uint32_t sample_count, float* sum_host);
 /* run.sh <scene> <out.ppm> in one call: "P6\nW H\n255\n" + bytes (src/scene.cpp:206-208,243-251) */
 int rtc_render_ppm(rtc_scene* s, uint32_t seed, const char* out_path);
+/* ---- batched views: one render of several cameras of the scene, sharing the wavefront batches.  View v samples the
+ *      Philox streams of a render with camera v set (rtc_scene_set_camera), so its sums equal those up to float summation
+ *      order.  hw1 / hw2 render one deterministic frame per view.  1 <= nviews <= 4096 and nviews * W * H <= 2^28, else
+ *      RTC_ERR_UNSUPPORTED; a bad camera in the list is RTC_ERR_ARG; both are checked before any device call.  A view
+ *      beyond the index BVH's extent rebuilds it, as rtc_scene_set_camera does.  rtc_render_counters paths grow by
+ *      nviews * W * H * sample_count. */
+/* nviews cameras (13 floats each); view v's pixel sums at accum_dev + 3 * v * W * H */
+int rtc_render_views_accumulate(rtc_scene* s, const float* cams_host, int nviews, uint32_t seed, uint32_t sample_begin,
+                                uint32_t sample_count, float* accum_dev, void* stream);
+/* the scene's SAMPLES for every view: nviews 8-bit images (3*W*H bytes each); sum_host optional (3*W*H floats each) */
+int rtc_render_views_u8(rtc_scene* s, const float* cams_host, int nviews, uint32_t seed, uint8_t* rgb_host, float* sum_host);
 /* ---- adaptive sampling: Scene::Render with a noise threshold instead of a fixed sample count per pixel (single
  *      device).  The frame is cut into RTC_ADAPTIVE_TILE x RTC_ADAPTIVE_TILE tiles (partial at the right and bottom
  *      edges).  Every tile starts with samples [0, n0), n0 = min(min_samples, max); a pass renders [n, target) for each

@@ -45,6 +45,8 @@ _SIGNATURES = {
     "rtc_scene_info": (C.c_int, [C.c_void_p, _u32]),
     "rtc_scene_stats": (C.c_int, [C.c_void_p, _u64]),
     "rtc_scene_override": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int]),
+    "rtc_scene_camera": (C.c_int, [C.c_void_p, _f32]),
+    "rtc_scene_set_camera": (C.c_int, [C.c_void_p, _f32]),
     "rtc_scene_prim_order": (C.c_int, [C.c_void_p, _i32]),
     "rtc_scene_prims": (C.c_int, [C.c_void_p, _i32, _f32]),
     "rtc_scene_nodes": (C.c_int, [C.c_void_p, _f32, _u32]),
@@ -74,6 +76,9 @@ _SIGNATURES = {
     "rtc_render_u8": (C.c_int, [C.c_void_p, C.c_uint32, _u8]),
     "rtc_render_sum": (C.c_int, [C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, _f32]),
     "rtc_render_ppm": (C.c_int, [C.c_void_p, C.c_uint32, C.c_char_p]),
+    "rtc_render_views_accumulate": (C.c_int, [C.c_void_p, _f32, C.c_int, C.c_uint32, C.c_uint32, C.c_uint32, C.c_void_p,
+                                              C.c_void_p]),
+    "rtc_render_views_u8": (C.c_int, [C.c_void_p, _f32, C.c_int, C.c_uint32, _u8, C.c_void_p]),
     "rtc_render_adaptive": (C.c_int, [C.c_void_p, C.c_uint32, C.c_float, C.c_uint32, C.c_uint32, _u8, _f32, _u32, _u64]),
     "rtc_render_adaptive_multi": (C.c_int, [C.c_void_p, _i32, C.c_int, C.c_uint32, C.c_float, C.c_uint32, C.c_uint32, _u8, _f32,
                                             _u32, _u64]),
@@ -125,6 +130,31 @@ def _check(lib, rc):
 
 def device_count():
     return load_library().rtc_device_count()
+
+
+CAMERA_FLOATS = 13   # position3 right3 up3 forward3 fov_x (rtc_b200.h RTC_CAMERA_FLOATS)
+
+
+def _camera_floats(pos=None, right=None, up=None, forward=None, fov_x=None, cam=None):
+    """One camera as the 13 float32 of the C-ABI: either `cam` (13 values) or pos / right / up / forward (3 each) and
+    fov_x (radians, as CAMERA_FOV_X)."""
+    if cam is None:
+        parts = [np.asarray(v, np.float32).reshape(-1) for v in (pos, right, up, forward)]
+        if any(p.size != 3 for p in parts) or fov_x is None:
+            raise ValueError("a camera needs pos, right, up, forward (3 floats each) and fov_x")
+        cam = np.concatenate(parts + [np.asarray([fov_x], np.float32)])
+    cam = np.ascontiguousarray(cam, np.float32).reshape(-1)
+    if cam.size != CAMERA_FLOATS:
+        raise ValueError("a camera is %d floats, got %d" % (CAMERA_FLOATS, cam.size))
+    return cam
+
+
+def _cameras(cameras):
+    """V cameras of 13 floats each as a (V, 13) float32 array."""
+    cams = np.ascontiguousarray(cameras, np.float32)
+    if cams.ndim != 2 or cams.shape[1] != CAMERA_FLOATS:
+        raise ValueError("expected cameras of %d floats each, got shape %s" % (CAMERA_FLOATS, cams.shape))
+    return cams
 
 
 def _c3(a):
@@ -230,6 +260,17 @@ class Scene:
         _check(self.lib, self.lib.rtc_scene_override(self.h, width, height, samples, ray_depth))
         self._refresh()
 
+    def camera(self):
+        """The camera the scene renders with: 13 float32, position3 right3 up3 forward3 fov_x."""
+        out = np.zeros(CAMERA_FLOATS, np.float32)
+        _check(self.lib, self.lib.rtc_scene_camera(self.h, out))
+        return out
+
+    def set_camera(self, cam=None, pos=None, right=None, up=None, forward=None, fov_x=None):
+        """Render from another camera (rtc_scene_set_camera): 13 floats, or pos / right / up / forward and fov_x.  The
+        frame size stays; a camera beyond the index BVH's extent rebuilds it."""
+        _check(self.lib, self.lib.rtc_scene_set_camera(self.h, _camera_floats(pos, right, up, forward, fov_x, cam)))
+
     def prim_order(self):
         out = np.zeros(self.nprims, np.int32)
         _check(self.lib, self.lib.rtc_scene_prim_order(self.h, out))
@@ -303,6 +344,25 @@ class Scene:
         out = np.zeros((self.height, self.width, 3), np.uint8)
         _check(self.lib, self.lib.rtc_render_u8(self.h, seed, out))
         return out
+
+    def RenderViews(self, cameras, seed=0, want_sum=False):
+        """Scene::Render of every camera in `cameras` (V cameras of 13 floats) in one
+        batched wavefront (rtc_render_views_u8).  Returns (V, H, W, 3) uint8, and the (V, H, W, 3) float32 sums with
+        want_sum.  View v equals set_camera(cameras[v]) + Render up to float summation order."""
+        cams = _cameras(cameras)
+        nv = cams.shape[0]
+        out = np.zeros((nv, self.height, self.width, 3), np.uint8)
+        total = np.zeros((nv, self.height, self.width, 3), np.float32) if want_sum else None
+        _check(self.lib, self.lib.rtc_render_views_u8(self.h, cams, nv, seed, out,
+                                                      total.ctypes.data_as(C.c_void_p) if want_sum else None))
+        return (out, total) if want_sum else out
+
+    def render_views_accumulate(self, accum_ptr, cameras, seed, sample_begin, sample_count, stream=None):
+        """Device-pointer variant of RenderViews: adds the sums of samples [sample_begin, sample_begin + sample_count)
+        of view v at float offset 3 * v * W * H of a float32 device buffer."""
+        cams = _cameras(cameras)
+        _check(self.lib, self.lib.rtc_render_views_accumulate(self.h, cams, cams.shape[0], seed, sample_begin, sample_count,
+                                                               C.c_void_p(accum_ptr), C.c_void_p(stream or 0)))
 
     def RenderAdaptive(self, tolerance, min_samples=16, max_samples=0, seed=0):
         """Scene::Render with a noise threshold (rtc_render_adaptive): each 8x8 tile takes samples until the difference

@@ -652,7 +652,6 @@ void HostScene::init() {
     F.rnodes.resize(2 * (size_t)nn);
     F.rmeta.resize(nn);
     std::vector<uint32_t> depth(nn, 0);
-    std::vector<Unit> units;
     if (nn > 0) {
         std::vector<uint32_t> stack{root};
         while (!stack.empty()) {
@@ -667,14 +666,6 @@ void HostScene::init() {
             if (nd.left == UINT32_MAX) {
                 F.rmeta[v] = u4{nd.first, nd.count, depth[v], 0};
                 if (nd.count > IREF_MAX_LEAF_PRIMS) throw std::runtime_error("a BVH leaf holds more than 64 primitives");
-                if (nd.count > 0) {
-                    const Primitive& p0 = prims[nd.first];
-                    bool ident = p0.rot.x == 0.f && p0.rot.y == 0.f && p0.rot.z == 0.f && p0.rot.w == 1.f &&
-                                 p0.pos.x == 0.f && p0.pos.y == 0.f && p0.pos.z == 0.f;
-                    bool fast = nd.count == 1 && p0.type == PT_TRIANGLE && ident;
-                    units.push_back(Unit{nd.box, nd.first, nd.count, 0.5f * (nd.box.mx + nd.box.mn), fast,
-                                         cone_of_leaf(prims, nd.first, nd.count, nd.box)});
-                }
             } else {
                 F.rmeta[v] = u4{nd.first, nodes[nd.right].first, depth[v], 0};
                 depth[nd.left] = depth[nd.right] = depth[v] + 1;
@@ -683,34 +674,8 @@ void HostScene::init() {
             }
         }
     }
-    std::sort(units.begin(), units.end(), [](const Unit& a, const Unit& b) { return a.first < b.first; });
-    F.units = (uint32_t)units.size();
-    F.ubox.assign(2 * (size_t)n, f4{0, 0, 0, 0});
-    for (const Unit& u : units) {
-        F.ubox[2 * (size_t)u.first] = f4{u.box.mn.x, u.box.mn.y, u.box.mn.z, 0.f};
-        F.ubox[2 * (size_t)u.first + 1] = f4{u.box.mx.x, u.box.mx.y, u.box.mx.z, 0.f};
-    }
-
-    timer.lap("reference nodes, units, cones");
-    // ---- index BVH
-    F.inodes.clear();
-    F.iroot = IREF_NONE;
-    if (!units.empty()) {
-        IndexBuilder ib{units, F.inodes, std::vector<float>(units.size() + 1, 0.f)};
-        double extent = std::max({std::fabs((double)cam.pos.x), std::fabs((double)cam.pos.y), std::fabs((double)cam.pos.z)});
-        for (const Unit& u : units)
-            for (float v : {u.box.mn.x, u.box.mn.y, u.box.mn.z, u.box.mx.x, u.box.mx.y, u.box.mx.z})
-                if (std::isfinite(v)) extent = std::max(extent, (double)std::fabs(v));
-        ib.slack = extent * (1.0 / 1048576.0);
-        ib.prepare();
-        timer.lap("index BVH: presort");
-        Cone whole;
-        uint32_t broot = ib.build(ib.tmp, 0, (uint32_t)units.size(), 0, whole, build_parallel_levels());
-        timer.lap("index BVH: sweep build");
-        F.iroot = (broot & IREF_LEAF) ? broot : ib.emit(broot, 1);
-        timer.lap("index BVH: collapse + emit");
-        F.index_depth = ib.wide_depth;
-    }
+    timer.lap("reference nodes");
+    build_index(std::max({std::fabs((double)cam.pos.x), std::fabs((double)cam.pos.y), std::fabs((double)cam.pos.z)}));
 
     // ---- LCA table: for a cut position c (boundary between primitive c-1 and c) the inner node
     // that splits there; range-min by depth over positions gives the lowest common ancestor of
@@ -736,6 +701,53 @@ void HostScene::init() {
         }
     }
     timer.lap("LCA table");
+}
+
+void HostScene::build_index(double cam_extent) {
+    PhaseTimer timer;
+    FlatScene& F = flat;
+    const uint32_t n = (uint32_t)prims.size();
+    std::vector<Unit> units;
+    for (const RefNode& nd : nodes) {
+        if (nd.left != UINT32_MAX || nd.count == 0) continue;
+        const Primitive& p0 = prims[nd.first];
+        bool ident = p0.rot.x == 0.f && p0.rot.y == 0.f && p0.rot.z == 0.f && p0.rot.w == 1.f &&
+                     p0.pos.x == 0.f && p0.pos.y == 0.f && p0.pos.z == 0.f;
+        bool fast = nd.count == 1 && p0.type == PT_TRIANGLE && ident;
+        units.push_back(Unit{nd.box, nd.first, nd.count, 0.5f * (nd.box.mx + nd.box.mn), fast,
+                             cone_of_leaf(prims, nd.first, nd.count, nd.box)});
+    }
+    // leaves start at distinct slots: the order does not depend on the order of the node walk
+    std::sort(units.begin(), units.end(), [](const Unit& a, const Unit& b) { return a.first < b.first; });
+    F.units = (uint32_t)units.size();
+    F.ubox.assign(2 * (size_t)n, f4{0, 0, 0, 0});
+    for (const Unit& u : units) {
+        F.ubox[2 * (size_t)u.first] = f4{u.box.mn.x, u.box.mn.y, u.box.mn.z, 0.f};
+        F.ubox[2 * (size_t)u.first + 1] = f4{u.box.mx.x, u.box.mx.y, u.box.mx.z, 0.f};
+    }
+
+    timer.lap("units, cones");
+    // ---- index BVH
+    F.inodes.clear();
+    F.iroot = IREF_NONE;
+    F.index_depth = 0;
+    double extent = cam_extent;
+    for (const Unit& u : units)
+        for (float v : {u.box.mn.x, u.box.mn.y, u.box.mn.z, u.box.mx.x, u.box.mx.y, u.box.mx.z})
+            if (std::isfinite(v)) extent = std::max(extent, (double)std::fabs(v));
+    F.index_extent = extent;
+    if (!units.empty()) {
+        IndexBuilder ib{units, F.inodes, std::vector<float>(units.size() + 1, 0.f)};
+        ib.slack = extent * (1.0 / 1048576.0);
+        ib.prepare();
+        timer.lap("index BVH: presort");
+        Cone whole;
+        uint32_t broot = ib.build(ib.tmp, 0, (uint32_t)units.size(), 0, whole, build_parallel_levels());
+        timer.lap("index BVH: sweep build");
+        F.iroot = (broot & IREF_LEAF) ? broot : ib.emit(broot, 1);
+        timer.lap("index BVH: collapse + emit");
+        F.index_depth = ib.wide_depth;
+    }
 }
 
 }  // namespace rtc

@@ -142,6 +142,8 @@ struct rtc_scene {
     DevBuf<float4> accum4[2];
     Event accum4_idle[2];
     int accum4_next = 0;
+    // the camera records of a batched render (rtc_render_views_accumulate), one set per float4 sum buffer, reused with it
+    DevBuf<DevCamera> views[2];
     // probe entry points (rtc_intersect, ...): staging buffers that only ever grow
     struct Probe {
         DevBuf<float> fin[3];
@@ -389,8 +391,10 @@ int prepare_arena(rtc_scene* s) {
         CU(s->accum4_idle[a].ensure());
     }
     CU(s->copy_stream.ensure());
-    CU(s->stats.ensure(kStatWords));
-    CU(cudaMemset(s->stats.p, 0, kStatWords * sizeof(unsigned long long)));
+    if (!s->stats.p) {   // the counters survive a new layout of the arena (rebuild_arenas)
+        CU(s->stats.ensure(kStatWords));
+        CU(cudaMemset(s->stats.p, 0, kStatWords * sizeof(unsigned long long)));
+    }
     lap("arena: cudaMalloc, pinned mirror");
     return RTC_OK;
 }
@@ -590,11 +594,16 @@ int ensure_wavefront(rtc_scene* s, uint64_t cap, int nlanes) {
 
 // Which (pixel, sample) path p of a render is: pixel p % npix of the frame and sample sample_first + p / npix when
 // plist is null (rtc_render_accumulate), else pixel plist[p % npix] and sample sample_first + 2 (p / npix) (an adaptive
-// pass renders the even or the odd samples of its pixel list)
+// pass renders the even or the odd samples of its pixel list).  With `views` (rtc_render_views_accumulate, no plist):
+// pixel p % npix of view (p / npix) % nviews, sample sample_first + p / (npix nviews), deposited at view npix + pixel;
+// view_recip is k_shade's reciprocal of npix (launch_shade).
 struct PathMap {
     const uint32_t* plist;
     uint32_t npix;
     uint32_t sample_first;
+    const DevCamera* views = nullptr;
+    uint32_t nviews = 1;
+    uint64_t view_recip = 0;
 };
 // fork: the lane streams of the next render_paths calls start after everything already queued on the caller's stream
 int fork_lanes(rtc_scene* s, cudaStream_t user) {
@@ -651,7 +660,7 @@ int render_paths(rtc_scene* s, const DevScene& S, uint32_t seed, const PathMap& 
         HitSoA hcur{L.hit_id[0].p}, hnxt{L.hit_id[1].p};
         s->span_begin(0, st);
         if (map.plist) launch_generate_list(c, S, cur, hcur, L.queue.p, L.trav_queue.p, tqc, first, count, seed, map.plist, map.npix, map.sample_first);
-        else launch_generate(c, S, cur, hcur, L.queue.p, L.trav_queue.p, tqc, first, count, seed, map.sample_first);
+        else launch_generate(c, S, cur, hcur, L.queue.p, L.trav_queue.p, tqc, first, count, seed, map.sample_first, map.views, map.nviews);
         s->span_end(st);
         s->launches++;
         for (uint32_t b = 1; b <= depth; ++b) {
@@ -661,7 +670,7 @@ int render_paths(rtc_scene* s, const DevScene& S, uint32_t seed, const PathMap& 
             s->span_end(st);
             s->span_begin(2, st);
             launch_shade(c, S, cur, hcur, nxt, hnxt, L.queue.p + 2 * (b - 1), L.queue.p + 2 * b, L.trav_queue.p, tqc + b, count,
-                         target, b, seed);
+                         target, b, seed, map.view_recip);
             s->span_end(st);
             s->launches += 2;
             PathSoA tmp = cur; cur = nxt; nxt = tmp;
@@ -669,6 +678,76 @@ int render_paths(rtc_scene* s, const DevScene& S, uint32_t seed, const PathMap& 
         }
         launch_tally(c, L.queue.p, tqc, depth, s->stats.p);
         s->launches++;
+    }
+    return RTC_OK;
+}
+
+// ---- cameras (rtc_scene_set_camera, rtc_render_views_*): 13 floats, position3 right3 up3 forward3 fov_x
+int check_camera(const float* c) {
+    if (!c) return fail(RTC_ERR_ARG, "null camera");
+    for (int i = 0; i < RTC_CAMERA_FLOATS; ++i)
+        if (!std::isfinite(c[i])) return fail(RTC_ERR_ARG, "camera value " + std::to_string(i) + " is not finite");
+    if (!(c[12] > 0.f && (double)c[12] < M_PI)) return fail(RTC_ERR_ARG, "camera fov_x must lie in (0, pi)");
+    return RTC_OK;
+}
+// `c` (checked) with the scene's frame size
+Camera camera_of(const HostScene& h, const float* c) {
+    Camera cam = h.cam;
+    cam.pos = mk3(c[0], c[1], c[2]);
+    cam.right = mk3(c[3], c[4], c[5]);
+    cam.up = mk3(c[6], c[7], c[8]);
+    cam.forward = mk3(c[9], c[10], c[11]);
+    cam.fov_x = c[12];
+    return cam;
+}
+double camera_extent(const float* c) { return std::max({std::fabs((double)c[0]), std::fabs((double)c[1]), std::fabs((double)c[2])}); }
+// A new layout of the arena of `s` on its device, uploaded synchronously: after the host scene's index BVH was rebuilt.
+// Everything that may still read the pinned mirror or the arenas -- asynchronous uploads, frames in flight, renders on
+// any stream -- is waited for first.
+int rebuild_arena(rtc_scene* s) {
+    CU(cudaSetDevice(s->device));
+    CU(cudaDeviceSynchronize());
+    { PinnedBuf<unsigned char> gone(std::move(s->arena_host)); }   // prepare_arena lays the arena out again
+    { DevBuf<unsigned char> gone(std::move(s->arena_dev[1])); }    // made again, at the new size, by the next asynchronous upload
+    s->arena_cur = 0;
+    return upload_scene(s, nullptr);
+}
+// The index BVH serves cameras out to flat.index_extent (its box slack is 2^-20 of it).  A camera farther out rebuilds
+// the index BVH for its extent -- primitive order, reference tree, LCA table and lights stay -- and uploads the new
+// arena to the scene's device and to every replica.  The extent only grows.
+int ensure_index_extent(rtc_scene* s, double extent) {
+    if (!(extent > s->host.flat.index_extent)) return RTC_OK;
+    Lap lap;
+    if (s->device >= 0) {   // no render may read the arenas or the pinned mirrors while they are rewritten
+        for (const auto& r : s->replicas) { CU(cudaSetDevice(r->device)); CU(cudaDeviceSynchronize()); }
+        CU(cudaSetDevice(s->device));
+        CU(cudaDeviceSynchronize());
+    }
+    try {
+        s->host.build_index(extent);
+    } catch (const std::exception& e) {
+        return fail(RTC_ERR_UNSUPPORTED, e.what());
+    }
+    lap("index BVH rebuild (host)");
+    if (s->device < 0) return RTC_OK;
+    int rc;
+    for (const auto& r : s->replicas)
+        if ((rc = rebuild_arena(r.get()))) return rc;
+    if ((rc = rebuild_arena(s))) return rc;
+    lap("arena rebuild + upload");
+    return RTC_OK;
+}
+// rtc_render_views_*: limits (RTC_ERR_UNSUPPORTED), then the cameras (RTC_ERR_ARG), before any device call
+constexpr int kMaxViews = 4096;
+int check_views(const rtc_scene* s, const float* cams, int nviews) {
+    if (!s) return fail(RTC_ERR_ARG, "null scene");
+    const uint64_t npix = (uint64_t)s->host.cam.width * s->host.cam.height;
+    if (nviews < 1 || nviews > kMaxViews) return fail(RTC_ERR_UNSUPPORTED, "nviews must be 1..4096");
+    if ((uint64_t)nviews * npix > (1ull << 28)) return fail(RTC_ERR_UNSUPPORTED, "nviews * width * height above 2^28 is not supported");
+    if (!cams) return fail(RTC_ERR_ARG, "null camera list");
+    for (int v = 0; v < nviews; ++v) {
+        int rc = check_camera(cams + (size_t)RTC_CAMERA_FLOATS * v);
+        if (rc) return fail(rc, "view " + std::to_string(v) + ": " + g_error);
     }
     return RTC_OK;
 }
@@ -750,6 +829,21 @@ int rtc_scene_override(rtc_scene* s, int width, int height, int samples, int ray
     if (samples >= 0) s->host.samples = (unsigned)samples;
     if (ray_depth >= 0) s->host.ray_depth = (unsigned)ray_depth;
     return RTC_OK;
+}
+int rtc_scene_camera(const rtc_scene* s, float out[RTC_CAMERA_FLOATS]) {
+    if (!s || !out) return fail(RTC_ERR_ARG, "null argument");
+    const Camera& c = s->host.cam;
+    const float v[RTC_CAMERA_FLOATS] = {c.pos.x, c.pos.y, c.pos.z, c.right.x, c.right.y, c.right.z, c.up.x, c.up.y, c.up.z,
+                                        c.forward.x, c.forward.y, c.forward.z, c.fov_x};
+    std::memcpy(out, v, sizeof v);
+    return RTC_OK;
+}
+int rtc_scene_set_camera(rtc_scene* s, const float cam[RTC_CAMERA_FLOATS]) {
+    if (!s) return fail(RTC_ERR_ARG, "null scene");
+    int rc = check_camera(cam);
+    if (rc) return rc;
+    s->host.cam = camera_of(s->host, cam);
+    return ensure_index_extent(s, camera_extent(cam));
 }
 int rtc_scene_prim_order(const rtc_scene* s, int32_t* out) {
     if (!s || !out) return fail(RTC_ERR_ARG, "null argument");
@@ -1061,6 +1155,90 @@ int rtc_render_ppm(rtc_scene* s, uint32_t seed, const char* out_path) {
     std::vector<uint8_t> img(3 * (size_t)s->host.cam.width * s->host.cam.height);
     int rc = rtc_render_u8(s, seed, img.data());
     return rc ? rc : write_ppm(out_path, s->host.cam.width, s->host.cam.height, img);
+}
+
+// ------------------------------------------------------------------ batched views
+// The views share the wavefront batches: path p is pixel p % npix of view (p / npix) % V, sample sample_begin +
+// p / (npix V), with view v's camera record in a small device array (k_generate) and its sums at view v's slice of one
+// float4 buffer of V npix pixels (k_shade deposits by the frame-wide pixel word, k_fold folds it).  The Philox streams
+// are those of a render of view v alone: k_shade keys them by the pixel within the view.
+int rtc_render_views_accumulate(rtc_scene* s, const float* cams_host, int nviews, uint32_t seed, uint32_t sample_begin,
+                                uint32_t sample_count, float* accum_dev, void* stream) {
+    int rc = check_views(s, cams_host, nviews);
+    if (rc) return rc;
+    if ((rc = need_device(s))) return rc;
+    const uint32_t V = (uint32_t)nviews;
+    const uint64_t npix = (uint64_t)s->host.cam.width * s->host.cam.height;
+    const uint64_t total = (uint64_t)V * npix * sample_count;
+    if (total == 0) return RTC_OK;
+    if (!accum_dev) return fail(RTC_ERR_ARG, "null accumulation buffer");
+    double extent = 0;
+    for (uint32_t v = 0; v < V; ++v) extent = std::max(extent, camera_extent(cams_host + (size_t)RTC_CAMERA_FLOATS * v));
+    if ((rc = ensure_index_extent(s, extent))) return rc;
+    std::vector<DevCamera> cams(V);
+    for (uint32_t v = 0; v < V; ++v) cams[v] = dev_camera(camera_of(s->host, cams_host + (size_t)RTC_CAMERA_FLOATS * v));
+    cudaStream_t user = (cudaStream_t)stream;
+    DevScene S;
+    if (s->host.dialect <= DIALECT_HW2) {
+        // one deterministic frame per view (sample 0, as rtc_render_accumulate): the frame kernel once per view, with that
+        // view's camera, into that view's slice
+        if (sample_begin > 0) return RTC_OK;
+        if ((rc = arena_begin(s, user, &S))) return rc;
+        LaunchCtx c{user, s->sms};
+        for (uint32_t v = 0; v < V; ++v) {
+            S.cam = cams[v];
+            float* slice = accum_dev + 3 * (size_t)v * npix;
+            if (s->host.dialect == DIALECT_HW1) launch_raycast_hw1(c, S, slice);
+            else launch_whitted_hw2(c, S, slice);
+            s->launches++;
+        }
+        if ((rc = arena_end(s, user))) return rc;
+        CU(cudaGetLastError());
+        return RTC_OK;
+    }
+    const uint64_t nsum = V * npix;
+    const int a4 = s->accum4_next;
+    s->accum4_next ^= 1;
+    DevBuf<float4>& accum4 = s->accum4[a4];
+    CU(accum4.ensure(nsum));
+    CU(s->views[a4].ensure(V));
+    CU(cudaStreamWaitEvent(user, s->accum4_idle[a4], 0));
+    CU(cudaMemcpyAsync(s->views[a4].p, cams.data(), V * sizeof(DevCamera), cudaMemcpyHostToDevice, user));
+    CU(cudaMemsetAsync(accum4.p, 0, nsum * sizeof(float4), user));
+    if ((rc = arena_begin(s, user, &S))) return rc;
+    if ((rc = fork_lanes(s, user))) return rc;
+    unsigned used = 0;
+    PathMap map{nullptr, (uint32_t)npix, sample_begin, s->views[a4].p, V, V > 1 ? UINT64_MAX / npix : 0};
+    if ((rc = render_paths(s, S, seed, map, total, accum4.p, &used))) return rc;
+    if ((rc = join_lanes(s, used, user))) return rc;
+    launch_fold(LaunchCtx{user, s->sms}, accum4.p, accum_dev, (uint32_t)nsum);
+    s->launches++;
+    CU(cudaEventRecord(s->accum4_idle[a4], user));
+    if ((rc = arena_end(s, user))) return rc;
+    CU(cudaGetLastError());
+    return RTC_OK;
+}
+int rtc_render_views_u8(rtc_scene* s, const float* cams_host, int nviews, uint32_t seed, uint8_t* rgb_host, float* sum_host) {
+    int rc = check_views(s, cams_host, nviews);
+    if (rc) return rc;
+    if (!rgb_host) return fail(RTC_ERR_ARG, "null argument");
+    if ((rc = need_device(s))) return rc;
+    uint32_t samples;
+    if ((rc = frame_samples(s, &samples))) return rc;
+    const size_t nvalues = 3 * (size_t)nviews * s->host.cam.width * s->host.cam.height;
+    if (nvalues == 0) return RTC_OK;
+    CU(s->accum.ensure(nvalues));
+    CU(s->rgb.ensure(nvalues));
+    CU(cudaMemsetAsync(s->accum.p, 0, nvalues * sizeof(float), nullptr));
+    if ((rc = rtc_render_views_accumulate(s, cams_host, nviews, seed, 0, samples, s->accum.p, nullptr))) return rc;
+    LaunchCtx c{nullptr, s->sms};
+    if (s->host.dialect == DIALECT_HW1) launch_resolve_flat(c, s->accum.p, 1.f / (float)samples, (uint32_t)nvalues, s->rgb.p);
+    else launch_resolve(c, s->accum.p, 1.f / (float)samples, (uint32_t)nvalues, s->rgb.p);
+    s->launches++;
+    CU(cudaGetLastError());
+    CU(cudaMemcpy(rgb_host, s->rgb.p, nvalues, cudaMemcpyDeviceToHost));
+    if (sum_host) CU(cudaMemcpy(sum_host, s->accum.p, nvalues * sizeof(float), cudaMemcpyDeviceToHost));
+    return RTC_OK;
 }
 
 // ------------------------------------------------------------------ adaptive sampling

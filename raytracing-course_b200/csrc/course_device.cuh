@@ -15,12 +15,12 @@ RT_D SceneHit closest_hit(const DevScene& S, vec3 o, vec3 d) { return scene_inte
 // `2 * (x + 0.5) / width - 1` and its product with the tangent are evaluated in double and rounded once.
 RT_D void centre_ray(const DevScene& S, uint32_t pixel, vec3& o, vec3& d) {
     uint32_t x = pixel % S.width, y = pixel / S.width;
-    float nx = (float)((2 * (x + 0.5) / (int)S.width - 1) * (double)S.tan_fov_x);
-    float ny = (float)(-1.f * (2 * (y + 0.5) / (int)S.height - 1) * (double)S.tan_fov_y);
-    o = mk3(S.cam_pos.x, S.cam_pos.y, S.cam_pos.z);
-    d.x = __fadd_rn(__fadd_rn(__fmul_rn(nx, S.cam_right.x), __fmul_rn(ny, S.cam_up.x)), __fmul_rn(1.f, S.cam_forward.x));
-    d.y = __fadd_rn(__fadd_rn(__fmul_rn(nx, S.cam_right.y), __fmul_rn(ny, S.cam_up.y)), __fmul_rn(1.f, S.cam_forward.y));
-    d.z = __fadd_rn(__fadd_rn(__fmul_rn(nx, S.cam_right.z), __fmul_rn(ny, S.cam_up.z)), __fmul_rn(1.f, S.cam_forward.z));
+    float nx = (float)((2 * (x + 0.5) / (int)S.width - 1) * (double)S.cam.tan_fov_x);
+    float ny = (float)(-1.f * (2 * (y + 0.5) / (int)S.height - 1) * (double)S.cam.tan_fov_y);
+    o = mk3(S.cam.pos.x, S.cam.pos.y, S.cam.pos.z);
+    d.x = __fadd_rn(__fadd_rn(__fmul_rn(nx, S.cam.right.x), __fmul_rn(ny, S.cam.up.x)), __fmul_rn(1.f, S.cam.forward.x));
+    d.y = __fadd_rn(__fadd_rn(__fmul_rn(nx, S.cam.right.y), __fmul_rn(ny, S.cam.up.y)), __fmul_rn(1.f, S.cam.forward.y));
+    d.z = __fadd_rn(__fadd_rn(__fmul_rn(nx, S.cam.right.z), __fmul_rn(ny, S.cam.up.z)), __fmul_rn(1.f, S.cam.forward.z));
 }
 
 // hw1 Scene::RayTrace: the colour of the closest primitive, the background otherwise (hw1 src/scene.cpp:167-179)

@@ -10,6 +10,27 @@
 
 namespace rtc {
 
+// Camera::GetToRay's inputs as the kernels read them (src/scene.cpp:180-187): position, axes, tan(fov_x / 2) and the
+// tangent of the vertical half-angle, tan(fov_x / 2) * height / width
+struct DevCamera {
+    float3 pos, right, up, forward;
+    float tan_fov_x, tan_fov_y;
+};
+// the one place a host camera becomes a DevCamera: the scene's own (fill_dev_scalars) and every view of a batched render
+inline DevCamera dev_camera(const Camera& cam) {
+    DevCamera C;
+    C.pos = make_float3(cam.pos.x, cam.pos.y, cam.pos.z);
+    C.right = make_float3(cam.right.x, cam.right.y, cam.right.z);
+    C.up = make_float3(cam.up.x, cam.up.y, cam.up.z);
+    C.forward = make_float3(cam.forward.x, cam.forward.y, cam.forward.z);
+    // Camera::GetToRay, src/scene.cpp:181-182 (tan evaluated in double, as the reference's
+    // unqualified tan() does; checked bit-exact against it in tests/)
+    float tx = (float)tan((double)(cam.fov_x / 2));
+    C.tan_fov_x = tx;
+    C.tan_fov_y = tx * (float)cam.height / (float)cam.width;
+    return C;
+}
+
 struct DevScene {
     // per primitive (final order), 16-byte aligned float4 arrays
     const float4* geo0;    // triangle (a, n.x) | other (d0, 0)
@@ -33,8 +54,7 @@ struct DevScene {
     uint32_t nprims, nbvh, nnodes, root, iroot, lca_levels, nlights, ref_depth;
     uint32_t iroot_ref[4];  // child references of the index root (k_traverse starts from the children pre_step entered)
     uint32_t width, height, ray_depth, nplanes;
-    float3 cam_pos, cam_right, cam_up, cam_forward;
-    float tan_fov_x, tan_fov_y;
+    DevCamera cam;
     float3 bg;
     // homework dialect (scene_host.h Dialect) and the constants that differ between the snapshots
     uint32_t dialect, nplights;
@@ -57,15 +77,7 @@ inline void fill_dev_scalars(const HostScene& host, DevScene& S) {
     }
     S.nlights = (uint32_t)host.lights.size(); S.ref_depth = host.flat.ref_depth;
     S.width = host.cam.width; S.height = host.cam.height; S.ray_depth = host.ray_depth;
-    S.cam_pos = make_float3(host.cam.pos.x, host.cam.pos.y, host.cam.pos.z);
-    S.cam_right = make_float3(host.cam.right.x, host.cam.right.y, host.cam.right.z);
-    S.cam_up = make_float3(host.cam.up.x, host.cam.up.y, host.cam.up.z);
-    S.cam_forward = make_float3(host.cam.forward.x, host.cam.forward.y, host.cam.forward.z);
-    // Camera::GetToRay, src/scene.cpp:181-182 (tan evaluated in double, as the reference's
-    // unqualified tan() does; checked bit-exact against it in tests/)
-    float tx = (float)tan((double)(host.cam.fov_x / 2));
-    S.tan_fov_x = tx;
-    S.tan_fov_y = tx * (float)host.cam.height / (float)host.cam.width;
+    S.cam = dev_camera(host.cam);
     S.bg = make_float3(host.background.x, host.background.y, host.background.z);
     S.nplights = (uint32_t)host.point_lights.size();
     S.dialect = (uint32_t)host.dialect;

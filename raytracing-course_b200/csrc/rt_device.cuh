@@ -935,14 +935,16 @@ RT_D float mix_pdf(const DevScene& S, vec3 x, vec3 n, vec3 d) {
 }
 
 // Camera::GetToRay, src/scene.cpp:180-187, without FMA contraction (bit-exact with the reference)
-RT_D void camera_ray(const DevScene& S, float x, float y, vec3& o, vec3& d) {
-    float nx = __fmul_rn(__fadd_rn(__fdiv_rn(__fmul_rn(2.f, x), (float)S.width), -1.f), S.tan_fov_x);
-    float ny = __fmul_rn(__fmul_rn(-1.f, __fadd_rn(__fdiv_rn(__fmul_rn(2.f, y), (float)S.height), -1.f)), S.tan_fov_y);
-    o = mk3(S.cam_pos.x, S.cam_pos.y, S.cam_pos.z);
-    d.x = __fadd_rn(__fadd_rn(__fmul_rn(nx, S.cam_right.x), __fmul_rn(ny, S.cam_up.x)), __fmul_rn(1.f, S.cam_forward.x));
-    d.y = __fadd_rn(__fadd_rn(__fmul_rn(nx, S.cam_right.y), __fmul_rn(ny, S.cam_up.y)), __fmul_rn(1.f, S.cam_forward.y));
-    d.z = __fadd_rn(__fadd_rn(__fmul_rn(nx, S.cam_right.z), __fmul_rn(ny, S.cam_up.z)), __fmul_rn(1.f, S.cam_forward.z));
+RT_D void camera_ray(const DevCamera& C, uint32_t width, uint32_t height, float x, float y, vec3& o, vec3& d) {
+    float nx = __fmul_rn(__fadd_rn(__fdiv_rn(__fmul_rn(2.f, x), (float)width), -1.f), C.tan_fov_x);
+    float ny = __fmul_rn(__fmul_rn(-1.f, __fadd_rn(__fdiv_rn(__fmul_rn(2.f, y), (float)height), -1.f)), C.tan_fov_y);
+    o = mk3(C.pos.x, C.pos.y, C.pos.z);
+    d.x = __fadd_rn(__fadd_rn(__fmul_rn(nx, C.right.x), __fmul_rn(ny, C.up.x)), __fmul_rn(1.f, C.forward.x));
+    d.y = __fadd_rn(__fadd_rn(__fmul_rn(nx, C.right.y), __fmul_rn(ny, C.up.y)), __fmul_rn(1.f, C.forward.y));
+    d.z = __fadd_rn(__fadd_rn(__fmul_rn(nx, C.right.z), __fmul_rn(ny, C.up.z)), __fmul_rn(1.f, C.forward.z));
 }
+// through the scene's own camera
+RT_D void camera_ray(const DevScene& S, float x, float y, vec3& o, vec3& d) { camera_ray(S.cam, S.width, S.height, x, y, o, d); }
 
 // GetReflection, src/scene.cpp:79-81
 RT_D vec3 reflect_dir(vec3 n, vec3 dir) { return dir - (2.0f * n) * dot(n, dir); }

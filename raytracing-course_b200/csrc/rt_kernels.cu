@@ -111,10 +111,11 @@ RT_D bool queue_slot(const QueueView& v, uint32_t at, uint32_t cap, uint32_t& sl
 }
 
 // ------------------------------------------------------------------------------- generate
-// Scene::Sample's jitter + Camera::GetToRay (src/scene.cpp:189-200) for the camera path of (pixel, sample), stored
-// in slot i, and its pre_step; returns the root children the ray enters (o, d, cd: what the traverse queue takes).
-RT_D uint32_t camera_path(const DevScene& S, PathSoA P, HitSoA H, uint32_t i, uint32_t pixel, uint32_t sample, uint32_t seed,
-                          vec3& o, vec3& d, float& cd) {
+// Scene::Sample's jitter + Camera::GetToRay (src/scene.cpp:189-200) through camera C for the camera path of (pixel,
+// sample), stored in slot i with `word` as its pixel word, and its pre_step; returns the root children the ray enters
+// (o, d, cd: what the traverse queue takes).
+RT_D uint32_t camera_path(const DevScene& S, const DevCamera& C, PathSoA P, HitSoA H, uint32_t i, uint32_t pixel, uint32_t word,
+                          uint32_t sample, uint32_t seed, vec3& o, vec3& d, float& cd) {
     uint32_t x = pixel % S.width, y = pixel / S.width;
     Rng g{seed, pixel, sample, 0};
     uint4 b = g.block(0);
@@ -122,18 +123,23 @@ RT_D uint32_t camera_path(const DevScene& S, PathSoA P, HitSoA H, uint32_t i, ui
     // hw3's Camera::GetToRay(float, float) still adds the half pixel of its integer ancestor
     // (hw3 src/scene.cpp:186-187): its jittered samples cover [x + 0.5, x + 1.5)
     if (S.dialect == DIALECT_HW3) { fx = __fadd_rn(fx, 0.5f); fy = __fadd_rn(fy, 0.5f); }
-    camera_ray(S, fx, fy, o, d);
+    camera_ray(C, S.width, S.height, fx, fy, o, d);
     uint32_t id;
     const uint32_t enters = pre_step(S, o, d, cd, id);
     WF_ST(P.o + i, make_float4(o.x, o.y, o.z, __uint_as_float(sample)));
     WF_ST(P.d + i, make_float4(d.x, d.y, d.z, cd));
-    WF_ST(P.beta + i, make_float4(1.f, 1.f, 1.f, __uint_as_float(pixel)));
+    WF_ST(P.beta + i, make_float4(1.f, 1.f, 1.f, __uint_as_float(word)));
     WF_ST(H.id + i, id);
     return enters;
 }
 // One thread per path.  Path ids run sample-major over the image: consecutive threads = consecutive pixels of a row.
+// With `views` (nviews cameras) path p is pixel p % npix of view (p / npix) % nviews and sample sample_begin +
+// p / (npix nviews); its pixel word is the frame-wide index view npix + pixel.  Without (VIEWS = false), the scene's own
+// camera, in a kernel of its own: a one-frame render runs the code it ran before views existed.
+template <bool VIEWS>
 __global__ void __launch_bounds__(256) k_generate(DevScene S, PathSoA P, HitSoA H, uint32_t* q, uint32_t* tq, uint32_t* tq_count,
-                                                   uint64_t first_path, uint32_t count, uint32_t seed, uint32_t sample_begin) {
+                                                   uint64_t first_path, uint32_t count, uint32_t seed, uint32_t sample_begin,
+                                                   const DevCamera* views, uint32_t nviews) {
     const uint32_t npix = S.width * S.height;
     const uint32_t lane = threadIdx.x & 31;
     const uint32_t rounded = (count + 31u) & ~31u;
@@ -143,9 +149,11 @@ __global__ void __launch_bounds__(256) k_generate(DevScene S, PathSoA P, HitSoA 
         float cd = 0.f;
         if (i < count) {
             uint64_t pid = first_path + i;
-            uint32_t sample = sample_begin + (uint32_t)(pid / npix);
+            const uint64_t frame = pid / npix;   // view-major: the frames of all views for one sample, then the next sample
             uint32_t pixel = (uint32_t)(pid % npix);
-            enters = camera_path(S, P, H, i, pixel, sample, seed, o, d, cd);
+            const uint32_t view = VIEWS ? (uint32_t)(frame % nviews) : 0u;
+            const uint32_t sample = sample_begin + (uint32_t)(VIEWS ? frame / nviews : frame);
+            enters = camera_path(S, VIEWS ? views[view] : S.cam, P, H, i, pixel, view * npix + pixel, sample, seed, o, d, cd);
         }
         enqueue(enters, i, o, d, cd, tq, tq_count, lane);
     }
@@ -166,7 +174,7 @@ __global__ void __launch_bounds__(256) k_generate_list(DevScene S, PathSoA P, Hi
             uint64_t pid = first_path + i;
             uint32_t sample = sample_first + 2u * (uint32_t)(pid / npix);
             uint32_t pixel = plist[pid % npix];
-            enters = camera_path(S, P, H, i, pixel, sample, seed, o, d, cd);
+            enters = camera_path(S, S.cam, P, H, i, pixel, pixel, sample, seed, o, d, cd);
         }
         enqueue(enters, i, o, d, cd, tq, tq_count, lane);
     }
@@ -428,6 +436,14 @@ RT_D void deposit(float4* accum4, uint32_t pixel, vec3 L) {
 #endif
 }
 
+// The pixel within its view of a frame-wide pixel word g = view npix + pixel (k_generate): g - npix floor(g / npix), the
+// quotient from recip = floor((2^64 - 1) / npix) -- exact or one short for every 32-bit g, so one correction -- or 0
+// for a single view (quotient 0: the word is the pixel).
+RT_D uint32_t view_pixel(uint32_t g, uint32_t npix, uint64_t recip) {
+    const uint32_t r = g - npix * (uint32_t)__umul64hi((uint64_t)g, recip);
+    return r >= npix ? r - npix : r;
+}
+
 // Scene::RayTrace's material switch (src/scene.cpp:96-177) for one bounce, recursion unrolled:
 // L = sum_k beta_k * E_k.  Surviving paths are written compacted (warp ballot + one atomic per
 // warp) into the next queue; every hit adds its beta * emission to the pixel sum at once (deposit).
@@ -447,11 +463,15 @@ RT_D void deposit(float4* accum4, uint32_t pixel, vec3 L) {
 // around the normal, weight 2 C cos; every other line of the switch is common to hw3, hw4 and hw5.
 // FEAT = the scene features this instantiation supports (rt_device.cuh prim_flags_for): the kernel is bound by
 // instruction fetch, and the course's dragon scenes use a third of its code (no rotation, no ellipsoid, diffuse).
-template <bool HW3, uint32_t FEAT>
+// VIEWS = the pixel words index the frames of several views (rtc_render_views_accumulate): the in-view pixel of the RNG
+// streams is then view_pixel(word), which costs the lean instantiations their spill-free 56 registers at 9 blocks; a
+// one-frame render keeps the kernel without it.
+template <bool HW3, uint32_t FEAT, bool VIEWS>
 __global__ void __launch_bounds__(RTC_SHADE_THREADS, (FEAT & (FE_ROTATION | FE_ELLIPSOID)) ? RTC_SHADE_MIN_BLOCKS_FULL : RTC_SHADE_MIN_BLOCKS_LEAN) k_shade(DevScene S, PathSoA P, HitSoA H, PathSoA N, HitSoA HN, const uint32_t* qin,
                                                 uint32_t* qout, uint32_t* tq, uint32_t* tq_count, float4* accum4, uint32_t bounce,
-                                                uint32_t seed, uint32_t cap) {
+                                                uint32_t seed, uint32_t cap, uint64_t view_recip) {
     const QueueView view = queue_view(qin);
+    const uint32_t npix = S.width * S.height;
     const uint32_t lane = threadIdx.x & 31;
     const float eps = S.eps;
     // camera paths (bounce 1) arrive unsorted; from then on the end of the queue a path sits at tells its coin
@@ -461,12 +481,13 @@ __global__ void __launch_bounds__(RTC_SHADE_THREADS, (FEAT & (FE_ROTATION | FE_E
     for (uint32_t at = blockIdx.x * blockDim.x + threadIdx.x; at < view.total; at += gridDim.x * blockDim.x) {
         bool alive = false;
         vec3 no = mk3(0, 0, 0), nd = mk3(0, 0, 0), beta = mk3(0, 0, 0);
-        uint32_t pixel = 0, sample = 0;
+        uint32_t word = 0, pixel = 0, sample = 0;   // the path's pixel word (frame-wide) and its pixel within its view
         uint32_t i; bool back;
         if (queue_slot(view, at, cap, i, back)) {
             const float4 b4 = WF_LD(P.beta + i), o4 = WF_LD(P.o + i);
             beta = ld3(b4);
-            pixel = __float_as_uint(b4.w); sample = __float_as_uint(o4.w);
+            word = __float_as_uint(b4.w); sample = __float_as_uint(o4.w);
+            pixel = VIEWS ? view_pixel(word, npix, view_recip) : word;
             uint32_t prim = WF_LD(H.id + i);
             Isect is;
             vec3 o = ld3(o4), d = ld3(WF_LD(P.d + i));
@@ -545,7 +566,7 @@ __global__ void __launch_bounds__(RTC_SHADE_THREADS, (FEAT & (FE_ROTATION | FE_E
                     }
                 }
             }
-            if (L.x != 0.f || L.y != 0.f || L.z != 0.f) deposit(accum4, pixel, L);
+            if (L.x != 0.f || L.y != 0.f || L.z != 0.f) deposit(accum4, word, L);
         }
         unsigned mask = __ballot_sync(kFullMask, alive);
         if (mask) {
@@ -573,7 +594,7 @@ __global__ void __launch_bounds__(RTC_SHADE_THREADS, (FEAT & (FE_ROTATION | FE_E
             if (alive) {
                 WF_ST(N.o + dst, make_float4(no.x, no.y, no.z, __uint_as_float(sample)));
                 WF_ST(N.d + dst, make_float4(nd.x, nd.y, nd.z, cd));
-                WF_ST(N.beta + dst, make_float4(beta.x, beta.y, beta.z, __uint_as_float(pixel)));
+                WF_ST(N.beta + dst, make_float4(beta.x, beta.y, beta.z, __uint_as_float(word)));
                 WF_ST(HN.id + dst, id);
             }
             if (emask) {
@@ -983,8 +1004,13 @@ static int grid_for(uint64_t n, int block, int sms, int per_sm) {
 }
 
 void launch_generate(const LaunchCtx& c, const DevScene& S, PathSoA P, HitSoA H, uint32_t* q, uint32_t* tq, uint32_t* tq_count,
-                     uint64_t first_path, uint32_t count, uint32_t seed, uint32_t sample_begin) {
-    k_generate<<<grid_for(count, 256, c.sms, 8), 256, 0, c.stream>>>(S, P, H, q, tq, tq_count, first_path, count, seed, sample_begin);
+                     uint64_t first_path, uint32_t count, uint32_t seed, uint32_t sample_begin, const DevCamera* views, uint32_t nviews) {
+    if (views)
+        k_generate<true><<<grid_for(count, 256, c.sms, 8), 256, 0, c.stream>>>(S, P, H, q, tq, tq_count, first_path, count, seed,
+                                                                               sample_begin, views, nviews);
+    else
+        k_generate<false><<<grid_for(count, 256, c.sms, 8), 256, 0, c.stream>>>(S, P, H, q, tq, tq_count, first_path, count, seed,
+                                                                                sample_begin, nullptr, 1);
 }
 void launch_generate_list(const LaunchCtx& c, const DevScene& S, PathSoA P, HitSoA H, uint32_t* q, uint32_t* tq, uint32_t* tq_count,
                           uint64_t first_path, uint32_t count, uint32_t seed, const uint32_t* plist, uint32_t npix, uint32_t sample_first) {
@@ -1057,9 +1083,13 @@ void launch_extend_reftree(const LaunchCtx& c, const DevScene& S, PathSoA P, Hit
 }
 void launch_shade(const LaunchCtx& c, const DevScene& S, PathSoA P, HitSoA H, PathSoA N, HitSoA HN, const uint32_t* qin,
                   uint32_t* qout, uint32_t* tq, uint32_t* tq_count, uint32_t max_count, float4* accum4, uint32_t bounce,
-                  uint32_t seed) {
+                  uint32_t seed, uint64_t view_recip) {
     const int grid = grid_for(max_count, RTC_SHADE_THREADS, c.sms, 2048 / RTC_SHADE_THREADS);
-#define RTC_SHADE(HW3, FEAT) k_shade<HW3, FEAT><<<grid, RTC_SHADE_THREADS, 0, c.stream>>>(S, P, H, N, HN, qin, qout, tq, tq_count, accum4, bounce, seed, max_count)
+#define RTC_SHADE(HW3, FEAT)                                                                                                  \
+    (view_recip ? k_shade<HW3, FEAT, true><<<grid, RTC_SHADE_THREADS, 0, c.stream>>>(S, P, H, N, HN, qin, qout, tq, tq_count, accum4, \
+                                                                                   bounce, seed, max_count, view_recip)            \
+                : k_shade<HW3, FEAT, false><<<grid, RTC_SHADE_THREADS, 0, c.stream>>>(S, P, H, N, HN, qin, qout, tq, tq_count, accum4, \
+                                                                                    bounce, seed, max_count, 0))
     // the smallest instantiation that covers the scene's features (DevScene::features)
 #ifdef RTC_SHADE_NO_SPECIALISATION
     const uint32_t feat = FE_ALL;

@@ -18,9 +18,11 @@ struct LaunchCtx {
     int sms;  // multiprocessor count of the device (grid sizing)
 };
 
-// camera rays of one wavefront batch + their pre_step (planes, index root, traverse queue)
+// camera rays of one wavefront batch + their pre_step (planes, index root, traverse queue): through the scene's camera
+// (views = null), or through nviews cameras, path p = pixel p % npix of view (p / npix) % nviews, sample sample_begin +
+// p / (npix nviews), pixel word view npix + pixel
 void launch_generate(const LaunchCtx& c, const DevScene& S, PathSoA P, HitSoA H, uint32_t* q, uint32_t* tq, uint32_t* tq_count,
-                     uint64_t first_path, uint32_t count, uint32_t seed, uint32_t sample_begin);
+                     uint64_t first_path, uint32_t count, uint32_t seed, uint32_t sample_begin, const DevCamera* views, uint32_t nviews);
 // the same over a pixel list: path p = pixel plist[p % npix], sample sample_first + 2 (p / npix)
 void launch_generate_list(const LaunchCtx& c, const DevScene& S, PathSoA P, HitSoA H, uint32_t* q, uint32_t* tq, uint32_t* tq_count,
                           uint64_t first_path, uint32_t count, uint32_t seed, const uint32_t* plist, uint32_t npix, uint32_t sample_first);
@@ -61,10 +63,11 @@ void launch_pre(const LaunchCtx& c, const DevScene& S, PathSoA P, HitSoA H, cons
 void launch_traverse(const LaunchCtx& c, const DevScene& S, PathSoA P, HitSoA H, uint32_t max_count, const uint32_t* tq,
                      const uint32_t* tq_count, uint32_t* cursor, bool count_visits, unsigned long long* stats);
 void launch_extend_reftree(const LaunchCtx& c, const DevScene& S, PathSoA P, HitSoA H, const uint32_t* q, uint32_t cap);
-// shading of queue P with hits H; survivors go to queue N with their pre_step results in HN / tq
+// shading of queue P with hits H; survivors go to queue N with their pre_step results in HN / tq.  view_recip: 0 when
+// the pixel words are pixels of one frame, floor((2^64 - 1) / (width height)) when they index several views' frames
 void launch_shade(const LaunchCtx& c, const DevScene& S, PathSoA P, HitSoA H, PathSoA N, HitSoA HN, const uint32_t* qin,
                   uint32_t* qout, uint32_t* tq, uint32_t* tq_count, uint32_t max_count, float4* accum4, uint32_t bounce,
-                  uint32_t seed);
+                  uint32_t seed, uint64_t view_recip);
 // accum += accum4 (xyz): the library's float4 pixel sums into the caller's buffer at the end of a frame
 void launch_fold(const LaunchCtx& c, const float4* accum4, float* accum, uint32_t npix);
 // the tail of a scene arena, rebuilt on the device after every upload of its head (c_api.cu issue_upload)

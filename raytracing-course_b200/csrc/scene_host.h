@@ -113,6 +113,9 @@ struct FlatScene {
     std::vector<f4> plights;           // hw2: 4 x f4 per light: (intensity, bits(directed)) (pos,0) (attenuation,0) (normalised dir,0)
     uint32_t index_depth = 0, ref_depth = 0, units = 0;
     uint32_t features = 0;             // SceneFeature bits present in this scene
+    // the extent the index BVH was built for: max(|camera position|inf, |unit box coordinates|inf); its child boxes are
+    // widened by 2^-20 of it (bvh_build.cpp IndexBuilder::slack), so a camera farther out needs a rebuild
+    double index_extent = 0;
 };
 
 struct HostScene {
@@ -134,6 +137,11 @@ struct HostScene {
     void parse(const std::string& text);
     // Scene::InitScene (src/scene.cpp:7-40) + our index structures + flattening
     void init();
+    // the units (reference leaves), their exact boxes and the index BVH over them, for cameras up to `cam_extent` (the
+    // largest |position|inf): the stage of init() after the reference tree, and the whole rebuild when a camera is set
+    // beyond flat.index_extent.  Reads prims and nodes in their final order; changes only units, ubox, inodes, iroot,
+    // index_depth and index_extent.
+    void build_index(double cam_extent);
 };
 
 // child reference encoding of the index BVH
