@@ -136,6 +136,13 @@ int rtc_render_reset_counters(rtc_scene* s);
 /* Warp-execution efficiency of k_traverse's per-warp scheduler (only with count_visits): out[0..3] = warp
  * iterations of kind VISIT / LEAF / FINISH / REFILL, out[4..7] = lanes that took part in them (of 32 each). */
 int rtc_traverse_lanes(rtc_scene* s, void* stream, uint64_t out[8]);
+/* Camera rays of rtc_render_accumulate and the adaptive renders are resolved from per-pixel lists of candidate index
+ * leaves (one beam traversal per pixel per call) instead of the index traversal, except in pixels whose list would be
+ * too long.  out[0]: such camera rays since the scene was created or rtc_render_reset_counters. */
+int rtc_camera_list_rays(rtc_scene* s, void* stream, uint64_t* out);
+/* The list length of every pixel (width * height, row-major) for the scene's camera as it stands, 0xFFFFFFFF for a pixel
+ * whose rays take the index traversal; synchronous. */
+int rtc_camera_list_lengths(rtc_scene* s, uint32_t* lengths_host);
 /* mean = 1/total_samples * sum ; tonemap ; gamma ; u8 -> rgb_dev (3 bytes per pixel, device) */
 int rtc_render_resolve(rtc_scene* s, const float* accum_dev, uint32_t total_samples, uint8_t* rgb_dev, void* stream);
 /* whole Scene::Render with the scene's own SAMPLES: host u8 image (3*W*H bytes) */

@@ -62,6 +62,8 @@ _SIGNATURES = {
     "rtc_render_counters": (C.c_int, [C.c_void_p, C.c_void_p, _u64]),
     "rtc_render_reset_counters": (C.c_int, [C.c_void_p]),
     "rtc_traverse_lanes": (C.c_int, [C.c_void_p, C.c_void_p, _u64]),
+    "rtc_camera_list_rays": (C.c_int, [C.c_void_p, C.c_void_p, _u64]),
+    "rtc_camera_list_lengths": (C.c_int, [C.c_void_p, np.ctypeslib.ndpointer(np.uint32, flags="C_CONTIGUOUS")]),
     "rtc_scene_arena_check": (C.c_int, [C.c_void_p, _u64]),
     "rtc_intersect_dev": (C.c_int, [C.c_void_p, C.c_long, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                     C.c_void_p, C.c_int, C.c_void_p]),
@@ -509,6 +511,19 @@ class Scene:
         kinds = ["visit", "leaf", "finish", "refill"]
         return {k: {"iterations": int(out[i]), "lanes": (float(out[4 + i]) / float(out[i]) if out[i] else 0.0)}
                 for i, k in enumerate(kinds)}
+
+    def camera_list_rays(self, stream=None):
+        """Camera rays resolved from per-pixel candidate lists (no index traversal) since the counters were reset."""
+        out = np.zeros(1, np.uint64)
+        _check(self.lib, self.lib.rtc_camera_list_rays(self.h, C.c_void_p(stream or 0), out))
+        return int(out[0])
+
+    def camera_list_lengths(self):
+        """(H, W) uint32: the candidate-list length of every pixel for the scene's camera, 0xFFFFFFFF where the pixel's
+        camera rays take the index traversal."""
+        out = np.zeros((self.height, self.width), np.uint32)
+        _check(self.lib, self.lib.rtc_camera_list_lengths(self.h, out))
+        return out
 
     def set_profiling(self, kernel_events=False, count_visits=False):
         _check(self.lib, self.lib.rtc_set_profiling(self.h, int(kernel_events), int(count_visits)))

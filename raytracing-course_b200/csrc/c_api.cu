@@ -88,7 +88,7 @@ using TimedEvent = Handle<cudaEvent_t, new_timed_event, cudaEventDestroy>;   // 
 
 constexpr uint64_t kDefaultBatchPaths = 1ull << 24;
 constexpr int kMaxDepthSlots = 64;
-constexpr int kStatWords = 16;
+constexpr int kStatWords = 24;   // rtc_render_counters (8), rtc_traverse_lanes (8), kStatListRays
 constexpr int kMaxWhittedDepth = 32;   // course_device.cuh kWhittedStack = kMaxWhittedDepth + 2
 }  // namespace
 
@@ -140,6 +140,9 @@ struct rtc_scene {
     Event resolved;                       // rtc_resolve_to_host_async: the image may leave the device
     // float4 pixel sums of the renders in flight (k_shade deposits, k_fold reads): two, used alternately
     DevBuf<float4> accum4[2];
+    // the camera candidate lists of the render that uses accum4[i] (k_pixel_candidates, kCandWords words per pixel): built
+    // at the start of every rtc_render_accumulate and guarded by accum4_idle[i] like the sums
+    DevBuf<uint32_t> cand[2];
     Event accum4_idle[2];
     int accum4_next = 0;
     // the camera records of a batched render (rtc_render_views_accumulate), one set per float4 sum buffer, reused with it
@@ -183,6 +186,7 @@ struct rtc_scene {
         DevBuf<float4> half[2];
         DevBuf<uint32_t> tiles[2], pixels[2], tile_n, counts, spp;
         DevBuf<float> halves;
+        DevBuf<uint32_t> cand;   // camera candidate lists of the render's pixels, built before its first pass
         PinnedBuf<uint32_t> counts_host;
     } adaptive;
     // rtc_denoise / rtc_render_denoised: the linear mean u (3 floats per pixel), D and V (k_denoise_prep) and the filtered
@@ -604,6 +608,7 @@ struct PathMap {
     const DevCamera* views = nullptr;
     uint32_t nviews = 1;
     uint64_t view_recip = 0;
+    const uint32_t* cand = nullptr;   // camera candidate lists of the scene's camera (build_camera_lists), or null
 };
 // fork: the lane streams of the next render_paths calls start after everything already queued on the caller's stream
 int fork_lanes(rtc_scene* s, cudaStream_t user) {
@@ -618,6 +623,21 @@ int join_lanes(rtc_scene* s, unsigned used, cudaStream_t user) {
         CU(cudaEventRecord(s->lanes[i].done, s->lanes[i].stream));
         CU(cudaStreamWaitEvent(user, s->lanes[i].done, 0));
     }
+    return RTC_OK;
+}
+// The candidate leaves of the camera rays of every pixel of the scene's camera into `buf` (kCandWords words per pixel), on
+// `st` after arena_begin: returns the lists for PathMap::cand, or null when the render does not use them (the
+// reference-tree traversal).  Built on every render call: the arena, the camera or the frame size may have changed since.
+int build_camera_lists(rtc_scene* s, const DevScene& S, DevBuf<uint32_t>& buf, cudaStream_t st, const uint32_t** cand) {
+    *cand = nullptr;
+    if (s->traversal == RTC_TRAVERSAL_REFTREE) return RTC_OK;
+    const size_t npix = (size_t)S.width * S.height;
+    CU(buf.ensure(kCandWords * npix));
+    s->span_begin(3, st);
+    launch_pixel_candidates(LaunchCtx{st, s->sms}, S, buf.p, s->count_visits, s->stats.p);
+    s->span_end(st);
+    s->launches++;
+    *cand = buf.p;
     return RTC_OK;
 }
 // The wavefront batches of `total` paths laid out by `map`: every hit deposits into `target` (float4 per pixel of the
@@ -659,8 +679,10 @@ int render_paths(rtc_scene* s, const DevScene& S, uint32_t seed, const PathMap& 
         PathSoA nxt{L.path[1][0].p, L.path[1][1].p, L.path[1][2].p};
         HitSoA hcur{L.hit_id[0].p}, hnxt{L.hit_id[1].p};
         s->span_begin(0, st);
-        if (map.plist) launch_generate_list(c, S, cur, hcur, L.queue.p, L.trav_queue.p, tqc, first, count, seed, map.plist, map.npix, map.sample_first);
-        else launch_generate(c, S, cur, hcur, L.queue.p, L.trav_queue.p, tqc, first, count, seed, map.sample_first, map.views, map.nviews);
+        if (map.plist) launch_generate_list(c, S, cur, hcur, L.queue.p, L.trav_queue.p, tqc, first, count, seed, map.plist, map.npix, map.sample_first,
+                                            map.cand, s->stats.p);
+        else launch_generate(c, S, cur, hcur, L.queue.p, L.trav_queue.p, tqc, first, count, seed, map.sample_first, map.views, map.nviews,
+                             map.cand, s->stats.p);
         s->span_end(st);
         s->launches++;
         for (uint32_t b = 1; b <= depth; ++b) {
@@ -1071,9 +1093,11 @@ int rtc_render_accumulate(rtc_scene* s, uint32_t seed, uint32_t sample_begin, ui
     CU(cudaStreamWaitEvent(user, s->accum4_idle[a4], 0));
     CU(cudaMemsetAsync(accum4.p, 0, npix * sizeof(float4), user));
     if ((rc = arena_begin(s, user, &S))) return rc;
+    PathMap map{nullptr, (uint32_t)npix, sample_begin};
+    if ((rc = build_camera_lists(s, S, s->cand[a4], user, &map.cand))) return rc;
     if ((rc = fork_lanes(s, user))) return rc;
     unsigned used = 0;
-    if ((rc = render_paths(s, S, seed, PathMap{nullptr, (uint32_t)npix, sample_begin}, total, accum4.p, &used))) return rc;
+    if ((rc = render_paths(s, S, seed, map, total, accum4.p, &used))) return rc;
     if ((rc = join_lanes(s, used, user))) return rc;
     launch_fold(LaunchCtx{user, s->sms}, accum4.p, accum_dev, (uint32_t)npix);
     s->launches++;
@@ -1103,6 +1127,34 @@ int rtc_traverse_lanes(rtc_scene* s, void* stream, uint64_t out[8]) {
     unsigned long long h[8];
     CU(cudaMemcpy(h, s->stats.p + 8, sizeof h, cudaMemcpyDeviceToHost));
     for (int i = 0; i < 8; ++i) out[i] = h[i];
+    return RTC_OK;
+}
+int rtc_camera_list_rays(rtc_scene* s, void* stream, uint64_t* out) {
+    int rc = need_device(s);
+    if (rc) return rc;
+    if (!out) return fail(RTC_ERR_ARG, "null argument");
+    CU(cudaStreamSynchronize((cudaStream_t)stream));
+    CU(sync_lanes(s));
+    unsigned long long h;
+    CU(cudaMemcpy(&h, s->stats.p + kStatListRays, sizeof h, cudaMemcpyDeviceToHost));
+    *out = h;
+    return RTC_OK;
+}
+int rtc_camera_list_lengths(rtc_scene* s, uint32_t* lengths_host) {
+    int rc = need_device(s);
+    if (rc) return rc;
+    if (!lengths_host) return fail(RTC_ERR_ARG, "null argument");
+    const size_t npix = (size_t)s->host.cam.width * s->host.cam.height;
+    if (npix == 0) return RTC_OK;
+    DevScene S;
+    if ((rc = arena_begin(s, nullptr, &S))) return rc;
+    DevBuf<uint32_t> buf;
+    CU(buf.ensure(kCandWords * npix));
+    launch_pixel_candidates(LaunchCtx{nullptr, s->sms}, S, buf.p, false, s->stats.p);
+    s->launches++;
+    if ((rc = arena_end(s, nullptr))) return rc;
+    CU(cudaGetLastError());
+    CU(cudaMemcpy(lengths_host, buf.p, npix * sizeof(uint32_t), cudaMemcpyDeviceToHost));
     return RTC_OK;
 }
 int rtc_render_reset_counters(rtc_scene* s) {
@@ -1286,6 +1338,8 @@ int adaptive_passes(rtc_scene* c, cudaStream_t user, uint32_t shard, uint32_t ns
     CU(cudaMemsetAsync(ad.counts.p, 0, 4 * sizeof(uint32_t), user));
     DevScene S;
     if ((rc = arena_begin(c, user, &S))) return rc;
+    const uint32_t* cand;
+    if ((rc = build_camera_lists(c, S, ad.cand, user, &cand))) return rc;
     // every tile of the shard is active with n = 0; lists of pass 0 in set 0
     launch_adaptive_tiles(lc, nullptr, nullptr, width, height, nullptr, shard_tiles, 0, 0.f, 0.f, tolerance, ADAPTIVE_FIRST, ad.tile_n.p,
                           ad.tiles[0].p, ad.pixels[0].p, ad.counts.p, shard, nshards);
@@ -1300,7 +1354,9 @@ int adaptive_passes(rtc_scene* c, cudaStream_t user, uint32_t shard, uint32_t ns
             const uint32_t first = n + ((n ^ h) & 1u);
             if (first >= target) continue;
             const uint64_t total = (uint64_t)((target - first + 1) / 2) * active_pix;
-            if ((rc = render_paths(c, S, seed, PathMap{ad.pixels[cur].p, active_pix, first}, total, ad.half[h].p, &used))) return rc;
+            PathMap map{ad.pixels[cur].p, active_pix, first};
+            map.cand = cand;
+            if ((rc = render_paths(c, S, seed, map, total, ad.half[h].p, &used))) return rc;
             st[1] += total;
         }
         if ((rc = join_lanes(c, used, user))) return rc;

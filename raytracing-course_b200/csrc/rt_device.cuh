@@ -949,4 +949,156 @@ RT_D void camera_ray(const DevScene& S, float x, float y, vec3& o, vec3& d) { ca
 // GetReflection, src/scene.cpp:79-81
 RT_D vec3 reflect_dir(vec3 n, vec3 dir) { return dir - (2.0f * n) * dot(n, dir); }
 
+// ------------------------------------------------------------------------------- per-pixel candidate leaves
+// All camera rays of a pixel start at C.pos and differ only by their jitter, so one conservative traversal of the index
+// tree with the pixel's whole beam of directions (pixel_candidates) finds every leaf the index traversal of any of its
+// rays can reach.  A camera ray then tests those leaves exactly (leaf_test) and replays the reference over the ones with
+// a hit (camera_path in rt_kernels.cu), with no node visit and no traverse-queue record.  Since the list is a superset
+// of what the ray's own traversal reaches and the exact leaf_test decides, the set of hit leaves and so the id are the
+// same (DESIGN.md "Camera rays from per-pixel candidate lists").
+//
+// A pixel whose beam reaches more than kMaxRecords leaves, or at whose nodes k_traverse could run out of stack, is
+// marked kPixelTraverse: its rays take pre_step and k_traverse as every other ray does.
+constexpr uint32_t kPixelTraverse = 0xFFFFFFFFu;
+// k_traverse's per-lane stack (rt_kernels.cu): inner-node stack from the bottom, noted leaves from the top
+constexpr int kStackWords = 56;
+// Slack of the beam's cone test against cone_cull_pair's half arithmetic: the ray's direction rounded to half (2^-11
+// relative), one product and two fused sums each rounded to half (2^-11 of |ax dx| + |ay dy| + |az dz| <= |axis| <= 1.001
+// each) stay below 4 * 2^-11 * 1.001 = 1.96e-3 together; the float work of cone_dir adds ~1e-6.  Twice that is kept.
+constexpr float kBeamConeSlack = 1.f / 256.f;
+// Relative slack of the beam's slab test against the per-ray slab_ch (approximate reciprocal, 1-2 ulp; fma of the centre
+// and the half-extent, one ulp each): a few 2^-23 of (|centre| + |half| + |origin|) / |d|.  1e-5 is ~40 times that.
+constexpr float kBeamBoxSlack = 1e-5f;
+
+// The directions camera_ray makes for the jittered samples of pixel (x, y) through camera C.  Every step of camera_ray
+// (correctly rounded products, sums, one division) is monotone in its input, so each direction component is monotone in
+// fx and in fy separately, and its range over the pixel is spanned by the four corner samples: jitter u = 0 and
+// u = 1 - 2^-24, the largest u01 (plus hw3's half pixel).  The range is exact for float directions, no widening needed.
+struct Beam {
+    vec3 o;        // common origin
+    vec3 lo, hi;   // per axis: least and greatest direction component of any sample
+    vec3 c;        // unit direction the cone test measures from
+    float r;       // bound on |normalize(d) - c| over the pixel's samples
+};
+RT_D Beam pixel_beam(const DevCamera& C, uint32_t width, uint32_t height, uint32_t dialect, uint32_t x, uint32_t y) {
+    const float umax = (float)0xFFFFFFu * (1.0f / 16777216.0f);
+    float fx[2] = {__fadd_rn((float)x, 0.f), __fadd_rn((float)x, umax)}, fy[2] = {__fadd_rn((float)y, 0.f), __fadd_rn((float)y, umax)};
+    if (dialect == DIALECT_HW3)
+        for (int i = 0; i < 2; ++i) { fx[i] = __fadd_rn(fx[i], 0.5f); fy[i] = __fadd_rn(fy[i], 0.5f); }
+    Beam B;
+    vec3 dn[4], sum = mk3(0.f, 0.f, 0.f);
+    for (int i = 0; i < 4; ++i) {
+        vec3 d;
+        camera_ray(C, width, height, fx[i & 1], fy[i >> 1], B.o, d);
+        B.lo = i ? mk3(fminf(B.lo.x, d.x), fminf(B.lo.y, d.y), fminf(B.lo.z, d.z)) : d;
+        B.hi = i ? mk3(fmaxf(B.hi.x, d.x), fmaxf(B.hi.y, d.y), fmaxf(B.hi.z, d.z)) : d;
+        dn[i] = normalize(d);
+        sum = sum + dn[i];
+    }
+    // the directions lie on the plane camera_ray maps the pixel to; on that plane {p : angle(p, c) <= a} is convex for
+    // a < 90 degrees, so the angle to c, and with it |normalize(d) - c|, is greatest at a corner (1e-5: float rounding)
+    B.c = normalize(sum);
+    B.r = 0.f;
+    for (int i = 0; i < 4; ++i) B.r = fmaxf(B.r, length(dn[i] - B.c));
+    B.r += 1e-5f;
+    return B;
+}
+// Slab entry / exit distances of one axis over the beam, widened by the slack of the per-ray test: (-inf, inf) when the
+// beam's direction interval holds 0 or a component so small that ray_inv clamps it.
+RT_D void beam_axis(float mn, float mx, float o, float lo, float hi, float slack, float& t_in, float& t_out) {
+    if (!(fminf(fabsf(lo), fabsf(hi)) >= 1e-20f) || (lo < 0.f) != (hi < 0.f)) { t_in = -kInfF; t_out = kInfF; return; }
+    const float il = 1.f / lo, ih = 1.f / hi;
+    const float a = mn - o, b = mx - o;
+    const float m = slack * (fabsf(mn) + fabsf(mx) + 2.f * fabsf(o)) * fmaxf(fabsf(il), fabsf(ih));
+    t_in = fminf(fminf(a * il, a * ih), fminf(b * il, b * ih)) - m;
+    t_out = fmaxf(fmaxf(a * il, a * ih), fmaxf(b * il, b * ih)) + m;
+}
+// The child boxes of one block of 4 children (centre / half-extent halves, index_visit_block's layout) and their cones,
+// against the whole beam: bit c set when child c may be hit by some ray of the beam.  A child is dropped only when every
+// direction of the beam fails slab_ch (interval slab test, NaN keeps the child) or every one is culled by cone_cull_pair.
+RT_D uint32_t beam_visit_block(const float4* nd, bool nocone, const Beam& B) {
+    const float4 q0 = ldg4(nd), q1 = ldg4(nd + 1), q2 = ldg4(nd + 2), q3 = ldg4(nd + 3);
+    const float2 c[3][2] = {{unpack_half2(q0.x), unpack_half2(q0.y)}, {unpack_half2(q0.z), unpack_half2(q0.w)}, {unpack_half2(q1.x), unpack_half2(q1.y)}};
+    const float2 h[3][2] = {{unpack_half2(q1.z), unpack_half2(q1.w)}, {unpack_half2(q2.x), unpack_half2(q2.y)}, {unpack_half2(q2.z), unpack_half2(q2.w)}};
+    const uint32_t ref[4] = {__float_as_uint(q3.x), __float_as_uint(q3.y), __float_as_uint(q3.z), __float_as_uint(q3.w)};
+    const float o[3] = {B.o.x, B.o.y, B.o.z}, lo[3] = {B.lo.x, B.lo.y, B.lo.z}, hi[3] = {B.hi.x, B.hi.y, B.hi.z};
+    float4 q4 = make_float4(0.f, 0.f, 0.f, 0.f), q5 = q4;
+#if RTC_NODE_CONES
+    if (!nocone) { q4 = ldg4(nd + 4); q5 = ldg4(nd + 5); }
+#else
+    (void)nocone;
+#endif
+    const float2 ax[2] = {unpack_half2(q4.x), unpack_half2(q4.y)}, ay[2] = {unpack_half2(q4.z), unpack_half2(q4.w)};
+    const float2 az[2] = {unpack_half2(q5.x), unpack_half2(q5.y)}, th[2] = {unpack_half2(q5.z), unpack_half2(q5.w)};
+    uint32_t mask = 0;
+    for (int i = 0; i < 4; ++i) {
+        if (ref[i] == IREF_NONE) continue;
+        auto pick = [i](const float2* v) { return (i & 1) ? v[i >> 1].y : v[i >> 1].x; };
+        float t1 = -kInfF, t2 = kInfF;
+        for (int a = 0; a < 3; ++a) {
+            const float cc = pick(c[a]), hh = pick(h[a]);
+#if RTC_NODE_CENTRE_HALF
+            const float mn = cc - hh, mx = cc + hh;
+#else
+            const float mn = cc, mx = hh;
+#endif
+            float ti, to;
+            beam_axis(mn, mx, o[a], lo[a], hi[a], kBeamBoxSlack, ti, to);
+            t1 = fmaxf(t1, ti);
+            t2 = fminf(t2, to);
+        }
+        if (t1 > t2 || t2 < 0.f) continue;
+        const float wx = pick(ax), wy = pick(ay), wz = pick(az), thr = pick(th);
+        const float len = sqrtf(wx * wx + wy * wy + wz * wz);
+        if (fabsf(B.c.x * wx + B.c.y * wy + B.c.z * wz) + B.r * len + kBeamConeSlack < thr) continue;
+        mask |= 1u << i;
+    }
+    return mask;
+}
+// The candidate leaves of pixel (x, y) into out[0 .. n) (any order; refs as in the index tree); returns n, or
+// kPixelTraverse.  `visits` (optional) counts the nodes visited.
+//   * More than kMaxRecords candidates: kPixelTraverse (a ray that could need more records takes k_traverse's fallback).
+//   * k_traverse overflows a lane only when, before a visit, its inner-node stack holds more than kStackWords -
+//     (2 kNodeWidth - 1) entries.  Before it visits node u a ray holds at most sum over u's ancestors a of (inner children
+//     of a the ray enters - 1), and a ray enters a subset of what the beam enters; `pend` carries that sum for the beam,
+//     and a pixel where it can reach the limit is kPixelTraverse.
+RT_D uint32_t pixel_candidates(const DevScene& S, const Beam& B, uint32_t* out, uint32_t* visits) {
+    if (S.iroot == IREF_NONE) return kPixelTraverse;
+    if (S.iroot & IREF_LEAF) { out[0] = S.iroot; return 1u; }
+    uint32_t stk[kIndexStack], pst[kIndexStack];
+    int sp = 0;
+    uint32_t n = 0, node = S.iroot, pend = 0;
+    for (;;) {
+        if ((int)pend + (int)(2 * kNodeWidth - 1) > kStackWords) return kPixelTraverse;
+        if (visits) ++*visits;
+        const float4* nd = S.inodes + kIndexNodeF4 * (size_t)(node & IREF_NODE_MASK);
+        const bool nocone = (node & IREF_NOCONE) != 0;
+        uint32_t inner = 0;
+        const int sp0 = sp;
+        for (uint32_t blk = 0; blk < kNodeWidth / 4; ++blk) {
+            const float4* bd = nd + kIndexBlockF4 * blk;
+            const uint32_t m = beam_visit_block(bd, nocone, B);
+            const float4 q3 = ldg4(bd + 3);
+            const uint32_t ref[4] = {__float_as_uint(q3.x), __float_as_uint(q3.y), __float_as_uint(q3.z), __float_as_uint(q3.w)};
+            for (int i = 0; i < 4; ++i) {
+                if (!(m >> i & 1u)) continue;
+                if (ref[i] & IREF_LEAF) {
+                    if (n == (uint32_t)kMaxRecords) return kPixelTraverse;
+                    out[n++] = ref[i];
+                } else {
+                    if (sp == kIndexStack) return kPixelTraverse;
+                    stk[sp++] = ref[i];
+                    ++inner;
+                }
+            }
+        }
+        for (int j = sp0; j < sp; ++j) pst[j] = pend + (inner > 0 ? inner - 1 : 0);
+        if (sp == 0) break;
+        --sp;
+        node = stk[sp];
+        pend = pst[sp];
+    }
+    return n;
+}
+
 }  // namespace rtc

@@ -17,6 +17,7 @@
 namespace rtc {
 
 static_assert(kNodeWidth == 4, "a traverse-queue entry carries the 4 root children a ray enters");
+static_assert(kCandWords == 1 + kMaxRecords, "a pixel candidate list holds up to kMaxRecords leaves");
 constexpr unsigned kFullMask = 0xFFFFFFFFu;
 #ifndef RTC_TRAVERSE_CHUNK
 #define RTC_TRAVERSE_CHUNK 64
@@ -113,9 +114,11 @@ RT_D bool queue_slot(const QueueView& v, uint32_t at, uint32_t cap, uint32_t& sl
 // ------------------------------------------------------------------------------- generate
 // Scene::Sample's jitter + Camera::GetToRay (src/scene.cpp:189-200) through camera C for the camera path of (pixel,
 // sample), stored in slot i with `word` as its pixel word, and its pre_step; returns the root children the ray enters
-// (o, d, cd: what the traverse queue takes).
+// (o, d, cd: what the traverse queue takes).  With `cand` (the pixel lists of k_pixel_candidates, camera C = the scene's
+// own) a pixel that has a list resolves its ray here -- closest plane, leaf_test of every candidate, replay -- and
+// returns 0: the ray is not queued.  `listed` counts those rays.
 RT_D uint32_t camera_path(const DevScene& S, const DevCamera& C, PathSoA P, HitSoA H, uint32_t i, uint32_t pixel, uint32_t word,
-                          uint32_t sample, uint32_t seed, vec3& o, vec3& d, float& cd) {
+                          uint32_t sample, uint32_t seed, const uint32_t* cand, uint32_t& listed, vec3& o, vec3& d, float& cd) {
     uint32_t x = pixel % S.width, y = pixel / S.width;
     Rng g{seed, pixel, sample, 0};
     uint4 b = g.block(0);
@@ -125,12 +128,40 @@ RT_D uint32_t camera_path(const DevScene& S, const DevCamera& C, PathSoA P, HitS
     if (S.dialect == DIALECT_HW3) { fx = __fadd_rn(fx, 0.5f); fy = __fadd_rn(fy, 0.5f); }
     camera_ray(C, S.width, S.height, fx, fy, o, d);
     uint32_t id;
-    const uint32_t enters = pre_step(S, o, d, cd, id);
+    const uint32_t npix = S.width * S.height;
+    const uint32_t n = cand ? __ldg(cand + pixel) : kPixelTraverse;
+    uint32_t enters = 0;
+    if (n == kPixelTraverse) {
+        enters = pre_step(S, o, d, cd, id);
+    } else {
+        int pid;
+        closest_plane(S, o, d, cd, pid);
+        id = pid < 0 ? HIT_MISS : (uint32_t)pid;
+        const vec3 inv = ray_inv(d), oi = o * inv;
+        LeafRec rec[kMaxRecords];
+        int k = 0;
+        for (uint32_t j = 0; j < n; ++j) {
+            const uint32_t ref = __ldg(cand + (size_t)(j + 1) * npix + pixel);
+            float bt, tc; int bid;
+            if (leaf_test(S, ref, o, d, inv, oi, bt, bid, tc, nullptr) && bid >= 0) {
+                rec[k].key = ref & 0xFFFFFFu; rec[k].id = bid; rec[k].t = bt; rec[k].tcull = tc;
+                ++k;
+            }
+        }
+        const BestHit bh = replay_reference(S, o, d, cd, rec, k);
+        if (bh.id != -1 && bh.t < cd) id = (uint32_t)bh.id;   // src/scene.cpp:68-74, as k_traverse stores it
+        ++listed;
+    }
     WF_ST(P.o + i, make_float4(o.x, o.y, o.z, __uint_as_float(sample)));
     WF_ST(P.d + i, make_float4(d.x, d.y, d.z, cd));
     WF_ST(P.beta + i, make_float4(1.f, 1.f, 1.f, __uint_as_float(word)));
     WF_ST(H.id + i, id);
     return enters;
+}
+// camera rays resolved from lists, one atomic per warp: stats[kStatListRays]
+RT_D void count_listed(uint32_t listed, unsigned long long* stats) {
+    const uint32_t sum = __reduce_add_sync(kFullMask, listed);
+    if (sum && (threadIdx.x & 31) == 0) atomicAdd(stats + kStatListRays, (unsigned long long)sum);
 }
 // One thread per path.  Path ids run sample-major over the image: consecutive threads = consecutive pixels of a row.
 // With `views` (nviews cameras) path p is pixel p % npix of view (p / npix) % nviews and sample sample_begin +
@@ -139,10 +170,12 @@ RT_D uint32_t camera_path(const DevScene& S, const DevCamera& C, PathSoA P, HitS
 template <bool VIEWS>
 __global__ void __launch_bounds__(256) k_generate(DevScene S, PathSoA P, HitSoA H, uint32_t* q, uint32_t* tq, uint32_t* tq_count,
                                                    uint64_t first_path, uint32_t count, uint32_t seed, uint32_t sample_begin,
-                                                   const DevCamera* views, uint32_t nviews) {
+                                                   const DevCamera* views, uint32_t nviews, const uint32_t* cand,
+                                                   unsigned long long* stats) {
     const uint32_t npix = S.width * S.height;
     const uint32_t lane = threadIdx.x & 31;
     const uint32_t rounded = (count + 31u) & ~31u;
+    uint32_t listed = 0;
     for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < rounded; i += gridDim.x * blockDim.x) {
         uint32_t enters = 0;
         vec3 o = mk3(0, 0, 0), d = mk3(0, 0, 0);
@@ -153,19 +186,23 @@ __global__ void __launch_bounds__(256) k_generate(DevScene S, PathSoA P, HitSoA 
             uint32_t pixel = (uint32_t)(pid % npix);
             const uint32_t view = VIEWS ? (uint32_t)(frame % nviews) : 0u;
             const uint32_t sample = sample_begin + (uint32_t)(VIEWS ? frame / nviews : frame);
-            enters = camera_path(S, VIEWS ? views[view] : S.cam, P, H, i, pixel, view * npix + pixel, sample, seed, o, d, cd);
+            enters = camera_path(S, VIEWS ? views[view] : S.cam, P, H, i, pixel, view * npix + pixel, sample, seed,
+                                 VIEWS ? nullptr : cand, listed, o, d, cd);
         }
         enqueue(enters, i, o, d, cd, tq, tq_count, lane);
     }
+    if (!VIEWS && cand) count_listed(listed, stats);
     if (blockIdx.x == 0 && threadIdx.x == 0) q[0] = count;
 }
 // The same over a pixel list (adaptive sampling): path id p is pixel plist[p % npix] and sample sample_first +
 // 2 (p / npix) -- every other sample, so that one call renders the even or the odd samples of a range.
 __global__ void __launch_bounds__(256) k_generate_list(DevScene S, PathSoA P, HitSoA H, uint32_t* q, uint32_t* tq, uint32_t* tq_count,
                                                         uint64_t first_path, uint32_t count, uint32_t seed, const uint32_t* plist,
-                                                        uint32_t npix, uint32_t sample_first) {
+                                                        uint32_t npix, uint32_t sample_first, const uint32_t* cand,
+                                                        unsigned long long* stats) {
     const uint32_t lane = threadIdx.x & 31;
     const uint32_t rounded = (count + 31u) & ~31u;
+    uint32_t listed = 0;
     for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < rounded; i += gridDim.x * blockDim.x) {
         uint32_t enters = 0;
         vec3 o = mk3(0, 0, 0), d = mk3(0, 0, 0);
@@ -174,11 +211,32 @@ __global__ void __launch_bounds__(256) k_generate_list(DevScene S, PathSoA P, Hi
             uint64_t pid = first_path + i;
             uint32_t sample = sample_first + 2u * (uint32_t)(pid / npix);
             uint32_t pixel = plist[pid % npix];
-            enters = camera_path(S, S.cam, P, H, i, pixel, pixel, sample, seed, o, d, cd);
+            enters = camera_path(S, S.cam, P, H, i, pixel, pixel, sample, seed, cand, listed, o, d, cd);
         }
         enqueue(enters, i, o, d, cd, tq, tq_count, lane);
     }
+    if (cand) count_listed(listed, stats);
     if (blockIdx.x == 0 && threadIdx.x == 0) q[0] = count;
+}
+
+// One thread per pixel: the candidate leaves of its beam through the scene's camera (rt_device.cuh pixel_candidates),
+// slot j of the list at cand[(1 + j) npix + pixel] and its length (or kPixelTraverse) at cand[pixel], so that the
+// consecutive pixels of k_generate's warps read consecutive words.  count_visits: node visits into stats[4].
+__global__ void __launch_bounds__(128) k_pixel_candidates(DevScene S, uint32_t* cand, bool count_visits, unsigned long long* stats) {
+    const uint32_t npix = S.width * S.height;
+    uint32_t visits = 0;
+    for (uint32_t p = blockIdx.x * blockDim.x + threadIdx.x; p < npix; p += gridDim.x * blockDim.x) {
+        const Beam B = pixel_beam(S.cam, S.width, S.height, S.dialect, p % S.width, p / S.width);
+        uint32_t refs[kMaxRecords];
+        const uint32_t n = pixel_candidates(S, B, refs, &visits);
+        cand[p] = n;
+        if (n != kPixelTraverse)
+            for (uint32_t j = 0; j < n; ++j) cand[(size_t)(j + 1) * npix + p] = refs[j];
+    }
+    if (count_visits) {
+        const uint32_t sum = __reduce_add_sync(kFullMask, visits);
+        if (sum && (threadIdx.x & 31) == 0) atomicAdd(stats + 4, (unsigned long long)sum);
+    }
 }
 
 // ------------------------------------------------------------------------------- extend, step 1
@@ -220,7 +278,7 @@ __global__ void __launch_bounds__(256) k_pre(DevScene S, PathSoA P, HitSoA H, co
 // profiles/r02_experiments.md.)
 // FINISH and REFILL as one kind of scheduler work: measured on B200 11.52 -> 10.90 ms (the two used to cost a vote and a
 // partly filled warp iteration each: 5.3 M + 5.4 M iterations per frame at 15.7 / 17.7 lanes)
-constexpr int kStackWords = 56;  // per lane: inner-node stack from the bottom, noted leaves from the top
+// per lane: kStackWords (rt_device.cuh) words, inner-node stack from the bottom, noted leaves from the top
 #define STK(i) stk[i]
 constexpr uint32_t kNone = 0xFFFFFFFFu;
 #ifndef RTC_LEAF_FIRST
@@ -1004,18 +1062,25 @@ static int grid_for(uint64_t n, int block, int sms, int per_sm) {
 }
 
 void launch_generate(const LaunchCtx& c, const DevScene& S, PathSoA P, HitSoA H, uint32_t* q, uint32_t* tq, uint32_t* tq_count,
-                     uint64_t first_path, uint32_t count, uint32_t seed, uint32_t sample_begin, const DevCamera* views, uint32_t nviews) {
+                     uint64_t first_path, uint32_t count, uint32_t seed, uint32_t sample_begin, const DevCamera* views, uint32_t nviews,
+                     const uint32_t* cand, unsigned long long* stats) {
     if (views)
         k_generate<true><<<grid_for(count, 256, c.sms, 8), 256, 0, c.stream>>>(S, P, H, q, tq, tq_count, first_path, count, seed,
-                                                                               sample_begin, views, nviews);
+                                                                               sample_begin, views, nviews, nullptr, nullptr);
     else
         k_generate<false><<<grid_for(count, 256, c.sms, 8), 256, 0, c.stream>>>(S, P, H, q, tq, tq_count, first_path, count, seed,
-                                                                                sample_begin, nullptr, 1);
+                                                                                sample_begin, nullptr, 1, cand, stats);
 }
 void launch_generate_list(const LaunchCtx& c, const DevScene& S, PathSoA P, HitSoA H, uint32_t* q, uint32_t* tq, uint32_t* tq_count,
-                          uint64_t first_path, uint32_t count, uint32_t seed, const uint32_t* plist, uint32_t npix, uint32_t sample_first) {
+                          uint64_t first_path, uint32_t count, uint32_t seed, const uint32_t* plist, uint32_t npix, uint32_t sample_first,
+                          const uint32_t* cand, unsigned long long* stats) {
     k_generate_list<<<grid_for(count, 256, c.sms, 8), 256, 0, c.stream>>>(S, P, H, q, tq, tq_count, first_path, count, seed, plist,
-                                                                          npix, sample_first);
+                                                                          npix, sample_first, cand, stats);
+}
+void launch_pixel_candidates(const LaunchCtx& c, const DevScene& S, uint32_t* cand, bool count_visits, unsigned long long* stats) {
+    const uint32_t npix = S.width * S.height;
+    if (npix == 0) return;
+    k_pixel_candidates<<<grid_for(npix, 128, c.sms, 16), 128, 0, c.stream>>>(S, cand, count_visits, stats);
 }
 void launch_adaptive_tiles(const LaunchCtx& c, const float4* A, const float4* B, uint32_t width, uint32_t height,
                            const uint32_t* tiles_in, uint32_t ntiles, uint32_t n, float inv_a, float inv_b, float tau, int mode,

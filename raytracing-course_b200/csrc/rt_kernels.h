@@ -20,12 +20,21 @@ struct LaunchCtx {
 
 // camera rays of one wavefront batch + their pre_step (planes, index root, traverse queue): through the scene's camera
 // (views = null), or through nviews cameras, path p = pixel p % npix of view (p / npix) % nviews, sample sample_begin +
-// p / (npix nviews), pixel word view npix + pixel
+// p / (npix nviews), pixel word view npix + pixel.  cand (scene camera only, may be null): the pixel candidate lists of
+// launch_pixel_candidates; a pixel with a list resolves its camera rays in the kernel, counted in stats[kStatListRays]
 void launch_generate(const LaunchCtx& c, const DevScene& S, PathSoA P, HitSoA H, uint32_t* q, uint32_t* tq, uint32_t* tq_count,
-                     uint64_t first_path, uint32_t count, uint32_t seed, uint32_t sample_begin, const DevCamera* views, uint32_t nviews);
+                     uint64_t first_path, uint32_t count, uint32_t seed, uint32_t sample_begin, const DevCamera* views, uint32_t nviews,
+                     const uint32_t* cand, unsigned long long* stats);
 // the same over a pixel list: path p = pixel plist[p % npix], sample sample_first + 2 (p / npix)
 void launch_generate_list(const LaunchCtx& c, const DevScene& S, PathSoA P, HitSoA H, uint32_t* q, uint32_t* tq, uint32_t* tq_count,
-                          uint64_t first_path, uint32_t count, uint32_t seed, const uint32_t* plist, uint32_t npix, uint32_t sample_first);
+                          uint64_t first_path, uint32_t count, uint32_t seed, const uint32_t* plist, uint32_t npix, uint32_t sample_first,
+                          const uint32_t* cand, unsigned long long* stats);
+// Per pixel of the scene's camera the candidate index leaves of its camera rays (rt_device.cuh pixel_candidates):
+// kCandWords words per pixel, laid out slot-major (word j of pixel p at cand[j npix + p]); word 0 is the list length or
+// kPixelTraverse.  count_visits: its node visits into stats[4].
+constexpr uint32_t kCandWords = 1 + 24;   // length + kMaxRecords leaf refs
+constexpr int kStatListRays = 16;         // stats word: camera rays resolved from candidate lists
+void launch_pixel_candidates(const LaunchCtx& c, const DevScene& S, uint32_t* cand, bool count_visits, unsigned long long* stats);
 // adaptive sampling (rtc_render_adaptive): square tiles of kAdaptiveTile pixels a side (= RTC_ADAPTIVE_TILE), one warp each
 constexpr uint32_t kAdaptiveTile = 8;
 static_assert(kAdaptiveTile * kAdaptiveTile == 64, "k_adaptive_tiles: one warp per tile, two pixels per lane");
