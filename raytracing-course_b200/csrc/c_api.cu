@@ -1381,56 +1381,6 @@ int adaptive_passes(rtc_scene* c, cudaStream_t user, uint32_t shard, uint32_t ns
     return arena_end(c, user);
 }
 }  // namespace
-int rtc_render_adaptive(rtc_scene* s, uint32_t seed, float tolerance, uint32_t min_samples, uint32_t max_samples,
-                        uint8_t* rgb_host, float* halves_host, uint32_t* spp_host, uint64_t stats[4]) {
-    if (!s) return fail(RTC_ERR_ARG, "null scene");
-    if (!std::isfinite(tolerance) || tolerance < 0.f) return fail(RTC_ERR_ARG, "tolerance must be finite and >= 0");
-    if (min_samples < 2) return fail(RTC_ERR_ARG, "min_samples must be at least 2");
-    int rc = need_device(s);
-    if (rc) return rc;
-    const uint32_t width = s->host.cam.width, height = s->host.cam.height;
-    const uint32_t npix = width * height;
-    const uint32_t ntiles = adaptive_tiles(width, height);
-    uint64_t st[4] = {0, 0, 0, 0};   // passes, paths, tiles, tiles stopped below the maximum
-    if (stats) std::memcpy(stats, st, sizeof st);
-    if (npix == 0) return RTC_OK;
-    const size_t nvalues = 3 * (size_t)npix;
-    CU(s->rgb.ensure(nvalues));
-    if (s->host.dialect <= DIALECT_HW2) {
-        // hw1 / hw2: the one deterministic frame, resolved as rtc_render_u8 does; it is the "even" half, spp = 1
-        CU(s->accum.ensure(nvalues));
-        if ((rc = render_frame(s, seed, 1, s->accum.p, s->rgb.p, nullptr))) return rc;
-        if (rgb_host) CU(cudaMemcpy(rgb_host, s->rgb.p, nvalues, cudaMemcpyDeviceToHost));
-        if (halves_host) {
-            std::vector<float> frame(nvalues);
-            CU(cudaMemcpy(frame.data(), s->accum.p, nvalues * sizeof(float), cudaMemcpyDeviceToHost));
-            for (size_t i = 0; i < npix; ++i)
-                for (int c = 0; c < 3; ++c) { halves_host[6 * i + c] = frame[3 * i + c]; halves_host[6 * i + 3 + c] = 0.f; }
-        }
-        if (spp_host) for (size_t i = 0; i < npix; ++i) spp_host[i] = 1;
-        const uint64_t one[4] = {1, npix, ntiles, 0};
-        if (stats) std::memcpy(stats, one, sizeof one);
-        return RTC_OK;
-    }
-    const uint32_t smax = max_samples ? max_samples : s->host.samples;
-    if (smax == 0) return fail(RTC_ERR_ARG, "scene has SAMPLES 0");
-    cudaStream_t user = nullptr;
-    st[2] = ntiles;
-    if ((rc = adaptive_passes(s, user, 0, 1, seed, tolerance, min_samples, smax, st))) return rc;
-    rtc_scene::Adaptive& ad = s->adaptive;
-    CU(ad.halves.ensure(halves_host ? 6 * (size_t)npix : 0));
-    CU(ad.spp.ensure(spp_host ? npix : 0));
-    launch_resolve_adaptive(LaunchCtx{user, s->sms}, ad.half[0].p, ad.half[1].p, ad.tile_n.p, width, npix, s->rgb.p,
-                            halves_host ? ad.halves.p : nullptr, spp_host ? ad.spp.p : nullptr);
-    s->launches++;
-    CU(cudaGetLastError());
-    if (rgb_host) CU(cudaMemcpy(rgb_host, s->rgb.p, nvalues, cudaMemcpyDeviceToHost));
-    if (halves_host) CU(cudaMemcpy(halves_host, ad.halves.p, 6 * (size_t)npix * sizeof(float), cudaMemcpyDeviceToHost));
-    if (spp_host) CU(cudaMemcpy(spp_host, ad.spp.p, (size_t)npix * sizeof(uint32_t), cudaMemcpyDeviceToHost));
-    CU(cudaStreamSynchronize(user));
-    if (stats) std::memcpy(stats, st, sizeof st);
-    return RTC_OK;
-}
 
 // ------------------------------------------------------------------ denoising
 namespace {
@@ -1438,41 +1388,17 @@ int check_strength(float strength) {
     if (!std::isfinite(strength) || strength < 0.f) return fail(RTC_ERR_ARG, "strength must be finite and >= 0");
     return RTC_OK;
 }
-// The filter on the half sums and sample counts in halves_dev / spp_dev (the layout of k_resolve_adaptive's optional
-// outputs, every spp >= 2), on the default stream: k_denoise_prep, then k_denoise_nlm unless strength is 0 (then the
-// image is that of the mean u, as rtc_render_adaptive resolves it).  Copies the image and the mean to the host.
-int denoise(rtc_scene* s, const float* halves_dev, const uint32_t* spp_dev, float strength, uint8_t* rgb_host, float* mean_host) {
-    const uint32_t width = s->host.cam.width, height = s->host.cam.height, npix = width * height;
-    rtc_scene::Denoise& dn = s->denoise;
-    CU(dn.u.ensure(3 * (size_t)npix));
-    CU(dn.d.ensure(npix));
-    CU(dn.v.ensure(npix));
-    CU(s->rgb.ensure(3 * (size_t)npix));
-    const LaunchCtx lc{nullptr, s->sms};
-    const bool filter = strength > 0.f;
-    launch_denoise_prep(lc, halves_dev, spp_dev, npix, dn.u.p, dn.d.p, dn.v.p, filter ? nullptr : s->rgb.p);
-    s->launches++;
-    CU(cudaGetLastError());
-    if (filter) {
-        CU(dn.mean.ensure(3 * (size_t)npix));
-        // k^2 saturates instead of overflowing: the weights are then all 1 where the patches' variance is non-zero
-        CU(launch_denoise_nlm(lc, dn.u.p, dn.d.p, dn.v.p, width, height, 0, (height + kDenoiseTileH - 1) / kDenoiseTileH, 0,
-                              std::fmin(strength * strength, FLT_MAX), dn.mean.p, s->rgb.p));
-        s->launches++;
-    }
-    if (rgb_host) CU(cudaMemcpy(rgb_host, s->rgb.p, 3 * (size_t)npix, cudaMemcpyDeviceToHost));
-    if (mean_host) CU(cudaMemcpy(mean_host, filter ? dn.mean.p : dn.u.p, 3 * (size_t)npix * sizeof(float), cudaMemcpyDeviceToHost));
-    CU(cudaStreamSynchronize(nullptr));
-    return RTC_OK;
-}
 }  // namespace
+// The filter on the caller's half sums and sample counts (every spp >= 2), on the default stream: k_denoise_prep, then
+// k_denoise_nlm unless strength is 0 (then the image is that of the mean u, as an adaptive render resolves it).
 int rtc_denoise(rtc_scene* s, const float* halves_host, const uint32_t* spp_host, float strength, uint8_t* rgb_host, float* mean_host) {
     if (!s) return fail(RTC_ERR_ARG, "null scene");
     if (!halves_host || !spp_host) return fail(RTC_ERR_ARG, "null halves or spp");
     int rc = check_strength(strength);
     if (rc) return rc;
     if (s->host.dialect <= DIALECT_HW2) return fail(RTC_ERR_ARG, "hw1 / hw2 scenes have no noise to filter");
-    const size_t npix = (size_t)s->host.cam.width * s->host.cam.height;
+    const uint32_t width = s->host.cam.width, height = s->host.cam.height;
+    const size_t npix = (size_t)width * height;
     for (size_t i = 0; i < npix; ++i)
         if (spp_host[i] < 2) return fail(RTC_ERR_ARG, "every pixel needs at least 2 samples (pixel " + std::to_string(i) + ")");
     if ((rc = need_device(s))) return rc;
@@ -1482,40 +1408,26 @@ int rtc_denoise(rtc_scene* s, const float* halves_host, const uint32_t* spp_host
     CU(ad.spp.ensure(npix));
     CU(cudaMemcpy(ad.halves.p, halves_host, 6 * npix * sizeof(float), cudaMemcpyHostToDevice));
     CU(cudaMemcpy(ad.spp.p, spp_host, npix * sizeof(uint32_t), cudaMemcpyHostToDevice));
-    return denoise(s, ad.halves.p, ad.spp.p, strength, rgb_host, mean_host);
-}
-int rtc_render_denoised(rtc_scene* s, uint32_t seed, float tolerance, uint32_t min_samples, uint32_t max_samples, float strength,
-                        uint8_t* rgb_host, float* mean_host, uint64_t stats[4]) {
-    if (!s) return fail(RTC_ERR_ARG, "null scene");
-    int rc = check_strength(strength);
-    if (rc) return rc;
-    const uint32_t width = s->host.cam.width, height = s->host.cam.height, npix = width * height;
-    if (s->host.dialect <= DIALECT_HW2) {
-        // the one deterministic frame, unfiltered: rtc_render_adaptive's, whose mean is the frame it leaves in s->accum
-        if ((rc = rtc_render_adaptive(s, seed, tolerance, min_samples, max_samples, rgb_host, nullptr, nullptr, stats))) return rc;
-        if (mean_host && npix) CU(cudaMemcpy(mean_host, s->accum.p, 3 * (size_t)npix * sizeof(float), cudaMemcpyDeviceToHost));
-        return RTC_OK;
-    }
-    if (!std::isfinite(tolerance) || tolerance < 0.f) return fail(RTC_ERR_ARG, "tolerance must be finite and >= 0");
-    if (min_samples < 2) return fail(RTC_ERR_ARG, "min_samples must be at least 2");
-    const uint32_t smax = max_samples ? max_samples : s->host.samples;
-    if (smax < 2) return fail(RTC_ERR_ARG, "the maximum sample count must be at least 2");
-    if ((rc = need_device(s))) return rc;
-    uint64_t st[4] = {0, 0, 0, 0};   // passes, paths, tiles, tiles stopped below the maximum
-    if (stats) std::memcpy(stats, st, sizeof st);
-    if (npix == 0) return RTC_OK;
-    st[2] = adaptive_tiles(width, height);
-    if ((rc = adaptive_passes(s, nullptr, 0, 1, seed, tolerance, min_samples, smax, st))) return rc;
-    rtc_scene::Adaptive& ad = s->adaptive;
-    CU(s->rgb.ensure(3 * (size_t)npix));
-    CU(ad.halves.ensure(6 * (size_t)npix));
-    CU(ad.spp.ensure(npix));
-    launch_resolve_adaptive(LaunchCtx{nullptr, s->sms}, ad.half[0].p, ad.half[1].p, ad.tile_n.p, width, npix, s->rgb.p, ad.halves.p,
-                            ad.spp.p);
+    rtc_scene::Denoise& dn = s->denoise;
+    CU(dn.u.ensure(3 * npix));
+    CU(dn.d.ensure(npix));
+    CU(dn.v.ensure(npix));
+    CU(s->rgb.ensure(3 * npix));
+    const LaunchCtx lc{nullptr, s->sms};
+    const bool filter = strength > 0.f;
+    launch_denoise_prep(lc, ad.halves.p, ad.spp.p, (uint32_t)npix, dn.u.p, dn.d.p, dn.v.p, filter ? nullptr : s->rgb.p);
     s->launches++;
     CU(cudaGetLastError());
-    if ((rc = denoise(s, ad.halves.p, ad.spp.p, strength, rgb_host, mean_host))) return rc;
-    if (stats) std::memcpy(stats, st, sizeof st);
+    if (filter) {
+        CU(dn.mean.ensure(3 * npix));
+        // k^2 saturates instead of overflowing: the weights are then all 1 where the patches' variance is non-zero
+        CU(launch_denoise_nlm(lc, dn.u.p, dn.d.p, dn.v.p, width, height, 0, (height + kDenoiseTileH - 1) / kDenoiseTileH, 0,
+                              std::fmin(strength * strength, FLT_MAX), dn.mean.p, s->rgb.p));
+        s->launches++;
+    }
+    if (rgb_host) CU(cudaMemcpy(rgb_host, s->rgb.p, 3 * npix, cudaMemcpyDeviceToHost));
+    if (mean_host) CU(cudaMemcpy(mean_host, filter ? dn.mean.p : dn.u.p, 3 * npix * sizeof(float), cudaMemcpyDeviceToHost));
+    CU(cudaStreamSynchronize(nullptr));
     return RTC_OK;
 }
 
@@ -1737,14 +1649,19 @@ int rtc_render_ppm_multi(rtc_scene* s, const int* devices, int ndev, uint32_t se
     return rc ? rc : write_ppm(out_path, s->host.cam.width, s->host.cam.height, img);
 }
 
-// Adaptive sampling on several devices: tile t of the frame belongs to devices[t % ndev], and every device runs the
-// pass loop of rtc_render_adaptive on its own tiles, on its own stream and host thread.  A tile's decisions read only its
-// own half sums, so the devices do not talk to each other until devices[0] resolves every pixel from its owner's
-// half sums and tile counts (k_resolve_adaptive_peers).
+// Adaptive sampling on one or several devices: tile t of the frame belongs to devices[t % ndev], and every device runs
+// the pass loop on its own tiles, on its own stream and host thread.  A tile's decisions read only its own half sums,
+// so the devices do not talk to each other until devices[0] resolves every pixel from its owner's half sums and tile
+// counts (k_resolve_adaptive_peers).  The one-device calls are the list of the scene's own device alone.
 namespace {
-int check_adaptive_multi_args(float tolerance, uint32_t min_samples, const int* devices, int ndev) {
+int check_adaptive_args(float tolerance, uint32_t min_samples) {
     if (!std::isfinite(tolerance) || tolerance < 0.f) return fail(RTC_ERR_ARG, "tolerance must be finite and >= 0");
     if (min_samples < 2) return fail(RTC_ERR_ARG, "min_samples must be at least 2");
+    return RTC_OK;
+}
+int check_adaptive_multi_args(float tolerance, uint32_t min_samples, const int* devices, int ndev) {
+    int rc = check_adaptive_args(tolerance, min_samples);
+    if (rc) return rc;
     if (!devices || ndev < 1 || ndev > kMaxPeers) return fail(RTC_ERR_ARG, "devices must list 1 to 16 entries");
     for (int i = 0; i < ndev; ++i)
         if (devices[i] < 0 || devices[i] >= 64) return fail(RTC_ERR_ARG, "bad device index");
@@ -1806,93 +1723,133 @@ int owner_halves(rtc_scene* c, const std::vector<rtc_scene*>& ctx, uint32_t widt
     }
     return RTC_OK;
 }
-}  // namespace
-int rtc_render_adaptive_multi(rtc_scene* s, const int* devices, int ndev, uint32_t seed, float tolerance, uint32_t min_samples,
-                              uint32_t max_samples, uint8_t* rgb_host, float* halves_host, uint32_t* spp_host, uint64_t stats[4]) {
-    if (!s) return fail(RTC_ERR_ARG, "null scene");
-    int rc = check_adaptive_multi_args(tolerance, min_samples, devices, ndev);
+// Every pixel of the frame resolved on entry `c` (its device current) after adaptive_passes_multi, from the half sums and
+// tile count of its tile's owner: the 8-bit image into c->rgb and, when their host pointers are given, the half sums
+// and spp.  The copies to the given host pointers are queued on c's multi_stream, not waited for.
+int gather_adaptive(rtc_scene* c, const std::vector<rtc_scene*>& ctx, uint8_t* rgb_host, float* halves_host, uint32_t* spp_host,
+                    std::vector<DevBuf<unsigned char>>& staged) {
+    const uint32_t width = c->host.cam.width, height = c->host.cam.height, npix = width * height;
+    const cudaStream_t st = c->multi_stream;
+    PeerHalves P;
+    int rc = owner_halves(c, ctx, width, 0, height, adaptive_tiles(width, height), staged, &P);
     if (rc) return rc;
-    rc = need_device(s);
+    rtc_scene::Adaptive& ad = c->adaptive;
+    CU(c->rgb.ensure(3 * (size_t)npix));
+    CU(ad.halves.ensure(halves_host ? 6 * (size_t)npix : 0));
+    CU(ad.spp.ensure(spp_host ? npix : 0));
+    launch_resolve_adaptive_peers(LaunchCtx{st, c->sms}, P, width, npix, c->rgb.p, halves_host ? ad.halves.p : nullptr,
+                                  spp_host ? ad.spp.p : nullptr);
+    c->launches++;
+    CU(cudaGetLastError());
+    if (rgb_host) CU(cudaMemcpyAsync(rgb_host, c->rgb.p, 3 * (size_t)npix, cudaMemcpyDeviceToHost, st));
+    if (halves_host) CU(cudaMemcpyAsync(halves_host, ad.halves.p, 6 * (size_t)npix * sizeof(float), cudaMemcpyDeviceToHost, st));
+    if (spp_host) CU(cudaMemcpyAsync(spp_host, ad.spp.p, (size_t)npix * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+    return RTC_OK;
+}
+// hw1 / hw2 have no samples to adapt: their one deterministic frame on context `c`, rendered and resolved as
+// rtc_render_u8 does, on the legacy default stream.  It is the "even" half with spp 1, its mean is the frame itself (left
+// in c->accum), and it is one pass over every tile.
+int deterministic_frame(rtc_scene* c, uint32_t seed, uint8_t* rgb_host, float* halves_host, uint32_t* spp_host, float* mean_host,
+                        uint64_t st[4]) {
+    const uint32_t width = c->host.cam.width, height = c->host.cam.height, npix = width * height;
+    const size_t nvalues = 3 * (size_t)npix;
+    CU(cudaSetDevice(c->device));
+    CU(c->rgb.ensure(nvalues));
+    CU(c->accum.ensure(nvalues));
+    int rc = render_frame(c, seed, 1, c->accum.p, c->rgb.p, nullptr);
     if (rc) return rc;
+    if (rgb_host) CU(cudaMemcpy(rgb_host, c->rgb.p, nvalues, cudaMemcpyDeviceToHost));
+    if (halves_host) {
+        std::vector<float> frame(nvalues);
+        CU(cudaMemcpy(frame.data(), c->accum.p, nvalues * sizeof(float), cudaMemcpyDeviceToHost));
+        for (size_t i = 0; i < npix; ++i)
+            for (int k = 0; k < 3; ++k) { halves_host[6 * i + k] = frame[3 * i + k]; halves_host[6 * i + 3 + k] = 0.f; }
+    }
+    if (spp_host) for (size_t i = 0; i < npix; ++i) spp_host[i] = 1;
+    if (mean_host) CU(cudaMemcpy(mean_host, c->accum.p, nvalues * sizeof(float), cudaMemcpyDeviceToHost));
+    const uint64_t one[4] = {1, npix, adaptive_tiles(width, height), 0};
+    std::memcpy(st, one, sizeof one);
+    return RTC_OK;
+}
+// The adaptive render of scene s (its device current, arguments checked) on the entries `devices`
+int adaptive_render(rtc_scene* s, const int* devices, int ndev, uint32_t seed, float tolerance, uint32_t min_samples,
+                    uint32_t max_samples, uint8_t* rgb_host, float* halves_host, uint32_t* spp_host, uint64_t stats[4]) {
     const uint32_t width = s->host.cam.width, height = s->host.cam.height;
     const uint32_t npix = width * height, ntiles = adaptive_tiles(width, height);
     uint64_t st[4] = {0, 0, 0, 0};   // passes (the most of any device), paths, tiles, tiles stopped below the maximum
     if (stats) std::memcpy(stats, st, sizeof st);
     if (npix == 0) return RTC_OK;
-    const size_t nvalues = 3 * (size_t)npix;
+    int rc;
     if (s->host.dialect <= DIALECT_HW2) {
-        // one deterministic frame, not split: rtc_render_adaptive on the first listed device
+        // one deterministic frame, not split: on the first listed device
         rtc_scene* head = replica_on(s, devices[0], 0);
         if (!head) return RTC_ERR_CUDA;
-        if ((rc = rtc_render_adaptive(head, seed, tolerance, min_samples, max_samples, rgb_host, halves_host, spp_host, stats)))
-            return rc;
-        CU(cudaSetDevice(s->device));
-        return RTC_OK;
+        if ((rc = deterministic_frame(head, seed, rgb_host, halves_host, spp_host, nullptr, st))) return rc;
+    } else {
+        const uint32_t smax = max_samples ? max_samples : s->host.samples;
+        if (smax == 0) return fail(RTC_ERR_ARG, "scene has SAMPLES 0");
+        std::vector<rtc_scene*> ctx;
+        if ((rc = device_contexts(s, devices, ndev, ctx))) return rc;
+        rtc_scene* head = ctx[0];
+        if ((rc = adaptive_passes_multi(ctx, seed, tolerance, min_samples, smax, ntiles, st))) return rc;
+        // the head device reads the owners' half sums and tile counts in place (peer access), or copies them over
+        CU(cudaSetDevice(head->device));
+        std::vector<DevBuf<unsigned char>> staged;
+        if ((rc = gather_adaptive(head, ctx, rgb_host, halves_host, spp_host, staged))) return rc;
+        CU(cudaStreamSynchronize(head->multi_stream));
+        staged.clear();   // while the head device is current
     }
-    const uint32_t smax = max_samples ? max_samples : s->host.samples;
-    if (smax == 0) return fail(RTC_ERR_ARG, "scene has SAMPLES 0");
-    std::vector<rtc_scene*> ctx;
-    if ((rc = device_contexts(s, devices, ndev, ctx))) return rc;
-    rtc_scene* head = ctx[0];
-    if ((rc = adaptive_passes_multi(ctx, seed, tolerance, min_samples, smax, ntiles, st))) return rc;
-    // the head device reads the owners' half sums and tile counts in place (peer access), or copies them over
-    CU(cudaSetDevice(head->device));
-    PeerHalves P;
-    std::vector<DevBuf<unsigned char>> staged;
-    if ((rc = owner_halves(head, ctx, width, 0, height, ntiles, staged, &P))) return rc;
-    rtc_scene::Adaptive& ad = head->adaptive;
-    CU(head->rgb.ensure(nvalues));
-    CU(ad.halves.ensure(halves_host ? 6 * (size_t)npix : 0));
-    CU(ad.spp.ensure(spp_host ? npix : 0));
-    launch_resolve_adaptive_peers(LaunchCtx{head->multi_stream, head->sms}, P, width, npix, head->rgb.p,
-                                  halves_host ? ad.halves.p : nullptr, spp_host ? ad.spp.p : nullptr);
-    head->launches++;
-    CU(cudaGetLastError());
-    if (rgb_host) CU(cudaMemcpyAsync(rgb_host, head->rgb.p, nvalues, cudaMemcpyDeviceToHost, head->multi_stream));
-    if (halves_host)
-        CU(cudaMemcpyAsync(halves_host, ad.halves.p, 6 * (size_t)npix * sizeof(float), cudaMemcpyDeviceToHost, head->multi_stream));
-    if (spp_host) CU(cudaMemcpyAsync(spp_host, ad.spp.p, (size_t)npix * sizeof(uint32_t), cudaMemcpyDeviceToHost, head->multi_stream));
-    CU(cudaStreamSynchronize(head->multi_stream));
-    staged.clear();   // while the head device is current
     CU(cudaSetDevice(s->device));
     if (stats) std::memcpy(stats, st, sizeof st);
     return RTC_OK;
 }
-
-// Denoising on several devices: rtc_render_adaptive_multi's passes, then entry i filters the image rows of the tile rows
-// [i T / n, (i + 1) T / n) of k_denoise_nlm's grid (T = ceil(H / kDenoiseTileH)), so that the bands together are the
-// one-device grid block for block.  It reads the rows it filters and kDenoiseApron more on either side from the tiles'
-// owners where they lie, on its own stream and host thread, and copies its rows of the image and the mean to the host.
-int rtc_render_denoised_multi(rtc_scene* s, const int* devices, int ndev, uint32_t seed, float tolerance, uint32_t min_samples,
-                              uint32_t max_samples, float strength, uint8_t* rgb_host, float* mean_host, float* halves_host,
-                              uint32_t* spp_host, uint64_t stats[4]) {
+}  // namespace
+int rtc_render_adaptive(rtc_scene* s, uint32_t seed, float tolerance, uint32_t min_samples, uint32_t max_samples,
+                        uint8_t* rgb_host, float* halves_host, uint32_t* spp_host, uint64_t stats[4]) {
     if (!s) return fail(RTC_ERR_ARG, "null scene");
-    int rc = check_strength(strength);
+    int rc = check_adaptive_args(tolerance, min_samples);
     if (rc) return rc;
-    if ((rc = check_adaptive_multi_args(tolerance, min_samples, devices, ndev))) return rc;
-    const bool deterministic = s->host.dialect <= DIALECT_HW2;
-    const uint32_t smax = max_samples ? max_samples : s->host.samples;
-    if (!deterministic && smax < 2) return fail(RTC_ERR_ARG, "the maximum sample count must be at least 2");
     if ((rc = need_device(s))) return rc;
+    return adaptive_render(s, &s->device, 1, seed, tolerance, min_samples, max_samples, rgb_host, halves_host, spp_host, stats);
+}
+int rtc_render_adaptive_multi(rtc_scene* s, const int* devices, int ndev, uint32_t seed, float tolerance, uint32_t min_samples,
+                              uint32_t max_samples, uint8_t* rgb_host, float* halves_host, uint32_t* spp_host, uint64_t stats[4]) {
+    if (!s) return fail(RTC_ERR_ARG, "null scene");
+    int rc = check_adaptive_multi_args(tolerance, min_samples, devices, ndev);
+    if (rc) return rc;
+    if ((rc = need_device(s))) return rc;
+    return adaptive_render(s, devices, ndev, seed, tolerance, min_samples, max_samples, rgb_host, halves_host, spp_host, stats);
+}
+
+// Denoising on one or several devices: adaptive_render's passes, then entry i filters the image rows of the tile rows
+// [i T / n, (i + 1) T / n) of k_denoise_nlm's grid (T = ceil(H / kDenoiseTileH)), so that the bands together are the
+// whole-frame grid block for block.  It reads the rows it filters and kDenoiseApron more on either side from the tiles'
+// owners where they lie, on its own stream and host thread, and copies its rows of the image and the mean to the host.
+namespace {
+int denoised_render(rtc_scene* s, const int* devices, int ndev, uint32_t seed, float tolerance, uint32_t min_samples,
+                    uint32_t max_samples, float strength, uint8_t* rgb_host, float* mean_host, float* halves_host,
+                    uint32_t* spp_host, uint64_t stats[4]) {
     const uint32_t width = s->host.cam.width, height = s->host.cam.height;
     const uint32_t npix = width * height, ntiles = adaptive_tiles(width, height);
     uint64_t st[4] = {0, 0, 0, 0};
     if (stats) std::memcpy(stats, st, sizeof st);
     if (npix == 0) return RTC_OK;
-    if (deterministic) {
-        // rtc_render_denoised's unfiltered frame on the first listed device, with rtc_render_adaptive's halves and spp
+    int rc;
+    if (s->host.dialect <= DIALECT_HW2) {
+        // the one deterministic frame, unfiltered, on the first listed device
         rtc_scene* head = replica_on(s, devices[0], 0);
         if (!head) return RTC_ERR_CUDA;
-        if ((rc = rtc_render_adaptive(head, seed, tolerance, min_samples, max_samples, rgb_host, halves_host, spp_host, stats))) return rc;
-        if (mean_host) CU(cudaMemcpy(mean_host, head->accum.p, 3 * (size_t)npix * sizeof(float), cudaMemcpyDeviceToHost));
+        if ((rc = deterministic_frame(head, seed, rgb_host, halves_host, spp_host, mean_host, st))) return rc;
         CU(cudaSetDevice(s->device));
+        if (stats) std::memcpy(stats, st, sizeof st);
         return RTC_OK;
     }
+    const uint32_t smax = max_samples ? max_samples : s->host.samples;
     std::vector<rtc_scene*> ctx;
     if ((rc = device_contexts(s, devices, ndev, ctx))) return rc;
     if ((rc = adaptive_passes_multi(ctx, seed, tolerance, min_samples, smax, ntiles, st))) return rc;
     const bool filter = strength > 0.f;
-    const float k2 = std::fmin(strength * strength, FLT_MAX);   // as in denoise()
+    const float k2 = std::fmin(strength * strength, FLT_MAX);   // as in rtc_denoise
     const uint32_t tile_rows = (height + kDenoiseTileH - 1) / kDenoiseTileH;
     auto band = [&](int i) -> int {
         rtc_scene* c = ctx[i];
@@ -1903,17 +1860,8 @@ int rtc_render_denoised_multi(rtc_scene* s, const int* devices, int ndev, uint32
         PeerHalves P;
         int r;
         if (i == 0 && (halves_host || spp_host)) {
-            // the whole half sums and spp, as rtc_render_adaptive_multi gathers them
-            rtc_scene::Adaptive& ad = c->adaptive;
-            CU(c->rgb.ensure(3 * (size_t)npix));
-            CU(ad.halves.ensure(halves_host ? 6 * (size_t)npix : 0));
-            CU(ad.spp.ensure(spp_host ? npix : 0));
-            if ((r = owner_halves(c, ctx, width, 0, height, ntiles, staged, &P))) return r;
-            launch_resolve_adaptive_peers(lc, P, width, npix, c->rgb.p, halves_host ? ad.halves.p : nullptr, spp_host ? ad.spp.p : nullptr);
-            c->launches++;
-            CU(cudaGetLastError());
-            if (halves_host) CU(cudaMemcpyAsync(halves_host, ad.halves.p, 6 * (size_t)npix * sizeof(float), cudaMemcpyDeviceToHost, st_i));
-            if (spp_host) CU(cudaMemcpyAsync(spp_host, ad.spp.p, (size_t)npix * sizeof(uint32_t), cudaMemcpyDeviceToHost, st_i));
+            // the whole half sums and spp, as adaptive_render gathers them (its image is overwritten by the filter's)
+            if ((r = gather_adaptive(c, ctx, nullptr, halves_host, spp_host, staged))) return r;
         }
         const uint32_t t0 = (uint32_t)((uint64_t)i * tile_rows / ndev), t1 = (uint32_t)((uint64_t)(i + 1) * tile_rows / ndev);
         if (t0 < t1) {
@@ -1948,6 +1896,32 @@ int rtc_render_denoised_multi(rtc_scene* s, const int* devices, int ndev, uint32
     CU(cudaSetDevice(s->device));
     if (stats) std::memcpy(stats, st, sizeof st);
     return RTC_OK;
+}
+}  // namespace
+int rtc_render_denoised(rtc_scene* s, uint32_t seed, float tolerance, uint32_t min_samples, uint32_t max_samples, float strength,
+                        uint8_t* rgb_host, float* mean_host, uint64_t stats[4]) {
+    if (!s) return fail(RTC_ERR_ARG, "null scene");
+    int rc = check_strength(strength);
+    if (rc) return rc;
+    if ((rc = check_adaptive_args(tolerance, min_samples))) return rc;
+    const uint32_t smax = max_samples ? max_samples : s->host.samples;
+    if (s->host.dialect > DIALECT_HW2 && smax < 2) return fail(RTC_ERR_ARG, "the maximum sample count must be at least 2");
+    if ((rc = need_device(s))) return rc;
+    return denoised_render(s, &s->device, 1, seed, tolerance, min_samples, max_samples, strength, rgb_host, mean_host, nullptr,
+                           nullptr, stats);
+}
+int rtc_render_denoised_multi(rtc_scene* s, const int* devices, int ndev, uint32_t seed, float tolerance, uint32_t min_samples,
+                              uint32_t max_samples, float strength, uint8_t* rgb_host, float* mean_host, float* halves_host,
+                              uint32_t* spp_host, uint64_t stats[4]) {
+    if (!s) return fail(RTC_ERR_ARG, "null scene");
+    int rc = check_strength(strength);
+    if (rc) return rc;
+    if ((rc = check_adaptive_multi_args(tolerance, min_samples, devices, ndev))) return rc;
+    const uint32_t smax = max_samples ? max_samples : s->host.samples;
+    if (s->host.dialect > DIALECT_HW2 && smax < 2) return fail(RTC_ERR_ARG, "the maximum sample count must be at least 2");
+    if ((rc = need_device(s))) return rc;
+    return denoised_render(s, devices, ndev, seed, tolerance, min_samples, max_samples, strength, rgb_host, mean_host, halves_host,
+                           spp_host, stats);
 }
 
 int rtc_set_profiling(rtc_scene* s, int kernel_events, int count_visits) {

@@ -791,15 +791,9 @@ RT_D void resolve_adaptive_pixel(uint32_t i, float4 a, float4 b, uint32_t n, uin
     }
     if (spp) spp[i] = n;
 }
-// The image of an adaptive render: pixel i took tile_n[its tile] samples, A / B hold its even / odd sums
-__global__ void __launch_bounds__(256) k_resolve_adaptive(const float4* A, const float4* B, const uint32_t* tile_n, uint32_t width,
-                                                           uint32_t npix, uint8_t* out, float* halves, uint32_t* spp) {
-    const uint32_t tiles_x = (width + kAdaptiveTile - 1) / kAdaptiveTile;
-    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < npix; i += gridDim.x * blockDim.x)
-        resolve_adaptive_pixel(i, A[i], B[i], tile_n[tile_of(i, width, tiles_x)], out, halves, spp);
-}
-// The same for a multi-device adaptive render, on the first device: tile t was rendered by device t % P.n, whose
-// half sums and tile counts are read where they lie (peer pointers over NVLink, or copies on this device)
+// The image of an adaptive render, on the first listed device: tile t was rendered by device t % P.n (one device: P.n =
+// 1), whose half sums and tile counts are read where they lie (its own memory, peer pointers over NVLink, or copies on
+// this device)
 __global__ void __launch_bounds__(256) k_resolve_adaptive_peers(PeerHalves P, uint32_t width, uint32_t npix, uint8_t* out,
                                                                  float* halves, uint32_t* spp) {
     const uint32_t tiles_x = (width + kAdaptiveTile - 1) / kAdaptiveTile;
@@ -1090,10 +1084,6 @@ void launch_adaptive_tiles(const LaunchCtx& c, const float4* A, const float4* B,
     k_adaptive_tiles<<<grid_for((uint64_t)ntiles * 32, 128, c.sms, 16), 128, 0, c.stream>>>(A, B, width, height, tiles_in, ntiles, n, inv_a,
                                                                                           inv_b, tau, mode, tile_n, tiles_out,
                                                                                           pixels_out, counts_out, shard, nshards);
-}
-void launch_resolve_adaptive(const LaunchCtx& c, const float4* A, const float4* B, const uint32_t* tile_n, uint32_t width, uint32_t npix,
-                             uint8_t* out, float* halves, uint32_t* spp) {
-    k_resolve_adaptive<<<grid_for(npix, 256, c.sms, 8), 256, 0, c.stream>>>(A, B, tile_n, width, npix, out, halves, spp);
 }
 void launch_resolve_adaptive_peers(const LaunchCtx& c, const PeerHalves& P, uint32_t width, uint32_t npix, uint8_t* out, float* halves,
                                    uint32_t* spp) {

@@ -45,9 +45,6 @@ void launch_adaptive_tiles(const LaunchCtx& c, const float4* A, const float4* B,
                            const uint32_t* tiles_in, uint32_t ntiles, uint32_t n, float inv_a, float inv_b, float tau, int mode,
                            uint32_t* tile_n, uint32_t* tiles_out, uint32_t* pixels_out, uint32_t* counts_out, uint32_t shard,
                            uint32_t nshards);
-// u8 image (and optionally the half sums, 6 floats per pixel, and the samples per pixel) from the even / odd sums
-void launch_resolve_adaptive(const LaunchCtx& c, const float4* A, const float4* B, const uint32_t* tile_n, uint32_t width, uint32_t npix,
-                             uint8_t* out, float* halves, uint32_t* spp);
 // denoising (rtc_denoise, rtc_render_denoised; DESIGN.md "Denoising"): the fixed constants of the non-local-means rule
 // -- search window (2R+1)^2, patch (2F+1)^2, box (2S+1)^2 that smooths the variance estimate, variance cancellation
 // alpha, epsilon -- and the output tile of one block
@@ -95,8 +92,9 @@ struct PeerAccums {
     int n;
 };
 void launch_resolve_peers(const LaunchCtx& c, const PeerAccums& A, float inv_samples, uint32_t nvalues, uint8_t* out, float* sum);
-// per-device half sums and tile counts of one multi-device adaptive render (tile t belongs to device t % n; pointers
-// valid on the device that launches), resolved as launch_resolve_adaptive does
+// per-device half sums and tile counts of one adaptive render (tile t belongs to device t % n; pointers valid on the
+// device that launches), resolved into the u8 image and optionally the half sums (6 floats per pixel) and the samples
+// per pixel
 struct PeerHalves {
     const float4* a[kMaxPeers];
     const float4* b[kMaxPeers];
