@@ -155,7 +155,7 @@ struct rtc_scene {
         DevBuf<float4> ray[2];
         DevBuf<uint32_t> hit, tq, q;
     } probe;
-    // per-device replicas for rtc_render_u8_multi (this scene's own device is not among them)
+    // per-device replicas for the multi-device calls (this scene's own device is not among them)
     std::vector<std::unique_ptr<rtc_scene>> replicas;
     Stream multi_stream;
     Event multi_done;
@@ -722,7 +722,12 @@ Camera camera_of(const HostScene& h, const float* c) {
     cam.fov_x = c[12];
     return cam;
 }
-double camera_extent(const float* c) { return std::max({std::fabs((double)c[0]), std::fabs((double)c[1]), std::fabs((double)c[2])}); }
+// the largest |position|inf of n cameras
+double camera_extent(const float* c, uint32_t n = 1) {
+    double e = 0;
+    for (uint32_t v = 0; v < n; ++v, c += RTC_CAMERA_FLOATS) e = std::max({e, std::fabs((double)c[0]), std::fabs((double)c[1]), std::fabs((double)c[2])});
+    return e;
+}
 // A new layout of the arena of `s` on its device, uploaded synchronously: after the host scene's index BVH was rebuilt.
 // Everything that may still read the pinned mirror or the arenas -- asynchronous uploads, frames in flight, renders on
 // any stream -- is waited for first.
@@ -771,6 +776,94 @@ int check_views(const rtc_scene* s, const float* cams, int nviews) {
         int rc = check_camera(cams + (size_t)RTC_CAMERA_FLOATS * v);
         if (rc) return fail(rc, "view " + std::to_string(v) + ": " + g_error);
     }
+    return RTC_OK;
+}
+
+// The body of rtc_render_accumulate and rtc_render_views_accumulate, their checks passed: adds the samples
+// [sample_begin, sample_begin + sample_count) into accum_dev, asynchronously on `user`.  cams_host null: the scene's
+// camera, one frame, camera rays from the candidate lists.  Else nviews cameras (13 floats each), view v's sums at
+// accum_dev + 3 v npix.
+// The views share the wavefront batches: path p is pixel p % npix of view (p / npix) % V, sample sample_begin +
+// p / (npix V), with view v's camera record in a small device array (k_generate) and its sums at view v's slice of one
+// float4 buffer of V npix pixels (k_shade deposits by the frame-wide pixel word, k_fold folds it).  The Philox streams
+// are those of a render of view v alone: k_shade keys them by the pixel within the view.
+int accumulate(rtc_scene* s, const float* cams_host, uint32_t nviews, uint32_t seed, uint32_t sample_begin, uint32_t sample_count,
+               float* accum_dev, cudaStream_t user) {
+    int rc;
+    const uint32_t V = nviews;
+    const uint64_t npix = (uint64_t)s->host.cam.width * s->host.cam.height;
+    std::vector<DevCamera> cams(cams_host ? V : 0);
+    for (uint32_t v = 0; v < cams.size(); ++v) cams[v] = dev_camera(camera_of(s->host, cams_host + (size_t)RTC_CAMERA_FLOATS * v));
+    DevScene S;
+    if (s->host.dialect <= DIALECT_HW2) {
+        // hw1 / hw2: ONE deterministic frame = sample 0.  A range that holds sample 0 adds the colour once, any
+        // other range adds nothing, so that sample ranges split over several devices still sum to one frame.  The frame
+        // kernel runs once per view, with that view's camera, into that view's slice.
+        if (sample_begin > 0) return RTC_OK;
+        if ((rc = arena_begin(s, user, &S))) return rc;
+        LaunchCtx c{user, s->sms};
+        for (uint32_t v = 0; v < V; ++v) {
+            if (cams_host) S.cam = cams[v];
+            float* slice = accum_dev + 3 * (size_t)v * npix;
+            if (s->host.dialect == DIALECT_HW1) launch_raycast_hw1(c, S, slice);
+            else launch_whitted_hw2(c, S, slice);
+            s->launches++;
+        }
+        if ((rc = arena_end(s, user))) return rc;
+        CU(cudaGetLastError());
+        return RTC_OK;
+    }
+    // the float4 pixel sums of this render: two buffers used alternately, so that two renders may be in flight on
+    // two streams; a third waits for the first to have been folded
+    const uint64_t nsum = V * npix;
+    const int a4 = s->accum4_next;
+    s->accum4_next ^= 1;
+    DevBuf<float4>& accum4 = s->accum4[a4];
+    CU(accum4.ensure(nsum));
+    PathMap map{nullptr, (uint32_t)npix, sample_begin};
+    if (cams_host) {
+        CU(s->views[a4].ensure(V));
+        map.views = s->views[a4].p;
+        map.nviews = V;
+        map.view_recip = V > 1 ? UINT64_MAX / npix : 0;
+    }
+    CU(cudaStreamWaitEvent(user, s->accum4_idle[a4], 0));
+    if (cams_host) CU(cudaMemcpyAsync(s->views[a4].p, cams.data(), V * sizeof(DevCamera), cudaMemcpyHostToDevice, user));
+    CU(cudaMemsetAsync(accum4.p, 0, nsum * sizeof(float4), user));
+    if ((rc = arena_begin(s, user, &S))) return rc;
+    if (!cams_host && (rc = build_camera_lists(s, S, s->cand[a4], user, &map.cand))) return rc;
+    if ((rc = fork_lanes(s, user))) return rc;
+    unsigned used = 0;
+    if ((rc = render_paths(s, S, seed, map, nsum * sample_count, accum4.p, &used))) return rc;
+    if ((rc = join_lanes(s, used, user))) return rc;
+    launch_fold(LaunchCtx{user, s->sms}, accum4.p, accum_dev, (uint32_t)nsum);
+    s->launches++;
+    CU(cudaEventRecord(s->accum4_idle[a4], user));
+    if ((rc = arena_end(s, user))) return rc;
+    CU(cudaGetLastError());
+    return RTC_OK;
+}
+// The 8-bit image of `samples` samples whose sums are A's entries (summed in entry order), on `st` of context c (its
+// device current); sum_dev (optional) receives the float total and may be A.p[0] itself.  hw1 writes colours as they
+// are: only the entry that holds sample 0 has any, and sum_dev is left alone (A.p[0] is the total).
+int resolve_sums(rtc_scene* c, const PeerAccums& A, uint32_t samples, size_t nvalues, uint8_t* rgb_dev, float* sum_dev, cudaStream_t st) {
+    const LaunchCtx lc{st, c->sms};
+    const float inv = 1.f / (float)samples;   // 1.f / samples * sum, src/scene.cpp:201
+    if (c->host.dialect == DIALECT_HW1) launch_resolve_flat(lc, A.p[0], inv, (uint32_t)nvalues, rgb_dev);
+    else launch_resolve_peers(lc, A, inv, (uint32_t)nvalues, rgb_dev, sum_dev);
+    c->launches++;
+    CU(cudaGetLastError());
+    return RTC_OK;
+}
+// words [first, first + n) of the scene's counters, once the work on `stream` and on the lanes is done
+int read_stats(rtc_scene* s, void* stream, int first, int n, uint64_t* out) {
+    static_assert(sizeof(uint64_t) == sizeof(unsigned long long), "rtc_scene::stats");
+    int rc = need_device(s);
+    if (rc) return rc;
+    if (!out) return fail(RTC_ERR_ARG, "null argument");
+    CU(cudaStreamSynchronize((cudaStream_t)stream));
+    CU(sync_lanes(s));
+    CU(cudaMemcpy(out, s->stats.p + first, n * sizeof(uint64_t), cudaMemcpyDeviceToHost));
     return RTC_OK;
 }
 
@@ -1069,77 +1162,16 @@ int rtc_render_accumulate(rtc_scene* s, uint32_t seed, uint32_t sample_begin, ui
     const uint64_t total = npix * sample_count;
     if (total == 0) return RTC_OK;   // an empty frame (no DIMENSIONS) or an empty sample range: nothing to add
     if (!accum_dev) return fail(RTC_ERR_ARG, "null accumulation buffer");
-    cudaStream_t user = (cudaStream_t)stream;
-    DevScene S;
-    if (s->host.dialect <= DIALECT_HW2) {
-        // hw1 / hw2: ONE deterministic frame = sample 0.  A range that holds sample 0 adds the colour once, any
-        // other range adds nothing, so that sample ranges split over several devices still sum to one frame.
-        if (sample_begin > 0) return RTC_OK;
-        if ((rc = arena_begin(s, user, &S))) return rc;
-        LaunchCtx c{user, s->sms};
-        if (s->host.dialect == DIALECT_HW1) launch_raycast_hw1(c, S, accum_dev);
-        else launch_whitted_hw2(c, S, accum_dev);
-        s->launches++;
-        if ((rc = arena_end(s, user))) return rc;
-        CU(cudaGetLastError());
-        return RTC_OK;
-    }
-    // the float4 pixel sums of this render: two buffers used alternately, so that two renders may be in flight on
-    // two streams; a third waits for the first to have been folded
-    const int a4 = s->accum4_next;
-    s->accum4_next ^= 1;
-    DevBuf<float4>& accum4 = s->accum4[a4];
-    CU(accum4.ensure(npix));
-    CU(cudaStreamWaitEvent(user, s->accum4_idle[a4], 0));
-    CU(cudaMemsetAsync(accum4.p, 0, npix * sizeof(float4), user));
-    if ((rc = arena_begin(s, user, &S))) return rc;
-    PathMap map{nullptr, (uint32_t)npix, sample_begin};
-    if ((rc = build_camera_lists(s, S, s->cand[a4], user, &map.cand))) return rc;
-    if ((rc = fork_lanes(s, user))) return rc;
-    unsigned used = 0;
-    if ((rc = render_paths(s, S, seed, map, total, accum4.p, &used))) return rc;
-    if ((rc = join_lanes(s, used, user))) return rc;
-    launch_fold(LaunchCtx{user, s->sms}, accum4.p, accum_dev, (uint32_t)npix);
-    s->launches++;
-    CU(cudaEventRecord(s->accum4_idle[a4], user));
-    if ((rc = arena_end(s, user))) return rc;
-    CU(cudaGetLastError());
-    return RTC_OK;
+    return accumulate(s, nullptr, 1, seed, sample_begin, sample_count, accum_dev, (cudaStream_t)stream);
 }
 int rtc_render_counters(rtc_scene* s, void* stream, uint64_t out[8]) {
-    int rc = need_device(s);
+    int rc = read_stats(s, stream, 0, 8, out);
     if (rc) return rc;
-    if (!out) return fail(RTC_ERR_ARG, "null argument");
-    CU(cudaStreamSynchronize((cudaStream_t)stream));
-    CU(sync_lanes(s));
-    unsigned long long h[8];
-    CU(cudaMemcpy(h, s->stats.p, sizeof h, cudaMemcpyDeviceToHost));
-    for (int i = 0; i < 8; ++i) out[i] = h[i];
     out[2] = s->launches;
     return RTC_OK;
 }
-int rtc_traverse_lanes(rtc_scene* s, void* stream, uint64_t out[8]) {
-    int rc = need_device(s);
-    if (rc) return rc;
-    if (!out) return fail(RTC_ERR_ARG, "null argument");
-    CU(cudaStreamSynchronize((cudaStream_t)stream));
-    CU(sync_lanes(s));
-    unsigned long long h[8];
-    CU(cudaMemcpy(h, s->stats.p + 8, sizeof h, cudaMemcpyDeviceToHost));
-    for (int i = 0; i < 8; ++i) out[i] = h[i];
-    return RTC_OK;
-}
-int rtc_camera_list_rays(rtc_scene* s, void* stream, uint64_t* out) {
-    int rc = need_device(s);
-    if (rc) return rc;
-    if (!out) return fail(RTC_ERR_ARG, "null argument");
-    CU(cudaStreamSynchronize((cudaStream_t)stream));
-    CU(sync_lanes(s));
-    unsigned long long h;
-    CU(cudaMemcpy(&h, s->stats.p + kStatListRays, sizeof h, cudaMemcpyDeviceToHost));
-    *out = h;
-    return RTC_OK;
-}
+int rtc_traverse_lanes(rtc_scene* s, void* stream, uint64_t out[8]) { return read_stats(s, stream, 8, 8, out); }
+int rtc_camera_list_rays(rtc_scene* s, void* stream, uint64_t* out) { return read_stats(s, stream, kStatListRays, 1, out); }
 int rtc_camera_list_lengths(rtc_scene* s, uint32_t* lengths_host) {
     int rc = need_device(s);
     if (rc) return rc;
@@ -1168,13 +1200,8 @@ int rtc_render_resolve(rtc_scene* s, const float* accum_dev, uint32_t total_samp
     int rc = need_device(s);
     if (rc) return rc;
     if (!accum_dev || !rgb_dev || total_samples == 0) return fail(RTC_ERR_ARG, "bad argument");
-    LaunchCtx c{(cudaStream_t)stream, s->sms};
-    uint32_t nvalues = 3u * s->host.cam.width * s->host.cam.height;
-    if (s->host.dialect == DIALECT_HW1) launch_resolve_flat(c, accum_dev, 1.f / (float)total_samples, nvalues, rgb_dev);
-    else launch_resolve(c, accum_dev, 1.f / (float)total_samples, nvalues, rgb_dev);  // 1.f / samples * sum, src/scene.cpp:201
-    s->launches++;
-    CU(cudaGetLastError());
-    return RTC_OK;
+    const PeerAccums A{{accum_dev}, 1};
+    return resolve_sums(s, A, total_samples, 3 * (size_t)s->host.cam.width * s->host.cam.height, rgb_dev, nullptr, (cudaStream_t)stream);
 }
 int rtc_render_sum(rtc_scene* s, uint32_t seed, uint32_t sample_begin, uint32_t sample_count, float* sum_host) {
     int rc = need_device(s);
@@ -1188,109 +1215,17 @@ int rtc_render_sum(rtc_scene* s, uint32_t seed, uint32_t sample_begin, uint32_t 
     CU(cudaMemcpy(sum_host, s->accum.p, nvalues * sizeof(float), cudaMemcpyDeviceToHost));
     return RTC_OK;
 }
-int rtc_render_u8(rtc_scene* s, uint32_t seed, uint8_t* rgb_host) {
-    int rc = need_device(s);
-    if (rc) return rc;
-    if (!rgb_host) return fail(RTC_ERR_ARG, "null argument");
-    uint32_t samples;
-    if ((rc = frame_samples(s, &samples))) return rc;
-    size_t nvalues = 3 * (size_t)s->host.cam.width * s->host.cam.height;
-    if (nvalues == 0) return RTC_OK;   // no DIMENSIONS: the reference writes a PPM header and no pixels
-    CU(s->accum.ensure(nvalues));
-    CU(s->rgb.ensure(nvalues));
-    if ((rc = render_frame(s, seed, samples, s->accum.p, s->rgb.p, nullptr))) return rc;
-    CU(cudaMemcpy(rgb_host, s->rgb.p, nvalues, cudaMemcpyDeviceToHost));
-    return RTC_OK;
-}
-int rtc_render_ppm(rtc_scene* s, uint32_t seed, const char* out_path) {
-    if (!s || !out_path) return fail(RTC_ERR_ARG, "null argument");
-    std::vector<uint8_t> img(3 * (size_t)s->host.cam.width * s->host.cam.height);
-    int rc = rtc_render_u8(s, seed, img.data());
-    return rc ? rc : write_ppm(out_path, s->host.cam.width, s->host.cam.height, img);
-}
-
 // ------------------------------------------------------------------ batched views
-// The views share the wavefront batches: path p is pixel p % npix of view (p / npix) % V, sample sample_begin +
-// p / (npix V), with view v's camera record in a small device array (k_generate) and its sums at view v's slice of one
-// float4 buffer of V npix pixels (k_shade deposits by the frame-wide pixel word, k_fold folds it).  The Philox streams
-// are those of a render of view v alone: k_shade keys them by the pixel within the view.
 int rtc_render_views_accumulate(rtc_scene* s, const float* cams_host, int nviews, uint32_t seed, uint32_t sample_begin,
                                 uint32_t sample_count, float* accum_dev, void* stream) {
     int rc = check_views(s, cams_host, nviews);
     if (rc) return rc;
     if ((rc = need_device(s))) return rc;
-    const uint32_t V = (uint32_t)nviews;
-    const uint64_t npix = (uint64_t)s->host.cam.width * s->host.cam.height;
-    const uint64_t total = (uint64_t)V * npix * sample_count;
+    const uint64_t total = (uint64_t)nviews * s->host.cam.width * s->host.cam.height * sample_count;
     if (total == 0) return RTC_OK;
     if (!accum_dev) return fail(RTC_ERR_ARG, "null accumulation buffer");
-    double extent = 0;
-    for (uint32_t v = 0; v < V; ++v) extent = std::max(extent, camera_extent(cams_host + (size_t)RTC_CAMERA_FLOATS * v));
-    if ((rc = ensure_index_extent(s, extent))) return rc;
-    std::vector<DevCamera> cams(V);
-    for (uint32_t v = 0; v < V; ++v) cams[v] = dev_camera(camera_of(s->host, cams_host + (size_t)RTC_CAMERA_FLOATS * v));
-    cudaStream_t user = (cudaStream_t)stream;
-    DevScene S;
-    if (s->host.dialect <= DIALECT_HW2) {
-        // one deterministic frame per view (sample 0, as rtc_render_accumulate): the frame kernel once per view, with that
-        // view's camera, into that view's slice
-        if (sample_begin > 0) return RTC_OK;
-        if ((rc = arena_begin(s, user, &S))) return rc;
-        LaunchCtx c{user, s->sms};
-        for (uint32_t v = 0; v < V; ++v) {
-            S.cam = cams[v];
-            float* slice = accum_dev + 3 * (size_t)v * npix;
-            if (s->host.dialect == DIALECT_HW1) launch_raycast_hw1(c, S, slice);
-            else launch_whitted_hw2(c, S, slice);
-            s->launches++;
-        }
-        if ((rc = arena_end(s, user))) return rc;
-        CU(cudaGetLastError());
-        return RTC_OK;
-    }
-    const uint64_t nsum = V * npix;
-    const int a4 = s->accum4_next;
-    s->accum4_next ^= 1;
-    DevBuf<float4>& accum4 = s->accum4[a4];
-    CU(accum4.ensure(nsum));
-    CU(s->views[a4].ensure(V));
-    CU(cudaStreamWaitEvent(user, s->accum4_idle[a4], 0));
-    CU(cudaMemcpyAsync(s->views[a4].p, cams.data(), V * sizeof(DevCamera), cudaMemcpyHostToDevice, user));
-    CU(cudaMemsetAsync(accum4.p, 0, nsum * sizeof(float4), user));
-    if ((rc = arena_begin(s, user, &S))) return rc;
-    if ((rc = fork_lanes(s, user))) return rc;
-    unsigned used = 0;
-    PathMap map{nullptr, (uint32_t)npix, sample_begin, s->views[a4].p, V, V > 1 ? UINT64_MAX / npix : 0};
-    if ((rc = render_paths(s, S, seed, map, total, accum4.p, &used))) return rc;
-    if ((rc = join_lanes(s, used, user))) return rc;
-    launch_fold(LaunchCtx{user, s->sms}, accum4.p, accum_dev, (uint32_t)nsum);
-    s->launches++;
-    CU(cudaEventRecord(s->accum4_idle[a4], user));
-    if ((rc = arena_end(s, user))) return rc;
-    CU(cudaGetLastError());
-    return RTC_OK;
-}
-int rtc_render_views_u8(rtc_scene* s, const float* cams_host, int nviews, uint32_t seed, uint8_t* rgb_host, float* sum_host) {
-    int rc = check_views(s, cams_host, nviews);
-    if (rc) return rc;
-    if (!rgb_host) return fail(RTC_ERR_ARG, "null argument");
-    if ((rc = need_device(s))) return rc;
-    uint32_t samples;
-    if ((rc = frame_samples(s, &samples))) return rc;
-    const size_t nvalues = 3 * (size_t)nviews * s->host.cam.width * s->host.cam.height;
-    if (nvalues == 0) return RTC_OK;
-    CU(s->accum.ensure(nvalues));
-    CU(s->rgb.ensure(nvalues));
-    CU(cudaMemsetAsync(s->accum.p, 0, nvalues * sizeof(float), nullptr));
-    if ((rc = rtc_render_views_accumulate(s, cams_host, nviews, seed, 0, samples, s->accum.p, nullptr))) return rc;
-    LaunchCtx c{nullptr, s->sms};
-    if (s->host.dialect == DIALECT_HW1) launch_resolve_flat(c, s->accum.p, 1.f / (float)samples, (uint32_t)nvalues, s->rgb.p);
-    else launch_resolve(c, s->accum.p, 1.f / (float)samples, (uint32_t)nvalues, s->rgb.p);
-    s->launches++;
-    CU(cudaGetLastError());
-    CU(cudaMemcpy(rgb_host, s->rgb.p, nvalues, cudaMemcpyDeviceToHost));
-    if (sum_host) CU(cudaMemcpy(sum_host, s->accum.p, nvalues * sizeof(float), cudaMemcpyDeviceToHost));
-    return RTC_OK;
+    if ((rc = ensure_index_extent(s, camera_extent(cams_host, (uint32_t)nviews)))) return rc;
+    return accumulate(s, cams_host, (uint32_t)nviews, seed, sample_begin, sample_count, accum_dev, (cudaStream_t)stream);
 }
 
 // ------------------------------------------------------------------ adaptive sampling
@@ -1578,24 +1513,22 @@ int device_contexts(rtc_scene* s, const int* devices, int ndev, std::vector<rtc_
     }
     return RTC_OK;
 }
-}  // namespace
-int rtc_render_u8_multi(rtc_scene* s, const int* devices, int ndev, uint32_t seed, uint8_t* rgb_host, float* sum_host) {
-    int rc = need_device(s);
-    if (rc) return rc;
-    if (!devices || ndev < 1 || ndev > kMaxPeers || !rgb_host) return fail(RTC_ERR_ARG, "bad argument");
+// The body of the 8-bit calls, their checks passed: one frame of the scene's SAMPLES on the entries `devices`, into
+// rgb_host and, when it is given, its float sums into sum_host; blocks until both are there.  cams_host null: the
+// scene's camera, else nviews views (their images one after the other).  Every entry renders its share of the samples
+// of every view into its own accum on its multi_stream; the ~30 launches of an entry's share are issued by a host
+// thread of its own (one thread issuing for 8 devices took 1.1 of a 3.9 ms frame).  The head (devices[0]) reads the
+// others' sums in place (peer access) or copies them over, resolves, and writes the total over its own sums.
+int frame_u8(rtc_scene* s, const int* devices, int ndev, const float* cams_host, uint32_t nviews, uint32_t seed, uint8_t* rgb_host,
+             float* sum_host) {
     uint32_t samples;
-    if ((rc = frame_samples(s, &samples))) return rc;
-    const size_t nvalues = 3 * (size_t)s->host.cam.width * s->host.cam.height;
-    if (nvalues == 0) return RTC_OK;
-    // the first listed device reduces: make it this scene's device or a replica there
+    int rc = frame_samples(s, &samples);
+    if (rc) return rc;
+    const size_t nvalues = 3 * (size_t)nviews * s->host.cam.width * s->host.cam.height;
+    if (nvalues == 0) return RTC_OK;   // no DIMENSIONS: the reference writes a PPM header and no pixels
+    if (cams_host && (rc = ensure_index_extent(s, camera_extent(cams_host, nviews)))) return rc;
     std::vector<rtc_scene*> ctx;
     if ((rc = device_contexts(s, devices, ndev, ctx))) return rc;
-    PeerAccums A;
-    std::memset(&A, 0, sizeof A);
-    A.n = ndev;
-    rtc_scene* head = ctx[0];
-    // every device renders its sample range into its own buffer on its own stream; the ~30 launches of a device's
-    // share are issued by a host thread of its own (one thread issuing for 8 devices took 1.1 of a 3.9 ms frame)
     auto issue = [&](int i) -> int {
         rtc_scene* c = ctx[i];
         CU(cudaSetDevice(c->device));
@@ -1604,14 +1537,19 @@ int rtc_render_u8_multi(rtc_scene* s, const int* devices, int ndev, uint32_t see
         CU(c->accum.ensure(nvalues));
         CU(cudaMemsetAsync(c->accum.p, 0, nvalues * sizeof(float), c->multi_stream));
         const uint32_t lo = (uint32_t)((uint64_t)i * samples / ndev), hi = (uint32_t)((uint64_t)(i + 1) * samples / ndev);
-        int r = rtc_render_accumulate(c, seed, lo, hi - lo, c->accum.p, c->multi_stream);
-        if (r) return r;
+        if (hi > lo) {
+            int r = accumulate(c, cams_host, nviews, seed, lo, hi - lo, c->accum.p, c->multi_stream);
+            if (r) return r;
+        }
         CU(cudaEventRecord(c->multi_done, c->multi_stream));
         return RTC_OK;
     };
     if ((rc = fan_out(ndev, issue))) return rc;
+    rtc_scene* head = ctx[0];
+    PeerAccums A;
+    std::memset(&A, 0, sizeof A);
+    A.n = ndev;
     for (int i = 0; i < ndev; ++i) A.p[i] = ctx[i]->accum.p;
-    // the head device reads the others' buffers in place (peer access), or copies them over when it cannot
     CU(cudaSetDevice(head->device));
     std::vector<DevBuf<unsigned char>> staged;
     for (int i = 1; i < ndev; ++i) {
@@ -1625,28 +1563,44 @@ int rtc_render_u8_multi(rtc_scene* s, const int* devices, int ndev, uint32_t see
         A.p[i] = (const float*)p;
     }
     CU(head->rgb.ensure(nvalues));
-    float* sum_dev = nullptr;
-    if (sum_host) { CU(head->frames[1].accum.ensure(nvalues)); sum_dev = head->frames[1].accum.p; }
-    LaunchCtx lc{head->multi_stream, head->sms};
-    if (head->host.dialect == DIALECT_HW1) {
-        // hw1 writes colours as they are: only the device that holds sample 0 has any
-        launch_resolve_flat(lc, A.p[0], 1.f, (uint32_t)nvalues, head->rgb.p);
-        if (sum_dev) CU(cudaMemcpyAsync(sum_dev, A.p[0], nvalues * sizeof(float), cudaMemcpyDeviceToDevice, head->multi_stream));
-    } else launch_resolve_peers(lc, A, 1.f / (float)samples, (uint32_t)nvalues, head->rgb.p, sum_dev);
-    head->launches++;
-    CU(cudaGetLastError());
+    // the total goes over A.p[0] = head->accum, which hw1's already is
+    if ((rc = resolve_sums(head, A, samples, nvalues, head->rgb.p, sum_host ? head->accum.p : nullptr, head->multi_stream))) return rc;
     CU(cudaMemcpyAsync(rgb_host, head->rgb.p, nvalues, cudaMemcpyDeviceToHost, head->multi_stream));
-    if (sum_host) CU(cudaMemcpyAsync(sum_host, sum_dev, nvalues * sizeof(float), cudaMemcpyDeviceToHost, head->multi_stream));
+    if (sum_host) CU(cudaMemcpyAsync(sum_host, head->accum.p, nvalues * sizeof(float), cudaMemcpyDeviceToHost, head->multi_stream));
     CU(cudaStreamSynchronize(head->multi_stream));
     staged.clear();   // while the head device is current
     CU(cudaSetDevice(s->device));
     return RTC_OK;
+}
+}  // namespace
+// The one-device calls are the scene's own device as the only entry: the scene itself, no replica, no thread
+int rtc_render_u8(rtc_scene* s, uint32_t seed, uint8_t* rgb_host) {
+    int rc = need_device(s);
+    if (rc) return rc;
+    if (!rgb_host) return fail(RTC_ERR_ARG, "null argument");
+    return frame_u8(s, &s->device, 1, nullptr, 1, seed, rgb_host, nullptr);
+}
+int rtc_render_views_u8(rtc_scene* s, const float* cams_host, int nviews, uint32_t seed, uint8_t* rgb_host, float* sum_host) {
+    int rc = check_views(s, cams_host, nviews);
+    if (rc) return rc;
+    if (!rgb_host) return fail(RTC_ERR_ARG, "null argument");
+    if ((rc = need_device(s))) return rc;
+    return frame_u8(s, &s->device, 1, cams_host, (uint32_t)nviews, seed, rgb_host, sum_host);
+}
+int rtc_render_u8_multi(rtc_scene* s, const int* devices, int ndev, uint32_t seed, uint8_t* rgb_host, float* sum_host) {
+    int rc = need_device(s);
+    if (rc) return rc;
+    if (!devices || ndev < 1 || ndev > kMaxPeers || !rgb_host) return fail(RTC_ERR_ARG, "bad argument");
+    return frame_u8(s, devices, ndev, nullptr, 1, seed, rgb_host, sum_host);
 }
 int rtc_render_ppm_multi(rtc_scene* s, const int* devices, int ndev, uint32_t seed, const char* out_path) {
     if (!s || !out_path) return fail(RTC_ERR_ARG, "null argument");
     std::vector<uint8_t> img(3 * (size_t)s->host.cam.width * s->host.cam.height);
     int rc = rtc_render_u8_multi(s, devices, ndev, seed, img.data(), nullptr);
     return rc ? rc : write_ppm(out_path, s->host.cam.width, s->host.cam.height, img);
+}
+int rtc_render_ppm(rtc_scene* s, uint32_t seed, const char* out_path) {
+    return rtc_render_ppm_multi(s, s ? &s->device : nullptr, 1, seed, out_path);   // a null scene is refused there
 }
 
 // Adaptive sampling on one or several devices: tile t of the frame belongs to devices[t % ndev], and every device runs

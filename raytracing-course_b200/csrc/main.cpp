@@ -140,8 +140,10 @@ int main(int argc, const char* argv[]) {
             rc = RTC_ERR_IO;
             written_error = true;
         }
-    } else if (devices.size() > 1) rc = rtc_render_ppm_multi(scene, devices.data(), (int)devices.size(), (uint32_t)env_int("RTC_SEED", 0), argv[2]);
-    else rc = rtc_render_ppm(scene, (uint32_t)env_int("RTC_SEED", 0), argv[2]);
+    } else {
+        const std::vector<int> list = devices.empty() ? std::vector<int>{device0} : devices;
+        rc = rtc_render_ppm_multi(scene, list.data(), (int)list.size(), (uint32_t)env_int("RTC_SEED", 0), argv[2]);
+    }
     if (rc != RTC_OK && !written_error) std::fprintf(stderr, "raytracing_hw5: %s\n", rtc_last_error());
     const auto t_rendered = now();
     if (timing)

@@ -698,13 +698,10 @@ __global__ void __launch_bounds__(256) k_fold(const float4* accum4, float* accum
         accum[3 * (size_t)i + 2] += v.z;
     }
 }
-__global__ void __launch_bounds__(256) k_resolve(const float* accum, float inv_samples, uint32_t nvalues, uint8_t* out) {
-    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < nvalues; i += gridDim.x * blockDim.x)
-        out[i] = to_u8(aces(__fmul_rn(inv_samples, accum[i])));
-}
-// Multi-device Scene::Render, last step on the first device: the per-device pixel sums (each device rendered its share
-// of the samples) are read where they lie -- peer pointers over NVLink -- summed in device order, and resolved to
-// 8 bits in the same pass (src/scene.cpp:201, 227-228, 247); `sum` (optional) keeps the float total.
+// Scene::Render, last step on the first device: the per-device pixel sums (each device rendered its share of the
+// samples; one device is the case n = 1) are read where they lie -- peer pointers over NVLink -- summed in device order,
+// and resolved to 8 bits in the same pass (src/scene.cpp:201, 227-228, 247); `sum` (optional) keeps the float total.
+// `sum` may be A.p[0]: element i is read and written by one thread only, which reads every entry's value i first.
 __global__ void __launch_bounds__(256) k_resolve_peers(PeerAccums A, float inv_samples, uint32_t nvalues, uint8_t* out, float* sum) {
     for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < nvalues; i += gridDim.x * blockDim.x) {
         float v = A.p[0][i];
@@ -779,7 +776,7 @@ RT_D uint32_t tile_of(uint32_t i, uint32_t width, uint32_t tiles_x) {
     return (i / width / kAdaptiveTile) * tiles_x + (i % width) / kAdaptiveTile;
 }
 // Pixel i of an adaptive image: it took n samples, a / b are its even / odd sums; out = to_u8(aces(1/n * (a + b)))
-// (k_resolve's expression); optionally halves (a.rgb, b.rgb per pixel) and spp (n).
+// (k_resolve_peers' expression); optionally halves (a.rgb, b.rgb per pixel) and spp (n).
 RT_D void resolve_adaptive_pixel(uint32_t i, float4 a, float4 b, uint32_t n, uint8_t* out, float* halves, uint32_t* spp) {
     const float inv = __fdiv_rn(1.f, (float)n);
     out[3 * (size_t)i + 0] = to_u8(aces(__fmul_rn(inv, __fadd_rn(a.x, b.x))));
@@ -1175,9 +1172,6 @@ void launch_tally(const LaunchCtx& c, const uint32_t* q, const uint32_t* tqc, ui
 }
 void launch_fold(const LaunchCtx& c, const float4* accum4, float* accum, uint32_t npix) {
     k_fold<<<grid_for(npix, 256, c.sms, 8), 256, 0, c.stream>>>(accum4, accum, npix);
-}
-void launch_resolve(const LaunchCtx& c, const float* accum, float inv_samples, uint32_t nvalues, uint8_t* out) {
-    k_resolve<<<grid_for(nvalues, 256, c.sms, 8), 256, 0, c.stream>>>(accum, inv_samples, nvalues, out);
 }
 void launch_resolve_peers(const LaunchCtx& c, const PeerAccums& A, float inv_samples, uint32_t nvalues, uint8_t* out, float* sum) {
     k_resolve_peers<<<grid_for(nvalues, 256, c.sms, 8), 256, 0, c.stream>>>(A, inv_samples, nvalues, out, sum);

@@ -82,10 +82,9 @@ void launch_expand_boxes(const LaunchCtx& c, const float4* sparse, uint32_t n, f
 void launch_fill_identity_rotations(const LaunchCtx& c, float4* rot, uint32_t n);
 void launch_expand_palette(const LaunchCtx& c, const float4* palette, const uint16_t* index, uint32_t n, float4* out0, float4* out1);
 void launch_tally(const LaunchCtx& c, const uint32_t* q, const uint32_t* tqc, uint32_t ray_depth, unsigned long long* stats);
-void launch_resolve(const LaunchCtx& c, const float* accum, float inv_samples, uint32_t nvalues, uint8_t* out);
 void launch_tonemap(const LaunchCtx& c, const float* rgb, uint32_t nvalues, uint8_t* out);
-// per-device accumulation buffers of one multi-device frame (device pointers valid on the device that launches:
-// its own memory or peer-mapped memory), summed in order and resolved to 8 bits
+// per-device accumulation buffers of one frame (device pointers valid on the device that launches: its own memory or
+// peer-mapped memory), summed in order and resolved to 8 bits; sum (optional) gets the total and may be p[0]
 constexpr int kMaxPeers = 16;
 struct PeerAccums {
     const float* p[kMaxPeers];
