@@ -82,6 +82,21 @@ int rtc_scene_override(rtc_scene* s, int width, int height, int samples, int ray
 #define RTC_CAMERA_FLOATS 13
 int rtc_scene_camera(const rtc_scene* s, float out[13]);
 int rtc_scene_set_camera(rtc_scene* s, const float cam[13]);
+/* ---- thin lens (depth of field, DESIGN.md "Thin lens"): aperture radius r >= 0 in world units, focus distance f > 0.
+ *      The camera sample of (pixel, sample) keeps its jitter and Camera::GetToRay's origin pos and direction
+ *      d = forward + nx right + ny up; the lens point (lx, ly) is the concentric (Shirley-Chiu) map of u01(.z), u01(.w) of
+ *      the Philox block whose .x, .y give the jitter (no extra random numbers: the pinhole streams stay as they are).
+ *      With e = lx right + ly up the ray starts at pos + r e and runs along d - (r / f) e: every ray of the sample passes
+ *      through pos + f d, the plane at distance f in front of the camera for orthonormal axes, and d's forward
+ *      coefficient stays 1 (t keeps its units).  The lens is scene state like the camera: rtc_scene_set_camera keeps it,
+ *      every render path and every view of a batched render uses it (with that view's axes); r = 0 (the default, f = 1)
+ *      is the pinhole.  rtc_camera_rays stays the pinhole Camera::GetToRay.  Works on host-only scenes too.
+ *      rtc_scene_set_lens, before any change: RTC_ERR_ARG for a null scene, a value that is not finite, r < 0 or f <= 0;
+ *      RTC_ERR_UNSUPPORTED for r > 0 on hw1 / hw2 (one deterministic frame, no samples to spread over a lens).  Lens
+ *      origins reach r (|right|inf + |up|inf) beyond the position: set_lens, set_camera and the views rebuild the index
+ *      BVH when that passes its extent, as for a far camera.  out: r, f. */
+int rtc_scene_set_lens(rtc_scene* s, float aperture_radius, float focus_distance);
+int rtc_scene_lens(const rtc_scene* s, float out[2]);
 /* final primitive order after std::partition + the BVH sorts (scene.cpp:17, bvh.cpp:129,168):
  * original file index of every slot; and the per-primitive record type,material + 26 floats
  * (col3 emission3 pos3 rot4(xyzw) ior d0(3) d1(3) d2(3) pad3) */
@@ -138,10 +153,10 @@ int rtc_render_reset_counters(rtc_scene* s);
 int rtc_traverse_lanes(rtc_scene* s, void* stream, uint64_t out[8]);
 /* Camera rays of rtc_render_accumulate and the adaptive renders are resolved from per-pixel lists of candidate index
  * leaves (one beam traversal per pixel per call) instead of the index traversal, except in pixels whose list would be
- * too long.  out[0]: such camera rays since the scene was created or rtc_render_reset_counters. */
+ * too long, and except with a thin lens (rtc_scene_set_lens), whose renders build no lists.  out[0]: such camera rays since the scene was created or rtc_render_reset_counters. */
 int rtc_camera_list_rays(rtc_scene* s, void* stream, uint64_t* out);
 /* The list length of every pixel (width * height, row-major) for the scene's camera as it stands, 0xFFFFFFFF for a pixel
- * whose rays take the index traversal; synchronous. */
+ * whose rays take the index traversal (every pixel with a lens); synchronous. */
 int rtc_camera_list_lengths(rtc_scene* s, uint32_t* lengths_host);
 /* mean = 1/total_samples * sum ; tonemap ; gamma ; u8 -> rgb_dev (3 bytes per pixel, device) */
 int rtc_render_resolve(rtc_scene* s, const float* accum_dev, uint32_t total_samples, uint8_t* rgb_dev, void* stream);

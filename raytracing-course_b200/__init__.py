@@ -47,6 +47,8 @@ _SIGNATURES = {
     "rtc_scene_override": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int]),
     "rtc_scene_camera": (C.c_int, [C.c_void_p, _f32]),
     "rtc_scene_set_camera": (C.c_int, [C.c_void_p, _f32]),
+    "rtc_scene_set_lens": (C.c_int, [C.c_void_p, C.c_float, C.c_float]),
+    "rtc_scene_lens": (C.c_int, [C.c_void_p, _f32]),
     "rtc_scene_prim_order": (C.c_int, [C.c_void_p, _i32]),
     "rtc_scene_prims": (C.c_int, [C.c_void_p, _i32, _f32]),
     "rtc_scene_nodes": (C.c_int, [C.c_void_p, _f32, _u32]),
@@ -272,6 +274,18 @@ class Scene:
         """Render from another camera (rtc_scene_set_camera): 13 floats, or pos / right / up / forward and fov_x.  The
         frame size stays; a camera beyond the index BVH's extent rebuilds it."""
         _check(self.lib, self.lib.rtc_scene_set_camera(self.h, _camera_floats(pos, right, up, forward, fov_x, cam)))
+
+    def set_lens(self, aperture_radius, focus_distance):
+        """Depth of field (rtc_scene_set_lens): a thin lens of aperture radius r >= 0 (world units; 0 = pinhole) focused at
+        distance f > 0 along the camera's forward axis.  Every later render of the scene, its views included, goes through
+        it; set_camera keeps it.  r > 0 on hw1 / hw2 scenes raises (they render one deterministic frame)."""
+        _check(self.lib, self.lib.rtc_scene_set_lens(self.h, float(aperture_radius), float(focus_distance)))
+
+    def lens(self):
+        """(aperture_radius, focus_distance) the scene renders with; (0, 1) until set_lens."""
+        out = np.zeros(2, np.float32)
+        _check(self.lib, self.lib.rtc_scene_lens(self.h, out))
+        return float(out[0]), float(out[1])
 
     def prim_order(self):
         out = np.zeros(self.nprims, np.int32)

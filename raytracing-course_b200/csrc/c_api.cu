@@ -627,10 +627,11 @@ int join_lanes(rtc_scene* s, unsigned used, cudaStream_t user) {
 }
 // The candidate leaves of the camera rays of every pixel of the scene's camera into `buf` (kCandWords words per pixel), on
 // `st` after arena_begin: returns the lists for PathMap::cand, or null when the render does not use them (the
-// reference-tree traversal).  Built on every render call: the arena, the camera or the frame size may have changed since.
+// reference-tree traversal; a thin lens, whose rays do not share an origin: DESIGN.md "Thin lens").  Built on every render
+// call: the arena, the camera or the frame size may have changed since.
 int build_camera_lists(rtc_scene* s, const DevScene& S, DevBuf<uint32_t>& buf, cudaStream_t st, const uint32_t** cand) {
     *cand = nullptr;
-    if (s->traversal == RTC_TRAVERSAL_REFTREE) return RTC_OK;
+    if (s->traversal == RTC_TRAVERSAL_REFTREE || s->host.lens_r > 0.f) return RTC_OK;
     const size_t npix = (size_t)S.width * S.height;
     CU(buf.ensure(kCandWords * npix));
     s->span_begin(3, st);
@@ -680,9 +681,9 @@ int render_paths(rtc_scene* s, const DevScene& S, uint32_t seed, const PathMap& 
         HitSoA hcur{L.hit_id[0].p}, hnxt{L.hit_id[1].p};
         s->span_begin(0, st);
         if (map.plist) launch_generate_list(c, S, cur, hcur, L.queue.p, L.trav_queue.p, tqc, first, count, seed, map.plist, map.npix, map.sample_first,
-                                            map.cand, s->stats.p);
+                                            map.cand, s->stats.p, dev_lens(s->host));
         else launch_generate(c, S, cur, hcur, L.queue.p, L.trav_queue.p, tqc, first, count, seed, map.sample_first, map.views, map.nviews,
-                             map.cand, s->stats.p);
+                             map.cand, s->stats.p, dev_lens(s->host));
         s->span_end(st);
         s->launches++;
         for (uint32_t b = 1; b <= depth; ++b) {
@@ -722,10 +723,15 @@ Camera camera_of(const HostScene& h, const float* c) {
     cam.fov_x = c[12];
     return cam;
 }
-// the largest |position|inf of n cameras
-double camera_extent(const float* c, uint32_t n = 1) {
+// the largest |ray origin|inf of n cameras with a thin lens of aperture radius lens_r: the lens origins lie up to
+// lens_r (|right|inf + |up|inf) beyond the position
+double camera_extent(const float* c, uint32_t n, float lens_r) {
     double e = 0;
-    for (uint32_t v = 0; v < n; ++v, c += RTC_CAMERA_FLOATS) e = std::max({e, std::fabs((double)c[0]), std::fabs((double)c[1]), std::fabs((double)c[2])});
+    for (uint32_t v = 0; v < n; ++v, c += RTC_CAMERA_FLOATS) {
+        const double reach = (double)lens_r * (std::max({std::fabs((double)c[3]), std::fabs((double)c[4]), std::fabs((double)c[5])}) +
+                                               std::max({std::fabs((double)c[6]), std::fabs((double)c[7]), std::fabs((double)c[8])}));
+        e = std::max({e, std::fabs((double)c[0]) + reach, std::fabs((double)c[1]) + reach, std::fabs((double)c[2]) + reach});
+    }
     return e;
 }
 // A new layout of the arena of `s` on its device, uploaded synchronously: after the host scene's index BVH was rebuilt.
@@ -958,7 +964,28 @@ int rtc_scene_set_camera(rtc_scene* s, const float cam[RTC_CAMERA_FLOATS]) {
     int rc = check_camera(cam);
     if (rc) return rc;
     s->host.cam = camera_of(s->host, cam);
-    return ensure_index_extent(s, camera_extent(cam));
+    return ensure_index_extent(s, camera_extent(cam, 1, s->host.lens_r));
+}
+int rtc_scene_set_lens(rtc_scene* s, float aperture_radius, float focus_distance) {
+    if (!s) return fail(RTC_ERR_ARG, "null scene");
+    if (!std::isfinite(aperture_radius) || !std::isfinite(focus_distance)) return fail(RTC_ERR_ARG, "lens values must be finite");
+    if (!(aperture_radius >= 0.f)) return fail(RTC_ERR_ARG, "lens aperture radius must be >= 0");
+    if (!(focus_distance > 0.f)) return fail(RTC_ERR_ARG, "lens focus distance must be > 0");
+    if (aperture_radius > 0.f && s->host.dialect <= DIALECT_HW2)
+        return fail(RTC_ERR_UNSUPPORTED, "hw1 / hw2 render one deterministic frame: a lens needs sampled dialects");
+    float cam[RTC_CAMERA_FLOATS];
+    rtc_scene_camera(s, cam);
+    int rc = ensure_index_extent(s, camera_extent(cam, 1, aperture_radius));
+    if (rc) return rc;
+    s->host.lens_r = aperture_radius;
+    s->host.lens_f = focus_distance;
+    return RTC_OK;
+}
+int rtc_scene_lens(const rtc_scene* s, float out[2]) {
+    if (!s || !out) return fail(RTC_ERR_ARG, "null argument");
+    out[0] = s->host.lens_r;
+    out[1] = s->host.lens_f;
+    return RTC_OK;
 }
 int rtc_scene_prim_order(const rtc_scene* s, int32_t* out) {
     if (!s || !out) return fail(RTC_ERR_ARG, "null argument");
@@ -1178,6 +1205,10 @@ int rtc_camera_list_lengths(rtc_scene* s, uint32_t* lengths_host) {
     if (!lengths_host) return fail(RTC_ERR_ARG, "null argument");
     const size_t npix = (size_t)s->host.cam.width * s->host.cam.height;
     if (npix == 0) return RTC_OK;
+    if (s->host.lens_r > 0.f) {   // lens renders build no lists: every camera ray takes the index traversal
+        std::fill(lengths_host, lengths_host + npix, 0xFFFFFFFFu);
+        return RTC_OK;
+    }
     DevScene S;
     if ((rc = arena_begin(s, nullptr, &S))) return rc;
     DevBuf<uint32_t> buf;
@@ -1224,7 +1255,7 @@ int rtc_render_views_accumulate(rtc_scene* s, const float* cams_host, int nviews
     const uint64_t total = (uint64_t)nviews * s->host.cam.width * s->host.cam.height * sample_count;
     if (total == 0) return RTC_OK;
     if (!accum_dev) return fail(RTC_ERR_ARG, "null accumulation buffer");
-    if ((rc = ensure_index_extent(s, camera_extent(cams_host, (uint32_t)nviews)))) return rc;
+    if ((rc = ensure_index_extent(s, camera_extent(cams_host, (uint32_t)nviews, s->host.lens_r)))) return rc;
     return accumulate(s, cams_host, (uint32_t)nviews, seed, sample_begin, sample_count, accum_dev, (cudaStream_t)stream);
 }
 
@@ -1526,7 +1557,7 @@ int frame_u8(rtc_scene* s, const int* devices, int ndev, const float* cams_host,
     if (rc) return rc;
     const size_t nvalues = 3 * (size_t)nviews * s->host.cam.width * s->host.cam.height;
     if (nvalues == 0) return RTC_OK;   // no DIMENSIONS: the reference writes a PPM header and no pixels
-    if (cams_host && (rc = ensure_index_extent(s, camera_extent(cams_host, nviews)))) return rc;
+    if (cams_host && (rc = ensure_index_extent(s, camera_extent(cams_host, nviews, s->host.lens_r)))) return rc;
     std::vector<rtc_scene*> ctx;
     if ((rc = device_contexts(s, devices, ndev, ctx))) return rc;
     auto issue = [&](int i) -> int {

@@ -31,6 +31,14 @@ inline DevCamera dev_camera(const Camera& cam) {
     return C;
 }
 
+// The thin lens as the camera kernels read it (DESIGN.md "Thin lens"): aperture radius r and r / f.  It travels as a
+// trailing kernel parameter of the kernels that make camera rays, not in DevScene: DevScene is the first parameter of
+// every kernel, and a larger DevScene would move every parameter after it, in every kernel.
+struct DevLens {
+    float r, r_over_f;
+};
+inline DevLens dev_lens(const HostScene& host) { return DevLens{host.lens_r, host.lens_r / host.lens_f}; }
+
 struct DevScene {
     // per primitive (final order), 16-byte aligned float4 arrays
     const float4* geo0;    // triangle (a, n.x) | other (d0, 0)

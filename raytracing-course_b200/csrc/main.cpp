@@ -12,6 +12,9 @@
 //                        the recommended strength, 0 leaves the image as rendered): every pixel at SAMPLES, or with
 //                        RTC_ADAPTIVE=<tau> adaptive sampling as above.  A value that is not a finite number >= 0 or a list
 //                        of several RTC_DEVICES is an error.
+//   RTC_LENS=<r>,<f>     depth of field: a thin lens of aperture radius r (world units) focused at distance f
+//                        (rtc_scene_set_lens); combines with every other variable.  A malformed value, or one the library
+//                        refuses (r < 0, f <= 0, not finite, r > 0 on hw1 / hw2), is an error.
 //   RTC_TIMING=1     phase times on stderr (with RTC_ADAPTIVE or RTC_DENOISE also the passes and paths rendered)
 // The same program serves the four earlier homework snapshots (hwN/run.sh -> build/raytracing_hwN): the dialect
 // is the digit in the name it is called by (raytracing_hw1 .. raytracing_hw4 are links to this binary), or
@@ -123,6 +126,27 @@ int main(int argc, const char* argv[]) {
         std::fprintf(stderr, "raytracing_hw5: %s\n", rtc_last_error());
         rtc_scene_free(scene);
         return 1;
+    }
+    if (const char* lens = std::getenv("RTC_LENS"); lens && *lens) {
+        char* end = nullptr;
+        const float r = std::strtof(lens, &end);
+        float f = 0.f;
+        bool ok = end != lens && *end == ',';
+        if (ok) {
+            const char* second = end + 1;
+            f = std::strtof(second, &end);
+            ok = end != second && !*end;
+        }
+        if (!ok) {
+            std::fprintf(stderr, "raytracing_hw5: RTC_LENS=%s is not <aperture radius>,<focus distance>\n", lens);
+            rtc_scene_free(scene);
+            return 1;
+        }
+        if (rtc_scene_set_lens(scene, r, f) != RTC_OK) {
+            std::fprintf(stderr, "raytracing_hw5: RTC_LENS=%s: %s\n", lens, rtc_last_error());
+            rtc_scene_free(scene);
+            return 1;
+        }
     }
     uint32_t info[8];
     rtc_scene_info(scene, info);

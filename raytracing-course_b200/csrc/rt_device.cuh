@@ -949,6 +949,50 @@ RT_D void camera_ray(const DevScene& S, float x, float y, vec3& o, vec3& d) { ca
 // GetReflection, src/scene.cpp:79-81
 RT_D vec3 reflect_dir(vec3 n, vec3 dir) { return dir - (2.0f * n) * dot(n, dir); }
 
+// ------------------------------------------------------------------------------- thin lens
+// Shirley-Chiu concentric map of (u, v) in [0, 1)^2 onto the unit disk, without FMA contraction (the oracle restates it
+// in C).  The angle is carried in units of pi, th = angle / pi in [-1/4, 3/4], and sin / cos (pi th) are evaluated in
+// double and rounded once to float: sincospi on the device (no argument-reduction table), sin / cos of the double
+// product pi th in the host builds (tests/host_emul, the oracle).  The two double results differ by an ulp of a double
+// at most, so the float lens points are the same unless one lies within that of a float rounding boundary.
+RT_D void concentric_disk(float u, float v, float& lx, float& ly) {
+    const float sx = __fadd_rn(__fmul_rn(2.f, u), -1.f), sy = __fadd_rn(__fmul_rn(2.f, v), -1.f);
+    if (sx == 0.f && sy == 0.f) { lx = 0.f; ly = 0.f; return; }
+    float rad, th;
+    if (fabsf(sx) > fabsf(sy)) { rad = sx; th = __fmul_rn(0.25f, __fdiv_rn(sy, sx)); }
+    else { rad = sy; th = __fadd_rn(0.5f, -__fmul_rn(0.25f, __fdiv_rn(sx, sy))); }
+    float s, c;
+#ifdef __CUDA_ARCH__
+    double sd, cd;
+    sincospi((double)th, &sd, &cd);
+    s = (float)sd;
+    c = (float)cd;
+#else
+    s = (float)sin(3.141592653589793 * (double)th);
+    c = (float)cos(3.141592653589793 * (double)th);
+#endif
+    lx = __fmul_rn(rad, c);
+    ly = __fmul_rn(rad, s);
+}
+// The lens step of a camera sample (DESIGN.md "Thin lens"): (o, d) from camera_ray, b = the sample's slot-0 block, whose
+// .x / .y gave the jitter; .z / .w pick the lens point (lx, ly).  With e = lx right + ly up the ray starts at o + r e and
+// runs along d - (r / f) e: every ray of the sample passes through o + f d, and d keeps its forward coefficient 1.
+RT_D void lens_ray(const DevCamera& C, DevLens L, uint4 b, vec3& o, vec3& d) {
+    float lx, ly;
+    concentric_disk(u01(b.z), u01(b.w), lx, ly);
+    const vec3 e = mk3(__fadd_rn(__fmul_rn(lx, C.right.x), __fmul_rn(ly, C.up.x)), __fadd_rn(__fmul_rn(lx, C.right.y), __fmul_rn(ly, C.up.y)),
+                       __fadd_rn(__fmul_rn(lx, C.right.z), __fmul_rn(ly, C.up.z)));
+    o = mk3(__fadd_rn(o.x, __fmul_rn(L.r, e.x)), __fadd_rn(o.y, __fmul_rn(L.r, e.y)), __fadd_rn(o.z, __fmul_rn(L.r, e.z)));
+    d = mk3(__fadd_rn(d.x, -__fmul_rn(L.r_over_f, e.x)), __fadd_rn(d.y, -__fmul_rn(L.r_over_f, e.y)),
+            __fadd_rn(d.z, -__fmul_rn(L.r_over_f, e.z)));
+}
+// The camera ray of a sample at film position (x, y): camera_ray, then, LENS, lens_ray with the sample's slot-0 block b
+template <bool LENS>
+RT_D void camera_sample(const DevCamera& C, uint32_t width, uint32_t height, float x, float y, uint4 b, DevLens L, vec3& o, vec3& d) {
+    camera_ray(C, width, height, x, y, o, d);
+    if (LENS) lens_ray(C, L, b, o, d);
+}
+
 // ------------------------------------------------------------------------------- per-pixel candidate leaves
 // All camera rays of a pixel start at C.pos and differ only by their jitter, so one conservative traversal of the index
 // tree with the pixel's whole beam of directions (pixel_candidates) finds every leaf the index traversal of any of its
@@ -958,7 +1002,8 @@ RT_D vec3 reflect_dir(vec3 n, vec3 dir) { return dir - (2.0f * n) * dot(n, dir);
 // same (DESIGN.md "Camera rays from per-pixel candidate lists").
 //
 // A pixel whose beam reaches more than kMaxRecords leaves, or at whose nodes k_traverse could run out of stack, is
-// marked kPixelTraverse: its rays take pre_step and k_traverse as every other ray does.
+// marked kPixelTraverse: its rays take pre_step and k_traverse as every other ray does.  A thin lens gives every sample its own origin;
+// lens renders build no lists (measured slower than the index traversal: DESIGN.md "Thin lens").
 constexpr uint32_t kPixelTraverse = 0xFFFFFFFFu;
 // k_traverse's per-lane stack (rt_kernels.cu): inner-node stack from the bottom, noted leaves from the top
 constexpr int kStackWords = 56;

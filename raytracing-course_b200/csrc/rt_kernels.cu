@@ -116,9 +116,9 @@ RT_D bool queue_slot(const QueueView& v, uint32_t at, uint32_t cap, uint32_t& sl
 // sample), stored in slot i with `word` as its pixel word, and its pre_step; returns the root children the ray enters
 // (o, d, cd: what the traverse queue takes).  With `cand` (the pixel lists of k_pixel_candidates, camera C = the scene's
 // own) a pixel that has a list resolves its ray here -- closest plane, leaf_test of every candidate, replay -- and
-// returns 0: the ray is not queued.  `listed` counts those rays.
-RT_D uint32_t camera_path(const DevScene& S, const DevCamera& C, PathSoA P, HitSoA H, uint32_t i, uint32_t pixel, uint32_t word,
-                          uint32_t sample, uint32_t seed, const uint32_t* cand, uint32_t& listed, vec3& o, vec3& d, float& cd) {
+// returns 0: the ray is not queued.  `listed` counts those rays.  LENS: through the thin lens L, never from lists.
+template <bool LENS> RT_D uint32_t camera_path(const DevScene& S, const DevCamera& C, PathSoA P, HitSoA H, uint32_t i, uint32_t pixel,
+                          uint32_t word, uint32_t sample, uint32_t seed, const uint32_t* cand, uint32_t& listed, vec3& o, vec3& d, float& cd, DevLens L) {
     uint32_t x = pixel % S.width, y = pixel / S.width;
     Rng g{seed, pixel, sample, 0};
     uint4 b = g.block(0);
@@ -126,10 +126,10 @@ RT_D uint32_t camera_path(const DevScene& S, const DevCamera& C, PathSoA P, HitS
     // hw3's Camera::GetToRay(float, float) still adds the half pixel of its integer ancestor
     // (hw3 src/scene.cpp:186-187): its jittered samples cover [x + 0.5, x + 1.5)
     if (S.dialect == DIALECT_HW3) { fx = __fadd_rn(fx, 0.5f); fy = __fadd_rn(fy, 0.5f); }
-    camera_ray(C, S.width, S.height, fx, fy, o, d);
+    camera_sample<LENS>(C, S.width, S.height, fx, fy, b, L, o, d);
     uint32_t id;
     const uint32_t npix = S.width * S.height;
-    const uint32_t n = cand ? __ldg(cand + pixel) : kPixelTraverse;
+    const uint32_t n = !LENS && cand ? __ldg(cand + pixel) : kPixelTraverse;
     uint32_t enters = 0;
     if (n == kPixelTraverse) {
         enters = pre_step(S, o, d, cd, id);
@@ -166,12 +166,12 @@ RT_D void count_listed(uint32_t listed, unsigned long long* stats) {
 // One thread per path.  Path ids run sample-major over the image: consecutive threads = consecutive pixels of a row.
 // With `views` (nviews cameras) path p is pixel p % npix of view (p / npix) % nviews and sample sample_begin +
 // p / (npix nviews); its pixel word is the frame-wide index view npix + pixel.  Without (VIEWS = false), the scene's own
-// camera, in a kernel of its own: a one-frame render runs the code it ran before views existed.
-template <bool VIEWS>
+// camera, in a kernel of its own: a one-frame render runs the code it ran before views existed.  LENS: the thin lens L.
+template <bool VIEWS, bool LENS>
 __global__ void __launch_bounds__(256) k_generate(DevScene S, PathSoA P, HitSoA H, uint32_t* q, uint32_t* tq, uint32_t* tq_count,
                                                    uint64_t first_path, uint32_t count, uint32_t seed, uint32_t sample_begin,
                                                    const DevCamera* views, uint32_t nviews, const uint32_t* cand,
-                                                   unsigned long long* stats) {
+                                                   unsigned long long* stats, DevLens L) {
     const uint32_t npix = S.width * S.height;
     const uint32_t lane = threadIdx.x & 31;
     const uint32_t rounded = (count + 31u) & ~31u;
@@ -186,8 +186,8 @@ __global__ void __launch_bounds__(256) k_generate(DevScene S, PathSoA P, HitSoA 
             uint32_t pixel = (uint32_t)(pid % npix);
             const uint32_t view = VIEWS ? (uint32_t)(frame % nviews) : 0u;
             const uint32_t sample = sample_begin + (uint32_t)(VIEWS ? frame / nviews : frame);
-            enters = camera_path(S, VIEWS ? views[view] : S.cam, P, H, i, pixel, view * npix + pixel, sample, seed,
-                                 VIEWS ? nullptr : cand, listed, o, d, cd);
+            enters = camera_path<LENS>(S, VIEWS ? views[view] : S.cam, P, H, i, pixel, view * npix + pixel, sample, seed,
+                                       VIEWS ? nullptr : cand, listed, o, d, cd, L);
         }
         enqueue(enters, i, o, d, cd, tq, tq_count, lane);
     }
@@ -196,10 +196,10 @@ __global__ void __launch_bounds__(256) k_generate(DevScene S, PathSoA P, HitSoA 
 }
 // The same over a pixel list (adaptive sampling): path id p is pixel plist[p % npix] and sample sample_first +
 // 2 (p / npix) -- every other sample, so that one call renders the even or the odd samples of a range.
-__global__ void __launch_bounds__(256) k_generate_list(DevScene S, PathSoA P, HitSoA H, uint32_t* q, uint32_t* tq, uint32_t* tq_count,
-                                                        uint64_t first_path, uint32_t count, uint32_t seed, const uint32_t* plist,
+template <bool LENS> __global__ void __launch_bounds__(256) k_generate_list(DevScene S, PathSoA P, HitSoA H, uint32_t* q, uint32_t* tq,
+                                                        uint32_t* tq_count, uint64_t first_path, uint32_t count, uint32_t seed, const uint32_t* plist,
                                                         uint32_t npix, uint32_t sample_first, const uint32_t* cand,
-                                                        unsigned long long* stats) {
+                                                        unsigned long long* stats, DevLens L) {
     const uint32_t lane = threadIdx.x & 31;
     const uint32_t rounded = (count + 31u) & ~31u;
     uint32_t listed = 0;
@@ -211,7 +211,7 @@ __global__ void __launch_bounds__(256) k_generate_list(DevScene S, PathSoA P, Hi
             uint64_t pid = first_path + i;
             uint32_t sample = sample_first + 2u * (uint32_t)(pid / npix);
             uint32_t pixel = plist[pid % npix];
-            enters = camera_path(S, S.cam, P, H, i, pixel, pixel, sample, seed, cand, listed, o, d, cd);
+            enters = camera_path<LENS>(S, S.cam, P, H, i, pixel, pixel, sample, seed, cand, listed, o, d, cd, L);
         }
         enqueue(enters, i, o, d, cd, tq, tq_count, lane);
     }
@@ -1054,19 +1054,32 @@ static int grid_for(uint64_t n, int block, int sms, int per_sm) {
 
 void launch_generate(const LaunchCtx& c, const DevScene& S, PathSoA P, HitSoA H, uint32_t* q, uint32_t* tq, uint32_t* tq_count,
                      uint64_t first_path, uint32_t count, uint32_t seed, uint32_t sample_begin, const DevCamera* views, uint32_t nviews,
-                     const uint32_t* cand, unsigned long long* stats) {
-    if (views)
-        k_generate<true><<<grid_for(count, 256, c.sms, 8), 256, 0, c.stream>>>(S, P, H, q, tq, tq_count, first_path, count, seed,
-                                                                               sample_begin, views, nviews, nullptr, nullptr);
+                     const uint32_t* cand, unsigned long long* stats, DevLens L) {
+    const int grid = grid_for(count, 256, c.sms, 8);
+    const bool lens = L.r > 0.f;
+    if (views && lens)
+        k_generate<true, true><<<grid, 256, 0, c.stream>>>(S, P, H, q, tq, tq_count, first_path, count, seed, sample_begin, views, nviews,
+                                                           nullptr, nullptr, L);
+    else if (views)
+        k_generate<true, false><<<grid, 256, 0, c.stream>>>(S, P, H, q, tq, tq_count, first_path, count, seed, sample_begin, views, nviews,
+                                                            nullptr, nullptr, L);
+    else if (lens)
+        k_generate<false, true><<<grid, 256, 0, c.stream>>>(S, P, H, q, tq, tq_count, first_path, count, seed, sample_begin, nullptr, 1,
+                                                            cand, stats, L);
     else
-        k_generate<false><<<grid_for(count, 256, c.sms, 8), 256, 0, c.stream>>>(S, P, H, q, tq, tq_count, first_path, count, seed,
-                                                                                sample_begin, nullptr, 1, cand, stats);
+        k_generate<false, false><<<grid, 256, 0, c.stream>>>(S, P, H, q, tq, tq_count, first_path, count, seed, sample_begin, nullptr, 1,
+                                                             cand, stats, L);
 }
 void launch_generate_list(const LaunchCtx& c, const DevScene& S, PathSoA P, HitSoA H, uint32_t* q, uint32_t* tq, uint32_t* tq_count,
                           uint64_t first_path, uint32_t count, uint32_t seed, const uint32_t* plist, uint32_t npix, uint32_t sample_first,
-                          const uint32_t* cand, unsigned long long* stats) {
-    k_generate_list<<<grid_for(count, 256, c.sms, 8), 256, 0, c.stream>>>(S, P, H, q, tq, tq_count, first_path, count, seed, plist,
-                                                                          npix, sample_first, cand, stats);
+                          const uint32_t* cand, unsigned long long* stats, DevLens L) {
+    const int grid = grid_for(count, 256, c.sms, 8);
+    if (L.r > 0.f)
+        k_generate_list<true><<<grid, 256, 0, c.stream>>>(S, P, H, q, tq, tq_count, first_path, count, seed, plist, npix, sample_first,
+                                                          cand, stats, L);
+    else
+        k_generate_list<false><<<grid, 256, 0, c.stream>>>(S, P, H, q, tq, tq_count, first_path, count, seed, plist, npix, sample_first,
+                                                           cand, stats, L);
 }
 void launch_pixel_candidates(const LaunchCtx& c, const DevScene& S, uint32_t* cand, bool count_visits, unsigned long long* stats) {
     const uint32_t npix = S.width * S.height;

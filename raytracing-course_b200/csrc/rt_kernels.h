@@ -21,14 +21,15 @@ struct LaunchCtx {
 // camera rays of one wavefront batch + their pre_step (planes, index root, traverse queue): through the scene's camera
 // (views = null), or through nviews cameras, path p = pixel p % npix of view (p / npix) % nviews, sample sample_begin +
 // p / (npix nviews), pixel word view npix + pixel.  cand (scene camera only, may be null): the pixel candidate lists of
-// launch_pixel_candidates; a pixel with a list resolves its camera rays in the kernel, counted in stats[kStatListRays]
+// launch_pixel_candidates; a pixel with a list resolves its camera rays in the kernel, counted in stats[kStatListRays].  L: the scene's
+// thin lens (dev_lens); r > 0 launches the lens instantiations, which move every camera ray through the lens and read no lists
 void launch_generate(const LaunchCtx& c, const DevScene& S, PathSoA P, HitSoA H, uint32_t* q, uint32_t* tq, uint32_t* tq_count,
                      uint64_t first_path, uint32_t count, uint32_t seed, uint32_t sample_begin, const DevCamera* views, uint32_t nviews,
-                     const uint32_t* cand, unsigned long long* stats);
+                     const uint32_t* cand, unsigned long long* stats, DevLens L);
 // the same over a pixel list: path p = pixel plist[p % npix], sample sample_first + 2 (p / npix)
 void launch_generate_list(const LaunchCtx& c, const DevScene& S, PathSoA P, HitSoA H, uint32_t* q, uint32_t* tq, uint32_t* tq_count,
                           uint64_t first_path, uint32_t count, uint32_t seed, const uint32_t* plist, uint32_t npix, uint32_t sample_first,
-                          const uint32_t* cand, unsigned long long* stats);
+                          const uint32_t* cand, unsigned long long* stats, DevLens L);
 // Per pixel of the scene's camera the candidate index leaves of its camera rays (rt_device.cuh pixel_candidates):
 // kCandWords words per pixel, laid out slot-major (word j of pixel p at cand[j npix + p]); word 0 is the list length or
 // kPixelTraverse.  count_visits: its node visits into stats[4].

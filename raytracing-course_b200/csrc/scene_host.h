@@ -131,6 +131,8 @@ struct HostScene {
     uint32_t root = 0;
     std::vector<int32_t> lights;   // emissive boxes / ellipsoids
     FlatScene flat;
+    // thin lens of the camera (rtc_scene_set_lens): aperture radius (0 = pinhole) and focus distance
+    float lens_r = 0.f, lens_f = 1.f;
 
     // Scene::Load (hw5 src/sceneload.cpp:112-176; hwN src/scene.cpp Scene::Load for the other dialects):
     // only the words of `dialect` are commands, the rest is reported as unexpected and skipped
